@@ -23,6 +23,25 @@ def test_reference_arm_json_line():
     assert "workload" in line["config"] and "model" not in line["config"]
 
 
+def test_dump_outputs_writes_float32_npy(tmp_path):
+    """`--dump-outputs` format: one float32 .npy file per array the step gives its caller, values unchanged."""
+    import types
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    g = torch.Generator().manual_seed(6)
+    op = types.SimpleNamespace(losses={"loss/coarse_loss": torch.tensor([1.5]), "loss/fine_loss": torch.tensor([2.5])},
+                               coarse=torch.rand(32, 55, 74, 1, generator=g), outputs=torch.rand(32, 55, 74, 1, generator=g))
+    bench.dump_outputs(op, str(tmp_path), torch)
+    assert sorted(os.listdir(tmp_path)) == ["coarse.npy", "fine.npy", "loss_coarse.npy", "loss_fine.npy"]
+    for name, t in (("coarse", op.coarse), ("fine", op.outputs), ("loss_coarse", op.losses["loss/coarse_loss"]),
+                    ("loss_fine", op.losses["loss/fine_loss"])):
+        a = np.load(tmp_path / (name + ".npy"))
+        assert a.dtype == np.float32
+        np.testing.assert_array_equal(a, t.numpy())
+
+
 def test_gpu_arm_needs_a_gpu():
     import torch
     if torch.cuda.is_available():
