@@ -16,6 +16,9 @@ A3D_ENOTSUP = -5
 IMPL_AUTO, IMPL_SIMT, IMPL_TC = 0, 1, 2
 EPI_RELU, EPI_SIGMOID = 1, 2
 OP_FWD, OP_DGRAD, OP_WGRAD = 0, 1, 2
+DM_SCALE_NONE, DM_SCALE_MEDIAN = 0, 1
+# a3d_depth_metrics slots (A3D_DM_*), in order
+DM_SLOTS = ("n", "abs_rel", "sq_rel", "sq", "log", "log_sq", "log10", "delta1", "delta2", "delta3", "nonfinite")
 
 
 class A3DError(RuntimeError):
@@ -146,6 +149,7 @@ SIGNATURES = {
     "a3d_image_cells_s2d": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "a3d_window_gather": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "a3d_window_scatter_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "a3d_depth_metrics": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _i, _f, _f, _i, _vp, _vp, _vp]),
     "a3d_comm_unique_id": (_i, [C.c_char_p, _vp]),
     "a3d_comm_init": (_i, [_vp, C.c_char_p, _vp, _i, _i]),
     "a3d_comm_destroy": (_i, [_vp]),

@@ -127,6 +127,55 @@ def setup_model(args, comm=None):
     return op, inp
 
 
+class Validator:
+    """--evalfreq: depth metrics of the training net's current parameters on the test split.  The inference net shares
+    the training net's parameter arena (no host round trip) and re-derives its pool-fused first-layer filter from it
+    before each pass; every rank evaluates its shard of the file and the metrics are summed over the gloo group."""
+
+    def __init__(self, args, op, rank, world):
+        from . import evaluate
+        self.args, self.op, self.rank, self.world = args, op, rank, world
+        self.shard = (rank, world)
+        inp = self._inputs()
+        self.eval_op = getattr(models, args.model)(inp.images, inp.depths, train=False)
+        inp.close()
+        self.eval_op.net.arena = op.net.arena
+        self.meters = evaluate.make_meters(self.eval_op, self.eval_op.net.ctx)
+        self.last_step = None
+
+    def _inputs(self):
+        return data.inputs(self.args.datadir, self.args.dataset, self.args.batchsize, "test", epochs=1, shard=self.shard)
+
+    def run(self, writer=None):
+        from . import evaluate
+        net = self.op.net
+        if hasattr(net, "flush"):
+            net.flush()                 # data parallel: dense rows other ranks own are current only after the publish
+        self.eval_op.net.refresh_derived()
+        inp = self._inputs()
+        self.eval_op.net.images, self.eval_op.net.depths = inp.images, inp.depths
+        for m in self.meters.values():
+            m.reset()
+        try:
+            evaluate.evaluate_split(self.eval_op, inp, self.meters)
+        finally:
+            inp.close()
+        step = self.op.global_step
+        scalars = {}
+        for name, m in self.meters.items():
+            m.reduce()
+            for k, v in m.result().items():
+                if k in evaluate.METRICS and v is not None:
+                    scalars[f"eval/{name}/{k}"] = v
+        if writer is not None:
+            writer.add_scalars(step, scalars)
+            writer.flush()
+        if self.rank == 0:
+            logger.info(f"step {step} eval " + " ".join(f"{k}={v:.4g}" for k, v in scalars.items()))
+        self.last_step = step
+        return scalars
+
+
 def main(argv=None):
     logging.basicConfig(level=logging.DEBUG, stream=sys.stdout,
                         format="%(asctime)s %(name)s %(levelname)s %(message)s")
@@ -158,6 +207,7 @@ def main(argv=None):
     if restore_checkpoint(op, ckptdir):
         logger.info(f"Restored checkpoint at global step {op.global_step}.")
 
+    validator = Validator(args, op, rank, world) if args.evalfreq > 0 else None
     stop_hook = StopAtSignalHook()
     # chief-only observability, as in the reference (src/ann3depth.py:98-111): loss summaries every --sumfreq
     # steps and a per-kernel trace of the first step after a (re)start and of every 5000th step, both in ckptdir
@@ -198,6 +248,10 @@ def main(argv=None):
             logger.info(f"step {op.global_step} losses {losses} global_step/sec {rate:.2f} "
                         f"images/sec {rate * args.batchsize * world:.1f}")
             last_log, last_log_step = now, op.global_step
+        if validator is not None and op.global_step % args.evalfreq == 0:
+            validator.run(writer)
+    if validator is not None and not stop_signal and validator.last_step != op.global_step:
+        validator.run(writer)                                                  # the final step
     if world > 1 and not stop_signal:
         # the step limit is reached by all ranks together; a signal that arrived since the last consensus point still
         # decides the exit code (and every rank takes part in the final checkpoint either way)
@@ -230,6 +284,8 @@ def parse_args(argv=None):
     parser.add_argument("--sumfreq", "-r", default=100, type=int, help="Create a summary every N steps.")
     parser.add_argument("--datadir", "-d", default="data", type=str, help="The data directory containing the datasets.")
     parser.add_argument("--timeout", "-k", default=4200, type=int, help="The time after which the process dies.")
+    parser.add_argument("--evalfreq", default=0, type=int,
+                        help="Evaluate the test split every N steps and at the last step (0: never; beyond the reference).")
     parser.add_argument("--cluster-spec", default="", type=str, help="(ignored: no parameter servers)")
     parser.add_argument("--job-name", default="local", type=str, help="(ignored)")
     parser.add_argument("--task-index", default=0, type=int, help="(ignored)")

@@ -89,6 +89,21 @@ __device__ __forceinline__ void split_rc(size_t i, int C, size_t& r, int& c) {
   }
 }
 
+// TF1 legacy bilinear mapping (tf.image.resize_images, align_corners=False): source coordinate = dst * (in/out),
+// lo = floor, hi = min(lo+1, in-1), weight = coordinate - lo.  Shared by a3d_resize_bilinear_tf1 and
+// a3d_depth_metrics, which samples the prediction at ground-truth pixels and must see the resize's values bit for bit.
+__device__ __forceinline__ void tf1_coord(int o, float scale, int in, int& lo, int& hi, float& w) {
+  float f = o * scale;
+  lo = (int)floorf(f);
+  hi = min(lo + 1, in - 1);
+  w = f - lo;
+}
+__device__ __forceinline__ float tf1_lerp(float tl, float tr, float bl, float br, float ly, float lx) {
+  float top = tl + (tr - tl) * lx;
+  float bot = bl + (br - bl) * lx;
+  return top + (bot - top) * ly;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -13,8 +13,7 @@ static inline int grid_for(a3d_ctx* ctx, size_t work_items, int block, int max_w
 }
 
 // ------------------------------------------------------------------------------------ resize
-// TF1 legacy bilinear: src = dst * (in/out); lo = floor(src); hi = min(lo+1, in-1); lerp = src-lo.
-// One thread per output pixel; the <= 4 channels of a pixel are adjacent so a warp reads a
+// TF1 legacy bilinear (tf1_coord / tf1_lerp, common.cuh).  One thread per output pixel; the <= 4 channels of a pixel are adjacent so a warp reads a
 // contiguous strip of each of the two source rows.
 template <bool OUT_BF16>
 __global__ void resize_bilinear_tf1_kernel(const float* __restrict__ src, int B, int H, int W, int C,
@@ -25,10 +24,10 @@ __global__ void resize_bilinear_tf1_kernel(const float* __restrict__ src, int B,
     size_t t = i / OW;
     int oy = (int)(t % OH);
     int b = (int)(t / OH);
-    float fy = oy * sy, fx = ox * sx;
-    int y0 = (int)floorf(fy), x0 = (int)floorf(fx);
-    int y1 = min(y0 + 1, H - 1), x1 = min(x0 + 1, W - 1);
-    float ly = fy - y0, lx = fx - x0;
+    int y0, y1, x0, x1;
+    float ly, lx;
+    tf1_coord(oy, sy, H, y0, y1, ly);
+    tf1_coord(ox, sx, W, x0, x1, lx);
     const float* r0 = src + ((size_t)b * H + y0) * W * C;
     const float* r1 = src + ((size_t)b * H + y1) * W * C;
     for (int c = 0; c < dstC; ++c) {
@@ -36,9 +35,7 @@ __global__ void resize_bilinear_tf1_kernel(const float* __restrict__ src, int B,
       if (c < C) {
         float tl = __ldg(r0 + (size_t)x0 * C + c), tr = __ldg(r0 + (size_t)x1 * C + c);
         float bl = __ldg(r1 + (size_t)x0 * C + c), br = __ldg(r1 + (size_t)x1 * C + c);
-        float top = tl + (tr - tl) * lx;
-        float bot = bl + (br - bl) * lx;
-        v = top + (bot - top) * ly;
+        v = tf1_lerp(tl, tr, bl, br, ly, lx);
       }
       if (OUT_BF16) reinterpret_cast<uint16_t*>(dst)[i * dstC + c] = f32_to_bf16_bits(v);
       else reinterpret_cast<float*>(dst)[i * dstC + c] = v;

@@ -203,6 +203,38 @@ class _RecordSource:
             torch.add(dp.view(depths.shape[1:]), 0.5, out=depths[i])
 
 
+class _SequentialSource(_RecordSource):
+    """One pass over the records of a TFRecord file in file order, no shuffle pool (evaluation on the test split):
+    shard (r, n) takes records r, r + n, r + 2n, ...  `fill` returns how many rows it wrote (0 at the end)."""
+
+    def __init__(self, path, batch, shard=(0, 1)):
+        super().__init__(path, batch, 0)
+        rank, world = shard
+        if not 0 <= rank < world:
+            raise ValueError(f"shard {shard}: need 0 <= rank < world")
+        self.order = list(range(rank, len(self.index), world))
+        self.cursor = 0
+
+    def _dequeue(self):
+        with self.lock:
+            if self.cursor >= len(self.order):
+                return None
+            self.cursor += 1
+            return self.order[self.cursor - 1]
+
+    def fill(self, images, depths):
+        for i in range(images.shape[0]):
+            j = self._dequeue()
+            if j is None:
+                return i
+            e = self.read(j)
+            im = torch.frombuffer(e["image"], dtype=torch.float32)
+            dp = torch.frombuffer(e["depth"], dtype=torch.float32)
+            torch.add(im.view(images.shape[1:]), 0.5, out=images[i])
+            torch.add(dp.view(depths.shape[1:]), 0.5, out=depths[i])
+        return images.shape[0]
+
+
 class Inputs:
     """`images`, `depths`: persistent CUDA buffers (the op's input tensors); `next_batch()` refills them in place.
 
@@ -212,14 +244,29 @@ class Inputs:
     enqueued before -- and copies the previous staging buffer into `images` / `depths` on the caller's stream (device to
     device, ~60 us).  The loop therefore runs at max(step, PCIe copy, host fill / num_threads), not at their sum.
     `synthetic="device"`: without a TFRecord file the batch is drawn on the GPU straight into `images` / `depths`
-    (no host work at all: the train loop then runs at the benchmark's device-resident speed)."""
+    (no host work at all: the train loop then runs at the benchmark's device-resident speed).
+
+    `epochs=1` (evaluation; beyond the reference): every record of the file (of the shard `(rank, world)`: records rank,
+    rank + world, ...) exactly once, in file order, one reader thread; no batch is taken at construction.
+    `next_batch()` then returns the number of rows it filled -- the last batch may be partial (its trailing rows are
+    stale) -- and 0 once the file is exhausted.  The file must exist."""
 
     def __init__(self, datadir, dataset, batch_size=32, train_or_test="train", device="cuda", seed=0,
-                 image_hw=(480, 640), depth_hw=(55, 73), synthetic="device", num_threads=2, host_slots=3):
+                 image_hw=(480, 640), depth_hw=(55, 73), synthetic="device", num_threads=2, host_slots=3, epochs=None,
+                 shard=(0, 1)):
         self.B, self.device = batch_size, torch.device(device)
         self.path = os.path.join(datadir, dataset, f"{train_or_test}.tfrecords")      # src/data.py:58-59
         self.source = None
-        if os.path.exists(self.path):
+        if epochs not in (None, 1):
+            raise ValueError("epochs must be None (repeat forever, shuffled) or 1 (one ordered pass)")
+        self.single_pass, self._exhausted = epochs == 1, False
+        if self.single_pass:
+            if not os.path.exists(self.path):
+                raise FileNotFoundError(f"{self.path} not found")
+            self.source = _SequentialSource(self.path, batch_size, shard)
+            image_hw, depth_hw = self.source.image_hw, self.source.depth_hw
+            num_threads = 1                            # batches must come out in file order
+        elif os.path.exists(self.path):
             self.source = _RecordSource(self.path, batch_size, seed)
             image_hw, depth_hw = self.source.image_hw, self.source.depth_hw
         elif synthetic == "host":
@@ -245,13 +292,15 @@ class Inputs:
                 for ev in self._drained:
                     ev.record(torch.cuda.current_stream())
             self._inflight = None            # (host slot, staging index) whose H2D is under way
+            self._rows = [batch_size] * len(self._h)        # rows the last fill of each host slot wrote
             self._n = 0
             for _ in range(max(num_threads, 1)):
                 t = threading.Thread(target=self._worker, daemon=True)
                 t.start()
                 self._threads.append(t)
             self._prefetch()
-        self.next_batch()
+        if not self.single_pass:
+            self.next_batch()
 
     # ---- worker threads: host batches
     def _worker(self):
@@ -261,14 +310,25 @@ class Inputs:
             except queue.Empty:
                 continue
             try:
-                self.source.fill(*self._h[k])
+                rows = self.source.fill(*self._h[k])
+                self._rows[k] = self.B if rows is None else rows
                 self._ready.put((k, None))
+                if rows == 0:                                        # single pass: nothing left to read
+                    return
             except Exception as e:                                   # surface reader errors in the training thread
                 self._ready.put((k, e))
                 return
 
     def _take_ready(self):
-        k, err = self._ready.get()
+        while True:
+            try:
+                k, err = self._ready.get(timeout=0.1)
+                break
+            except queue.Empty:
+                # a worker exits after its first error (or at the end of a single pass); once none is left, nothing
+                # will arrive -- fail instead of waiting forever
+                if not any(t.is_alive() for t in self._threads) and self._ready.empty():
+                    raise IOError(f"{self.path}: no reader thread left (an earlier read failed)")
         if err is not None:
             raise err
         return k
@@ -293,7 +353,10 @@ class Inputs:
             self.images.uniform_(0.0, 1.0, generator=self.gen)
             self.depths.uniform_(0.05, 1.0, generator=self.gen)
             return self.images, self.depths
+        if self._exhausted:
+            return 0
         k, j = self._inflight
+        rows = self._rows[k]
         if j is None:                                  # CPU tensors (tests): plain copies
             self.images.copy_(self._h[k][0])
             self.depths.copy_(self._h[k][1])
@@ -306,6 +369,12 @@ class Inputs:
             self._drained[j].record(cur)
             self._staged[j].synchronize()              # the H2D has read the pinned batch: hand it back to the workers
             self._free.put(k)
+        if self.single_pass:
+            if rows == 0:
+                self._exhausted = True
+                return 0
+            self._prefetch()
+            return rows
         self._prefetch()                               # overlaps the step the caller enqueues next
         return self.images, self.depths
 
@@ -321,5 +390,6 @@ class Inputs:
 
 def inputs(datadir, dataset, batch_size=32, train_or_test="train", epochs=None, **kw):
     """Same call as the reference's `data.inputs` (src/data.py:28-29); returns an `Inputs` object whose
-    `.images` / `.depths` are the tensors to hand to `models.<model>(images, depths)`."""
-    return Inputs(datadir, dataset, batch_size, train_or_test, **kw)
+    `.images` / `.depths` are the tensors to hand to `models.<model>(images, depths)`.  `epochs=1` (with `shard=(rank,
+    world)`): one ordered pass for evaluation, see `Inputs`."""
+    return Inputs(datadir, dataset, batch_size, train_or_test, epochs=epochs, **kw)

@@ -613,6 +613,24 @@ class Context:
                                                 _stream()), "window_scatter_sum")
         return g_src
 
+    # ------------------------------------------------------------------ evaluation
+    def depth_metrics(self, pred, gt, min_depth, max_depth, median=False, sums=None, scale=None):
+        """pred f32 [B,ph,pw(,1)], gt f32 [B,gh,gw(,1)] -> sums f64 [B, len(L.DM_SLOTS)] (a3d_depth_metrics);
+        `scale` f32 [B] (optional) receives the median scale."""
+        B, ph, pw = pred.shape[:3]
+        gh, gw = gt.shape[1:3]
+        if gt.shape[0] != B or pred.dim() == 4 and pred.shape[3] != 1 or gt.dim() == 4 and gt.shape[3] != 1:
+            raise ValueError("depth_metrics: pred [B,ph,pw(,1)] and gt [B,gh,gw(,1)] with the same B")
+        for t in (pred, gt):
+            if t.dtype != torch.float32 or not t.is_cuda or not t.is_contiguous():
+                raise ValueError("depth_metrics: pred and gt must be contiguous float32 CUDA tensors")
+        if sums is None:
+            sums = torch.empty(B, len(L.DM_SLOTS), dtype=torch.float64, device=pred.device)
+        mode = L.DM_SCALE_MEDIAN if median else L.DM_SCALE_NONE
+        L.check(self.lib.a3d_depth_metrics(self.h, _ptr(pred), B, ph, pw, _ptr(gt), gh, gw, min_depth, max_depth, mode,
+                                           _ptr(sums), _ptr(scale), _stream()), "depth_metrics")
+        return sums
+
     # ------------------------------------------------------------------ data parallel
     def comm_init(self, id_bytes: bytes, rank: int, nranks: int, nccl_path: str | None = None):
         buf = C.create_string_buffer(id_bytes, 128)

@@ -348,6 +348,32 @@ int a3d_window_gather(a3d_ctx*, const uint16_t* src, int B, int Hs, int Ws, int 
 int a3d_window_scatter_sum(a3d_ctx*, const uint16_t* g_out, int B, int Hs, int Ws, int C, int rows, int cols, int win,
                            int stride, uint16_t* g_src, void* stream);
 
+/* ---- depth-estimation metrics (Eigen et al. 2014), beyond the reference (it has no evaluation) -----------------------
+ * pred f32 [B,ph,pw] is sampled at every pixel of gt f32 [B,gh,gw] with the TF1 legacy bilinear mapping of
+ * a3d_resize_bilinear_tf1, bit for bit (no upsampled map is materialised).  Valid pixels: min_depth < gt <= max_depth
+ * (0 < min_depth < max_depth).  p~ = the sampled prediction clamped to [min_depth, max_depth]; a NaN maps to min_depth.
+ * scale_mode A3D_DM_SCALE_NONE: p = p~.  A3D_DM_SCALE_MEDIAN: s = median(gt) / median(p~) over the valid pixels (float32
+ * division of the two exact lower medians, the elements of rank floor((n-1)/2)), p = clamp(s * p~); s = 1 for an image
+ * without a valid pixel.  With d = ln p - ln g, writes sums[b][A3D_DM_*] (float64, overwritten per image) over the
+ * valid pixels, and scale[b] = s if `scale` is non-null.  The ratio tests are float32: max(p/g, g/p) < 1.25^k.
+ * No workspace, no host sync, CUDA-graph capturable; the sums do not depend on scheduling (fixed reduction order). */
+#define A3D_DM_SCALE_NONE    0
+#define A3D_DM_SCALE_MEDIAN  1
+#define A3D_DM_N          0   /* number of valid pixels */
+#define A3D_DM_ABS_REL    1   /* sum |p - g| / g */
+#define A3D_DM_SQ_REL     2   /* sum (p - g)^2 / g */
+#define A3D_DM_SQ         3   /* sum (p - g)^2 */
+#define A3D_DM_LOG        4   /* sum d */
+#define A3D_DM_LOG_SQ     5   /* sum d^2 */
+#define A3D_DM_LOG10      6   /* sum |d| / ln 10 = sum |log10 p - log10 g| */
+#define A3D_DM_DELTA1     7   /* count max(p/g, g/p) < 1.25 */
+#define A3D_DM_DELTA2     8   /* count ... < 1.25^2 */
+#define A3D_DM_DELTA3     9   /* count ... < 1.25^3 */
+#define A3D_DM_NONFINITE 10   /* count of valid pixels whose sampled prediction was NaN or +-inf */
+#define A3D_DM_SLOTS     11
+int a3d_depth_metrics(a3d_ctx*, const float* pred, int B, int ph, int pw, const float* gt, int gh, int gw,
+                      float min_depth, float max_depth, int scale_mode, double* sums, float* scale, void* stream);
+
 /* ---- data parallelism (replaces the PS/gRPC replication of src/ann3depth.py:78-92) ---------- */
 /* NCCL is dlopen()ed at first use (path = NULL -> "libnccl.so.2"). */
 int a3d_comm_unique_id(const char* nccl_path, void* id128);              /* 128-byte ncclUniqueId */
