@@ -35,6 +35,17 @@ class ConvDesc(C.Structure):
                  "dil_w", "pix_pitch")]
 
 
+class AugmentDesc(C.Structure):
+    """Mirror of `a3d_augment_desc` (include/a3d.h)."""
+    _fields_ = [(n, C.c_float) for n in
+                ("scale_lo", "scale_hi", "max_rotation_deg", "crop_fraction", "flip_prob", "color_lo", "color_hi",
+                 "aspect")]
+
+
+A3D_U8 = 2
+AUG_PARAMS = 16                       # A3D_AUG_PARAMS: floats per image in the packed parameter rows
+AUG_VALUE_COLOR, AUG_VALUE_DEPTH = 0, 1
+
 _vp, _i, _f, _sz, _u = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_uint
 
 # name -> (restype, argtypes); every symbol include/a3d.h declares
@@ -150,6 +161,9 @@ SIGNATURES = {
     "a3d_window_gather": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "a3d_window_scatter_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "a3d_depth_metrics": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _i, _f, _f, _i, _vp, _vp, _vp]),
+    "a3d_augment_draw": (_i, [_vp, C.POINTER(AugmentDesc), _i, C.c_uint64, _vp, _vp, _vp]),
+    "a3d_resize_affine_tf1_s2d": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
+    "a3d_resize_affine_tf1": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _vp, _i, _vp]),
     "a3d_comm_unique_id": (_i, [C.c_char_p, _vp]),
     "a3d_comm_init": (_i, [_vp, C.c_char_p, _vp, _i, _i]),
     "a3d_comm_destroy": (_i, [_vp]),

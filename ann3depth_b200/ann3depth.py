@@ -22,6 +22,7 @@ import time
 import torch
 
 from . import data, models
+from .augment import from_flag as augment_from_flag
 from .summary import EventWriter, SummaryHook, TraceHook
 from .init import glorot_params
 
@@ -122,7 +123,8 @@ def setup_model(args, comm=None):
     """src/ann3depth.py:134-145."""
     model = getattr(models, args.model)
     inp = data.inputs(args.datadir, args.dataset, args.batchsize, seed=100 + int(os.environ.get("RANK", 0)))
-    op = model(inp.images, inp.depths, comm=comm)
+    aug = augment_from_flag(getattr(args, "augment", "none"))          # the training op only; evaluation sees raw inputs
+    op = model(inp.images, inp.depths, comm=comm, augment=aug)
     op.net.load_params(glorot_params(seed=1, model=args.model))
     return op, inp
 
@@ -286,6 +288,9 @@ def parse_args(argv=None):
     parser.add_argument("--timeout", "-k", default=4200, type=int, help="The time after which the process dies.")
     parser.add_argument("--evalfreq", default=0, type=int,
                         help="Evaluate the test split every N steps and at the last step (0: never; beyond the reference).")
+    parser.add_argument("--augment", default="none", choices=["none", "eigen"],
+                        help="Training-time augmentation: 'eigen' = random scale, rotation, crop, flip and colour of "
+                             "Eigen et al. 2014, section 3.3, on the GPU (beyond the reference).")
     parser.add_argument("--cluster-spec", default="", type=str, help="(ignored: no parameter servers)")
     parser.add_argument("--job-name", default="local", type=str, help="(ignored)")
     parser.add_argument("--task-index", default=0, type=int, help="(ignored)")

@@ -64,7 +64,7 @@ def pair_indices(h=H, w=W):
 class DCNFNet:
     def __init__(self, ctx: ops.Context, batch: int, in_hw=(480, 640), depth_hw=(480, 640), train=True,
                  impl=L.IMPL_AUTO, naive_loss=True, comm=None, graph="reference", r_nonneg=False, train_pairwise=False,
-                 predict="unary", unary="fullconv"):
+                 predict="unary", unary="fullconv", augment=None, augment_seed=3):
         """Beyond-reference options (SURVEY.md 8f N4; defaults reproduce the reference):
              graph="grid4"        every neighbour pair of the tile grid (82 pairs != 48 nodes) instead of the reference's
                                   checkerboard star graph (src/models.py:20-30);
@@ -72,7 +72,11 @@ class DCNFNet:
              train_pairwise=True  the CRF's gradient w.r.t. r flows into `pairwise_layers` (TF 1.3 blocks it at
                                   ScatterNdUpdate, src/models.py:138-141) and SGD updates that layer too;
              predict="map"        the output is the CRF's MAP estimate y* = A^-1 z (Liu et al. eq. 12), bilinearly upsampled,
-                                  instead of the unary prediction the reference upsamples (src/models.py:187-191)."""
+                                  instead of the unary prediction the reference upsamples (src/models.py:187-191);
+             augment=Augment(...) training-time augmentation of image and depth (augment.py), drawn on the device from
+                                  (augment_seed + rank, step_dev, image) and applied by the two resizes."""
+        if augment is not None and not train:
+            raise ValueError("augment is a training option: an inference net (train=False) sees its inputs unchanged")
         self.ctx, self.B, self.train, self.impl, self.naive = ctx, batch, train, impl, naive_loss
         assert graph in ("reference", "grid4") and predict in ("unary", "map") and unary in ("fullconv", "patches")
         self.r_nonneg, self.train_pairwise, self.predict = r_nonneg, train_pairwise, predict
@@ -96,6 +100,16 @@ class DCNFNet:
         z = torch.zeros
         self.images = z(B, in_hw[0], in_hw[1], 3, **f32)
         self.depths = z(B, depth_hw[0], depth_hw[1], 1, **f32)
+        self.augment = augment
+        self.aug_params = self.aug_desc = None
+        self.external_aug = False
+        if augment is not None:
+            # device global step: the draw's counter, so replays of the captured step draw fresh parameters.  Only an
+            # augmenting net has one; the unaugmented step stays exactly as it was.
+            self.step_dev = torch.zeros(1, dtype=torch.int64, device=self.dev)
+            self.aug_desc = augment.desc()
+            self.augment_seed = augment_seed + (comm.rank if comm is not None else 0)
+            self.aug_params = z(B, L.AUG_PARAMS, **f32)
         self.im = z(B, H, W, 3, **f32)
         self.dp = z(B, H, W, 1, **f32)
         # Unary CNN (src/models.py:61-83).  unary = "fullconv" (default): the patches are plain windows (stride 40, zero
@@ -210,12 +224,26 @@ class DCNFNet:
     def export_grads(self):
         return self.arena.export_tf(self.arena.g)
 
+    def set_augment_params(self, params):
+        """Parity hook: use explicit augmentation parameters [B,16] (include/a3d.h A3D_AUG_*) instead of the device
+        draw."""
+        if self.augment is None:
+            raise ValueError("set_augment_params needs a net built with augment=Augment(...)")
+        self.aug_params.copy_(params.to(torch.float32))
+        self.external_aug = True
+
     # ------------------------------------------------------------------ forward
     def forward(self):
         c, B, NP = self.ctx, self.B, self.NP
         U, K = "unary/unary_layers/", "/kernel"
-        c.resize_bilinear_tf1(self.images, H, W, out=self.im)
-        c.resize_bilinear_tf1(self.depths, H, W, out=self.dp)
+        if self.augment is not None:
+            if not self.external_aug:
+                c.augment_draw(self.aug_desc, self.aug_params, self.augment_seed, self.step_dev)
+            c.resize_affine_tf1(self.images, H, W, self.aug_params, depth=False, out=self.im)
+            c.resize_affine_tf1(self.depths, H, W, self.aug_params, depth=True, out=self.dp)
+        else:
+            c.resize_bilinear_tf1(self.images, H, W, out=self.im)
+            c.resize_bilinear_tf1(self.depths, H, W, out=self.dp)
         # unary part (src/models.py:61-89) on all B*48 patches at once
         if self.unary == "fullconv":
             c.image_cells_s2d(self.im, PATCH_PAD, self.cells)
@@ -318,6 +346,8 @@ class DCNFNet:
             lo, hi = self.arena.group_range("Pairwise")
             self.ctx.sgd(self.arena.w[lo:hi], self.arena.g[lo:hi], self.arena.wb[lo:hi], SGD_LR, 1.0)
         self.refresh_derived()
+        if self.augment is not None:
+            self.ctx.increment_i64(self.step_dev)
 
     def train_step(self, use_graph=False):
         """One `session.run(model_op)` (src/models.py:198-200).  use_graph (single GPU): the ~45 launches of the step are
@@ -326,9 +356,12 @@ class DCNFNet:
         if use_graph and not self.comm:
             if self._graph is None:
                 saved = (self.arena.w.clone(), self.arena.wb.clone())
+                step0 = self.step_dev.clone() if self.augment is not None else None
                 self._enqueue_step()
                 torch.cuda.synchronize()
                 self.arena.w.copy_(saved[0]); self.arena.wb.copy_(saved[1])
+                if step0 is not None:
+                    self.step_dev.copy_(step0)
                 self.refresh_derived()
                 gr = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(gr):

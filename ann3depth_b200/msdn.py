@@ -43,8 +43,10 @@ class MSDNNet:
 
     def __init__(self, ctx: ops.Context, batch: int, in_hw=(480, 640), depth_hw=(55, 73), train=True,
                  beta2=ADAM_BETA2_REFERENCE, impl=L.IMPL_AUTO, dropout_seed=2, comm=None, grad_dtype=torch.float32,
-                 overlap=True, fuse_dense_adam=True, dtype="bf16"):
+                 overlap=True, fuse_dense_adam=True, dtype="bf16", augment=None, augment_seed=3):
         self.ctx, self.B, self.train, self.beta2, self.impl = ctx, batch, train, beta2, impl
+        if augment is not None and not train:
+            raise ValueError("augment is a training option: an inference net (train=False) sees its inputs unchanged")
         # dtype = "bf16" (default): BF16 storage of activations / activation gradients / the weight mirror, tcgen05
         # kind::f16.  dtype = "tf32": everything stays float32 in memory -- the reference's own storage type
         # (src/models.py:211-251) -- and the contractions run on tcgen05 kind::tf32 (north star: 1e-4 forward agreement).
@@ -87,6 +89,16 @@ class MSDNNet:
         self.depths = z(B, depth_hw[0], depth_hw[1], 1, **f32)
         self.keep_mask = torch.ones(B, 4096, dtype=torch.uint8, device=self.dev)
         self.external_mask = False
+        # training-time augmentation (augment.Augment, beyond the reference): one transform per image and step, drawn on
+        # the device from (seed, step_dev, image) and applied by the resizes that open the step.  Each data-parallel
+        # rank draws with its own seed (its batch differs anyway).
+        self.augment = augment
+        self.aug_params = self.aug_desc = None
+        self.external_aug = False
+        if augment is not None:
+            self.aug_desc = augment.desc()
+            self.augment_seed = augment_seed + (comm.rank if comm is not None else 0)
+            self.aug_params = torch.zeros(B, L.AUG_PARAMS, dtype=torch.float32, device=self.dev)
         # ---- forward activations
         # resized image in space-to-depth(4) layout: 4x4 pixel blocks -> 48 channels (+16 zero) = 128-byte pixels.
         # Both first layers are 3x3 stride-1 convolutions on it (coarse 11x11 s4; fine 9x9 s2 + pool = 11x11 s4).
@@ -199,6 +211,30 @@ class MSDNNet:
         self.keep_mask.copy_(mask.to(torch.uint8))
         self.external_mask = True
 
+    def set_augment_params(self, params):
+        """Parity hook: use explicit augmentation parameters [B,16] (include/a3d.h A3D_AUG_*) instead of the device
+        draw."""
+        if self.augment is None:
+            raise ValueError("set_augment_params needs a net built with augment=Augment(...)")
+        self.aug_params.copy_(params.to(torch.float32))
+        self.external_aug = True
+
+    def _augment_draw(self):
+        if not self.external_aug:
+            self.ctx.augment_draw(self.aug_desc, self.aug_params, self.augment_seed, self.step_dev)
+
+    def _resize_image(self):
+        if self.augment is not None:
+            self.ctx.resize_affine_tf1_s2d(self.images, IN_H, IN_W, 4, self.aug_params, out=self.img4)
+        else:
+            self.ctx.resize_bilinear_tf1_s2d(self.images, IN_H, IN_W, 4, out=self.img4)
+
+    def _resize_target(self):
+        if self.augment is not None:
+            self.ctx.resize_affine_tf1(self.depths, OUT_H, OUT_W, self.aug_params, depth=True, out=self.tar)
+        else:
+            self.ctx.resize_bilinear_tf1(self.depths, OUT_H, OUT_W, out=self.tar)
+
     # ------------------------------------------------------------------ forward
     def forward(self):
         """src/models.py:281-290.  Reads self.images / self.depths, fills self.coarse / self.fine / losses."""
@@ -211,8 +247,10 @@ class MSDNNet:
     def _forward(self):
         c, B = self.ctx, self.B
         K = "/kernel"
-        c.resize_bilinear_tf1_s2d(self.images, IN_H, IN_W, 4, out=self.img4)
-        c.resize_bilinear_tf1(self.depths, OUT_H, OUT_W, out=self.tar)
+        if self.augment is not None:
+            self._augment_draw()
+        self._resize_image()
+        self._resize_target()
         # coarse (src/models.py:208-236)
         n = "coarse/conv/conv2d_"
         c.conv2d_fwd(self.d_c0, self.img4, self.w(n + "0" + K), self.bias(n + "0"), relu=True, out=self.c0)
@@ -416,12 +454,18 @@ class MSDNNet:
         n0 = "coarse/conv/conv2d_"
         prep = os.environ.get("A3D_DGRAD_PREPARE", "1") != "0"
         e_start = mark(s0)
+        e_draw = None
+        if self.augment is not None:             # the transform both resizes apply
+            self._augment_draw()
+            e_draw = mark(s0)
         for side in (s2, s3):                 # every side stream forks from the step's start (a stream that happens to
             if side is not s0:                # get no work in some mode must still be part of the capture to be joined)
                 side.wait_event(e_start)
         with torch.cuda.stream(s1):
             s1.wait_event(e_start)
-            c.resize_bilinear_tf1(self.depths, OUT_H, OUT_W, out=self.tar)
+            if e_draw is not None:
+                s1.wait_event(e_draw)
+            self._resize_target()
             if not self.external_mask:
                 c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
             e_aux = mark(s1)
@@ -436,7 +480,7 @@ class MSDNNet:
                     c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K), out=self._wflip[i])
             e_flip = mark(s1)
         # ---- main: preprocessing
-        c.resize_bilinear_tf1_s2d(self.images, IN_H, IN_W, 4, out=self.img4)
+        self._resize_image()
         c.stamp("resize done")
         e_img = mark(s0)
         # ---- fine stream, part 1: first conv + pool need only the image

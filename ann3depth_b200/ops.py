@@ -129,6 +129,33 @@ class Context:
                                                      out.shape[-1], _stream()), "resize_s2d")
         return out
 
+    # ------------------------------------------------------------------ augmentation (include/a3d.h a3d_augment_desc)
+    def augment_draw(self, desc, params, seed, counter_dev=None):
+        """params [B, 16] float32 <- one random transform per image from (seed, *counter_dev, image index)."""
+        assert params.dtype == torch.float32 and params.shape[-1] == L.AUG_PARAMS and params.is_contiguous()
+        L.check(self.lib.a3d_augment_draw(self.h, C.byref(desc), params.shape[0], seed & (2 ** 64 - 1),
+                                          _ptr(counter_dev), _ptr(params), _stream()), "augment_draw")
+        return params
+
+    def resize_affine_tf1_s2d(self, src, OH, OW, s, params, out):
+        """Augmented resize + space-to-depth(s): src f32 or uint8 [B, H, W, 3], out bf16 or f32 [B, OH/s, OW/s, dstC]."""
+        B, H, W, Cc = src.shape
+        sd = L.A3D_U8 if src.dtype == torch.uint8 else L.A3D_F32
+        dd = L.A3D_F32 if out.dtype == torch.float32 else L.A3D_BF16
+        L.check(self.lib.a3d_resize_affine_tf1_s2d(self.h, _ptr(src), sd, B, H, W, Cc, _ptr(out), dd, OH, OW, s,
+                                                   out.shape[-1], _ptr(params), _stream()), "resize_affine_s2d")
+        return out
+
+    def resize_affine_tf1(self, src, OH, OW, params, depth, out=None):
+        """Augmented resize, f32 NHWC; depth=True: values / s (targets), False: values * c_rgb (images)."""
+        B, H, W, Cc = src.shape
+        if out is None:
+            out = torch.empty(B, OH, OW, Cc, dtype=torch.float32, device=src.device)
+        mode = L.AUG_VALUE_DEPTH if depth else L.AUG_VALUE_COLOR
+        L.check(self.lib.a3d_resize_affine_tf1(self.h, _ptr(src), B, H, W, Cc, _ptr(out), OH, OW, _ptr(params), mode,
+                                               _stream()), "resize_affine")
+        return out
+
     def conv2d_pool4_fwd(self, d, x, w, bias, relu=True, out=None, idx=None):
         """conv + bias + ReLU + 2x2 max-pool as one GEMM over the pool-embedded filter (K = 4 x 64)."""
         if out is None:

@@ -374,6 +374,57 @@ int a3d_window_scatter_sum(a3d_ctx*, const uint16_t* g_out, int B, int Hs, int W
 int a3d_depth_metrics(a3d_ctx*, const float* pred, int B, int ph, int pw, const float* gt, int gh, int gw,
                       float min_depth, float max_depth, int scale_mode, double* sums, float* scale, void* stream);
 
+/* ---- training-time augmentation (Eigen et al. 2014, section 3.3), beyond the reference (it has none) ------------------
+ * Every image of a batch gets one random transform, shared by the image and its depth target:
+ *   output pixel (oy, ox) of an OH x OW output sits at the TF1 legacy position (u, v) = (ox*W/OW, oy*H/OH) (tf1_coord);
+ *   p = (u/W, v/H); T(p) = c + R(theta) F (p - 1/2) f/s = M p + m (M, m: the normalised 2x3 matrix below), with
+ *   R(theta) a rotation in the pixel space of a frame of height/width `aspect`, F = diag(+-1, 1) the horizontal flip,
+ *   f the crop fraction, s the scale, c the crop centre;
+ *   the source is sampled at T(p) * (W, H), clamped to [0, W-1] x [0, H-1] (border replicated), with TF1 bilinear.
+ * Each tensor applies the transform in its own pixel units, so a 480x640 image and a 55x73 depth map see one geometry.
+ * Values: images are multiplied per channel by c_rgb after interpolation (one rounding to the storage type); depths by
+ * 1/s.  With identity parameters both resize entry points write exactly what the plain TF1 resizes write. */
+typedef struct a3d_augment_desc {
+  float scale_lo, scale_hi;     /* s ~ U[scale_lo, scale_hi], > 0 */
+  float max_rotation_deg;       /* theta ~ U[-max, max] degrees */
+  float crop_fraction;          /* f in (0, 1]: the window spans f/s of the frame */
+  float flip_prob;              /* P(horizontal flip) */
+  float color_lo, color_hi;     /* c_rgb ~ U[color_lo, color_hi]^3 */
+  float aspect;                 /* height / width of the frame the rotation is a rotation of (0.75 for 480x640) */
+} a3d_augment_desc;
+/* params [B][A3D_AUG_PARAMS] float32, one row per image */
+#define A3D_AUG_M00       0    /* T_x(p) = M00 p_x + M01 p_y + M02 */
+#define A3D_AUG_M01       1
+#define A3D_AUG_M02       2
+#define A3D_AUG_M10       3    /* T_y(p) = M10 p_x + M11 p_y + M12 */
+#define A3D_AUG_M11       4
+#define A3D_AUG_M12       5
+#define A3D_AUG_COLOR     6    /* c_r, c_g, c_b at 6, 7, 8 */
+#define A3D_AUG_INV_SCALE 9    /* 1/s */
+#define A3D_AUG_SCALE    10    /* raw draws, for inspection: s, theta (degrees), flip (0/1), c_x, c_y, f */
+#define A3D_AUG_THETA    11
+#define A3D_AUG_FLIP     12
+#define A3D_AUG_CX       13
+#define A3D_AUG_CY       14
+#define A3D_AUG_CROP     15
+#define A3D_AUG_PARAMS   16
+#define A3D_AUG_VALUE_COLOR 0  /* a3d_resize_affine_tf1 value rule: v * c_rgb[c] (C <= 3) */
+#define A3D_AUG_VALUE_DEPTH 1  /* v / s */
+#define A3D_U8 2               /* source dtype of a3d_resize_affine_tf1_s2d: 8-bit pixels, read as pixel / 255 */
+/* Draws params[b] from a splitmix64 hash of (seed, *counter_dev, b) in float64 (ranges of `desc`), on the device: a
+ * replayed CUDA graph draws fresh parameters whenever *counter_dev (the global step) moves.  counter_dev may be NULL
+ * (counter 0).  c_x, c_y ~ 1/2 + U[-1, 1] (1 - f/s)/2: the unrotated window lies inside the frame. */
+int a3d_augment_draw(a3d_ctx*, const a3d_augment_desc* desc, int B, uint64_t seed, const int64_t* counter_dev,
+                     float* params, void* stream);
+/* The MSDN image path: augmented resize written in the space-to-depth(s) layout of a3d_resize_bilinear_tf1_s2d.
+ * src_dtype A3D_F32 or A3D_U8 (pixel / 255); dst_dtype A3D_BF16 or A3D_F32.  C == 3, s == 4, dstC % 4 == 0, >= 48
+ * (channels [48, dstC) zero), dst 16-byte aligned.  Colour value rule. */
+int a3d_resize_affine_tf1_s2d(a3d_ctx*, const void* src, int src_dtype, int B, int H, int W, int C, void* dst,
+                              int dst_dtype, int OH, int OW, int s, int dstC, const float* params, void* stream);
+/* Generic NHWC: src f32 [B,H,W,C] -> dst f32 [B,OH,OW,C], C <= 4; value_mode A3D_AUG_VALUE_COLOR | _DEPTH. */
+int a3d_resize_affine_tf1(a3d_ctx*, const float* src, int B, int H, int W, int C, float* dst, int OH, int OW,
+                          const float* params, int value_mode, void* stream);
+
 /* ---- data parallelism (replaces the PS/gRPC replication of src/ann3depth.py:78-92) ---------- */
 /* NCCL is dlopen()ed at first use (path = NULL -> "libnccl.so.2"). */
 int a3d_comm_unique_id(const char* nccl_path, void* id128);              /* 128-byte ncclUniqueId */
