@@ -12,6 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("A3D_LIB") or os.path.join(_HERE, "liba3d.so")     # A3D_LIB: alternate build (experiments)
 
 A3D_F32, A3D_BF16 = 0, 1
+A3D_E4M3 = 3                          # E4M3 codes: the FP8 inference mode
 A3D_ENOTSUP = -5
 IMPL_AUTO, IMPL_SIMT, IMPL_TC = 0, 1, 2
 EPI_RELU, EPI_SIGMOID = 1, 2
@@ -164,6 +165,14 @@ SIGNATURES = {
     "a3d_augment_draw": (_i, [_vp, C.POINTER(AugmentDesc), _i, C.c_uint64, _vp, _vp, _vp]),
     "a3d_resize_affine_tf1_s2d": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "a3d_resize_affine_tf1": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _vp, _i, _vp]),
+    "a3d_quantize_rows_e4m3": (_i, [_vp, _vp, _i, _i, C.c_longlong, _vp, _vp, _vp]),
+    "a3d_quantize_ws_bytes_e4m3": (_sz, [_i, _sz]),
+    "a3d_quantize_e4m3": (_i, [_vp, _vp, _i, _sz, _vp, _vp, _vp, _sz, _vp]),
+    "a3d_maxpool2x2_quantize_e4m3": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _sz, _vp]),
+    "a3d_resize_bilinear_tf1_s2d_e4m3": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _vp]),
+    "a3d_conv2d_fwd_fp8": (_i, [_vp, C.POINTER(ConvDesc), _vp, _vp, _vp, _vp, _vp, _vp, _i, _u, _vp, _sz, _vp]),
+    "a3d_conv2d_pool4_fwd_fp8": (_i, [_vp, C.POINTER(ConvDesc), _vp, _vp, _vp, _vp, _vp, _vp, _u, _vp]),
+    "a3d_dense_fwd_fp8": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _u, _vp]),
     "a3d_comm_unique_id": (_i, [C.c_char_p, _vp]),
     "a3d_comm_init": (_i, [_vp, C.c_char_p, _vp, _i, _i]),
     "a3d_comm_destroy": (_i, [_vp]),
@@ -174,6 +183,7 @@ SIGNATURES = {
     "a3d_debug_tc_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "a3d_debug_tc_gemm_v": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "a3d_debug_tc_gemm_tf32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "a3d_debug_tc_gemm_fp8": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _vp]),
 }
 
 _lib = None

@@ -169,6 +169,16 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// The same with E4M3 inputs (one byte per element, 32 per UMMA K step), f32 accumulate.
+__device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                        uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}\n"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive on an mbarrier once all previously issued UMMAs of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -213,6 +223,17 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn_ma
 __host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N, int a_mn_major, int b_mn_major) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// kind::f8f6f4: A/B format 0 (E4M3), F32 accumulate
+__host__ __device__ constexpr uint32_t make_idesc_f8f6f4(int M, int N, int a_mn_major, int b_mn_major) {
+  return (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
+         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// Two f32 -> two E4M3 codes (round to nearest even, saturating at +-448): lo lands in the low byte
+__device__ __forceinline__ uint16_t cvt_e4m3x2(float lo, float hi) {
+  uint16_t r;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
+  return r;
 }
 
 }  // namespace ptx

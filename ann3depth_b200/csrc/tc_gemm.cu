@@ -23,11 +23,12 @@ CUtensorMapSwizzle swizzle_for(int row_bytes) {
                            : CU_TENSOR_MAP_SWIZZLE_NONE;
 }
 
-// Operand element type of a tensor map: 2 = bf16; 4 = f32 read as TFLOAT32 -- the TMA unit rounds the low 13 mantissa
+// Operand element type of a tensor map: 2 = bf16; 1 = E4M3; 4 = f32 read as TFLOAT32 -- the TMA unit rounds the low 13 mantissa
 // bits away (round to nearest) on the way into shared memory, so kind::tf32 MMAs see properly rounded TF32 values
 // instead of truncated ones.  A3D_TF32_TMAP=0 selects plain FLOAT32 maps (the MMA then truncates).
 CUtensorMapDataType tmap_dtype(int elt) {
   if (elt == 2) return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  if (elt == 1) return CU_TENSOR_MAP_DATA_TYPE_UINT8;       // E4M3 codes: the TMA unit only moves the bytes
   static int v = -1;
   if (v < 0) { const char* e = getenv("A3D_TF32_TMAP"); v = e ? atoi(e) : 1; }
   return v ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
@@ -1267,4 +1268,202 @@ extern "C" int a3d_debug_tc_gemm_tf32(a3d_ctx* ctx, const float* A, const float*
 #undef A3D_T32
   a3d_set_error("debug gemm tf32: no kernel for BN=%d KCB=%d a_mn=%d b_mn=%d", bn, kcb, a_mn, b_mn);
   return A3D_ENOTSUP;
+}
+
+// =====================================================================================================================
+// FP8 inference mode (fp8.cu): E4M3 operands, tcgen05.mma kind::f8f6f4, f32 accumulation.  Every operand is K-major with
+// 128- or 64-byte rows per stage (SWIZZLE_128B / 64B); the epilogue multiplies each accumulator by its row and column
+// scales (tc::Params::rs / cs) before bias and activation.  Split-K partial sums are scaled before they are added, which
+// is the same linear map.  Own tuner kinds (6 conv, 7 pool-fused conv, 8 dense), so no bf16 choice is ever reused.
+// =====================================================================================================================
+namespace {
+template <int BN, int KCB, int MS = A3D_MIN_STAGES>
+using CfgF8 = tc::Cfg<BN, KCB, false, false, 64, MS, false, 128, 1>;
+
+int launch_f8(a3d_ctx* ctx, int bn, int kcb, int deep, const CUtensorMap& tmA, const CUtensorMap& tmB, const tc::Params& p,
+              int splits, cudaStream_t st) {
+#define A3D_F8(BN, KCB) \
+  if (bn == BN && kcb == KCB && !deep) return launch_cfg<CfgF8<BN, KCB>>(ctx, tmA, tmB, p, splits, st);
+  A3D_F8(32, 128) A3D_F8(64, 128) A3D_F8(96, 128) A3D_F8(128, 128) A3D_F8(192, 128) A3D_F8(256, 128)
+  A3D_F8(32, 64) A3D_F8(64, 64) A3D_F8(96, 64) A3D_F8(128, 64) A3D_F8(192, 64) A3D_F8(256, 64)
+#undef A3D_F8
+#define A3D_F8D(BN) \
+  if (bn == BN && kcb == 128 && deep) return launch_cfg<CfgF8<BN, 128, 3>>(ctx, tmA, tmB, p, splits, st);
+  A3D_F8D(64) A3D_F8D(96) A3D_F8D(128) A3D_F8D(192) A3D_F8D(256)
+#undef A3D_F8D
+  a3d_set_error("fp8 gemm: no kernel for BN=%d KCB=%d deep=%d", bn, kcb, deep);
+  return A3D_ENOTSUP;
+}
+}  // namespace
+
+// y = act(conv(x, w) * x_scale[image] * w_scale[filter] + bias); pool4: the fused 2x2 max-pool of a3d_tc_conv_fwd (K = 256
+// = 4 window positions x 64 filters), the column scales applied before the max.  ws: [N*P*Q][K] f32 split-K accumulator.
+int a3d_tc_conv_fwd_fp8(a3d_ctx* ctx, const a3d_conv_desc* d, const uint8_t* x, const float* x_scale, const uint8_t* w,
+                        const float* w_scale, const float* bias, void* y, int y_dtype, unsigned flags, void* ws,
+                        size_t ws_bytes, cudaStream_t st, int pool4) {
+  if (d->C % 64 || d->stride_h > 8 || d->stride_w > 8 || d->R > 256 || d->S > 256 || d->dil_w > 1 ||
+      (d->pix_pitch && d->pix_pitch != d->C)) {
+    a3d_set_error("fp8 conv fwd: needs C %% 64 == 0 (64- or 128-byte pixels), no dil_w / pix_pitch views (C=%d)", d->C);
+    return A3D_ENOTSUP;
+  }
+  const int kc = d->C % 128 == 0 ? 128 : 64;        // channels = bytes per TMA load
+  const int cblocks = d->C / kc;
+  const int num_kb = d->R * d->S * cblocks;
+  const long long M = (long long)d->N * d->P * d->Q;
+  const long long J = (long long)d->R * d->S * d->C;
+  CUtensorMap tmA;
+  int rc = make_tmap_im2col(ctx, &tmA, x, d->N, d->H, d->W, d->C, -d->pad_t, -d->pad_l, d->P, d->Q, d->stride_h,
+                            d->stride_w, kc, 128, 1);
+  if (rc) return rc;
+  tc::Params p{};
+  p.M = (int)M; p.N = d->K; p.num_kb = num_kb; p.kb_per_split = num_kb; p.a_mode = tc::A_IM2COL;
+  p.PQ = d->P * d->Q; p.Q = d->Q; p.sh = d->stride_h; p.sw = d->stride_w; p.lower_h = -d->pad_t; p.lower_w = -d->pad_l;
+  p.S = d->S; p.cblocks = cblocks;
+  p.rs = x_scale; p.rs_div = p.PQ; p.cs = w_scale;
+  if (pool4) {
+    if (d->K != 256 || y_dtype != A3D_BF16 || d->ldy % 8 || (reinterpret_cast<uintptr_t>(y) & 15)) {
+      a3d_set_error("fp8 conv pool4 fwd: needs K == 256 (4 x 64) and a bf16 output with 16-byte aligned rows");
+      return A3D_ENOTSUP;
+    }
+    CUtensorMap tmB;
+    rc = make_tmap_2d(ctx, &tmB, w, 256, J, J, kc, 256, 1);
+    if (rc) return rc;
+    p.epi = tc::EPI_POOL4_BF16; p.out = y; p.ldo = d->ldy; p.bias = bias; p.flags = flags;
+    auto run = [&](int c) -> int {
+      if (kc == 64) return c ? launch_cfg<CfgF8<256, 64, 3>>(ctx, tmA, tmB, p, 1, st) : launch_cfg<CfgF8<256, 64>>(ctx, tmA, tmB, p, 1, st);
+      return c ? launch_cfg<CfgF8<256, 128, 3>>(ctx, tmA, tmB, p, 1, st) : launch_cfg<CfgF8<256, 128>>(ctx, tmA, tmB, p, 1, st);
+    };
+    TuneKey key{};
+    const int kv[16] = {7, d->N, d->H, d->W, d->C, d->K, d->R, d->S, d->stride_h, d->stride_w, d->pad_t, d->pad_l,
+                        d->P, d->Q, d->ldy};
+    memcpy(key.v, kv, sizeof(kv));
+    return run(autotune(key, 2, run, st));
+  }
+  const bool can_split = ws && ws_bytes >= (size_t)M * d->K * sizeof(float);
+  auto launch = [&](int bn, int splits, int deep) -> int {
+    CUtensorMap tmB;
+    int r = make_tmap_2d(ctx, &tmB, w, d->K, J, J, kc, bn, 1);
+    if (r) return r;
+    tc::Params q = p;
+    if (!can_split) splits = 1;
+    q.kb_per_split = ceil_div(num_kb, splits);
+    splits = ceil_div(num_kb, q.kb_per_split);
+    if (splits == 1) {
+      q.epi = y_dtype == A3D_F32 ? tc::EPI_ROW_F32 : tc::EPI_ROW_BF16;
+      q.out = y; q.ldo = d->ldy; q.bias = bias; q.flags = flags; q.atomic = 0;
+      return launch_f8(ctx, bn, kc, deep, tmA, tmB, q, 1, st);
+    }
+    A3D_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)M * d->K * sizeof(float), st));
+    q.epi = tc::EPI_ROW_F32; q.out = ws; q.ldo = d->K; q.bias = nullptr; q.flags = 0; q.atomic = 1;
+    r = launch_f8(ctx, bn, kc, deep, tmA, tmB, q, splits, st);
+    if (r) return r;
+    return finish(ctx, reinterpret_cast<const float*>(ws), bias, nullptr, 0.f, y, y_dtype == A3D_F32, (size_t)M, d->K,
+                  d->ldy, flags, st);
+  };
+  // candidate 0 = the bf16 heuristic's tile; then every width that pads K by at most a third, unsplit and with ~1-2
+  // waves of split-K, with the default and (128-byte rows) the deeper ring
+  struct Cand { int bn, splits, deep; };
+  Cand cand[48];
+  int nc = 0;
+  auto tiles_of = [&](int bn) { return (int)(ceil_div(M, 128) * ceil_div(d->K, bn)); };
+  {
+    const int bn0 = pick_bn(d->K) < 32 ? 32 : pick_bn(d->K);
+    cand[nc++] = {bn0, can_split ? pick_splits(ctx, tiles_of(bn0), num_kb, 8) : 1, 0};
+  }
+  static const int widths[] = {32, 64, 96, 128, 192, 256};
+  for (int i = 0; i < 6; ++i) {
+    const int bn = widths[i];
+    if (ceil_div(d->K, bn) * bn > d->K + d->K / 3 + 15) continue;
+    const int tiles = tiles_of(bn);
+    const int sopts[3] = {1, ctx->sm_count / tiles, 2 * ctx->sm_count / tiles};
+    for (int t = 0; t < 3; ++t) {
+      int sp = sopts[t];
+      const int max_s = num_kb / 8 > 0 ? num_kb / 8 : 1;
+      if (sp > max_s) sp = max_s;
+      if (sp < 1 || !can_split) sp = 1;
+      for (int deep = 0; deep < 2; ++deep) {
+        if (deep && (kc != 128 || bn == 32)) continue;
+        bool dup = false;
+        for (int k = 0; k < nc; ++k) dup |= cand[k].bn == bn && cand[k].splits == sp && cand[k].deep == deep;
+        if (!dup && nc < 48) cand[nc++] = {bn, sp, deep};
+      }
+    }
+  }
+  if (const char* force = getenv("A3D_FP8_CONV_FORCE")) {            // "bn,splits,deep": tests and A/B runs
+    int fbn = 0, fsp = 1, fd = 0;
+    if (sscanf(force, "%d,%d,%d", &fbn, &fsp, &fd) >= 1 && fbn > 0) return launch(fbn, fsp, fd);
+  }
+  TuneKey key{};
+  const int kv[16] = {6, d->N, d->H, d->W, d->C, d->K, d->R, d->S, d->stride_h, d->stride_w, d->pad_t, d->pad_l,
+                      d->P, d->Q, d->ldy, y_dtype * 2 + (can_split ? 1 : 0)};
+  memcpy(key.v, kv, sizeof(kv));
+  const int best = autotune(key, nc, [&](int c) { return launch(cand[c].bn, cand[c].splits, cand[c].deep); }, st);
+  return launch(cand[best].bn, cand[best].splits, cand[best].deep);
+}
+
+// dense forward, batch M <= 256 as the UMMA N dimension (as a3d_tc_dense_fwd): the weights [N][K] stream once as the
+// 128-row operand; acc_ws [M][N] f32 receives the scaled split-K sums, `finish` adds bias and activation.
+int a3d_tc_dense_fwd_fp8(a3d_ctx* ctx, const uint8_t* x, int ldx, const float* x_scale, const uint8_t* w,
+                         const float* w_scale, const float* bias, void* y, int y_dtype, float* acc_ws, int M, int N, int K,
+                         unsigned flags, cudaStream_t st) {
+  if (K % 128 || ldx % 16 || M > 256 || !acc_ws) {
+    a3d_set_error("fp8 dense fwd: needs K %% 128 == 0, ldx %% 16 == 0, batch <= 256, a workspace (K=%d M=%d)", K, M);
+    return A3D_ENOTSUP;
+  }
+  const int bn = M <= 32 ? 32 : M <= 64 ? 64 : M <= 128 ? 128 : 256;
+  CUtensorMap tmA, tmB;
+  int rc = make_tmap_2d(ctx, &tmA, w, N, K, K, 128, 128, 1);
+  if (rc) return rc;
+  rc = make_tmap_2d(ctx, &tmB, x, M, K, ldx, 128, bn, 1);
+  if (rc) return rc;
+  tc::Params p{};
+  p.M = N; p.N = M; p.num_kb = K / 128; p.a_mode = tc::A_TILED;
+  p.rs = w_scale; p.rs_div = 1; p.cs = x_scale;
+  p.epi = tc::EPI_COL_F32; p.out = acc_ws; p.ldo = N; p.atomic = 1;
+  const int tiles = ceil_div(N, 128);
+  int splits0 = pick_splits(ctx, tiles, p.num_kb, 4);
+  if (splits0 * tiles < 2 * ctx->sm_count && p.num_kb / (splits0 * 2) >= 4) splits0 *= 2;
+  auto launch = [&](int splits) -> int {          // splits >= 1000: interleaved k-blocks (Params::kb_interleave)
+    tc::Params q = p;
+    q.kb_interleave = splits >= 1000;
+    splits %= 1000;
+    q.kb_per_split = ceil_div(q.num_kb, splits);
+    splits = ceil_div(q.num_kb, q.kb_per_split);
+    A3D_CHECK_CUDA(cudaMemsetAsync(acc_ws, 0, (size_t)M * N * sizeof(float), st));
+    int r = launch_f8(ctx, bn, 128, 0, tmA, tmB, q, splits, st);
+    if (r) return r;
+    return finish(ctx, acc_ws, bias, nullptr, 0.f, y, y_dtype == A3D_F32, (size_t)M, N, N, flags, st);
+  };
+  int cand[24];
+  int nc = split_candidates(ctx, tiles, p.num_kb, splits0, cand);
+  for (int i = 0, n0 = nc; i < n0; ++i)
+    if (cand[i] > 1) cand[nc++] = 1000 + cand[i];
+  if (const char* force = getenv("A3D_FP8_DENSE_FORCE")) return launch(atoi(force));
+  TuneKey key{};
+  const int kv[16] = {8, M, N, K, ldx, y_dtype, (int)flags};
+  memcpy(key.v, kv, sizeof(kv));
+  return launch(cand[autotune(key, nc, [&](int c) { return launch(cand[c]); }, st)]);
+}
+
+// ---- E4M3 (kind::f8f6f4) engine test hook: D[M][N] (f32) = A * B^T with A [M][K], B [N][K] E4M3 codes, K-major,
+// kcb = 128 or 64 bytes of K per stage; row / column scales when rs / cs are given (rs_div rows share one row scale).
+extern "C" int a3d_debug_tc_gemm_fp8(a3d_ctx* ctx, const uint8_t* A, const uint8_t* B, float* D, int M, int N, int K, int bn,
+                                     int kcb, int splits, const float* rs, int rs_div, const float* cs, void* stream) {
+  A3D_REQUIRE(ctx && A && B && D && (!rs == !cs) && rs_div >= 1, "debug gemm fp8: bad argument");
+  A3D_REQUIRE((kcb == 128 || kcb == 64) && K % kcb == 0, "debug gemm fp8: kcb 128 or 64 and K %% kcb == 0");
+  cudaStream_t st = as_stream(stream);
+  CUtensorMap tmA, tmB;
+  int rc = make_tmap_2d(ctx, &tmA, A, M, K, K, kcb, 128, 1);
+  if (rc) return rc;
+  rc = make_tmap_2d(ctx, &tmB, B, N, K, K, kcb, bn, 1);
+  if (rc) return rc;
+  tc::Params p{};
+  p.M = M; p.N = N; p.num_kb = K / kcb; p.a_mode = tc::A_TILED;
+  p.rs = rs; p.rs_div = rs_div; p.cs = cs;
+  if (splits < 1) splits = 1;
+  p.kb_per_split = ceil_div(p.num_kb, splits);
+  splits = ceil_div(p.num_kb, p.kb_per_split);
+  p.epi = tc::EPI_ROW_F32; p.out = D; p.ldo = N; p.atomic = splits > 1;
+  if (splits > 1) A3D_CHECK_CUDA(cudaMemsetAsync(D, 0, (size_t)M * N * sizeof(float), st));
+  return launch_f8(ctx, bn, kcb, 0, tmA, tmB, p, splits, st);
 }

@@ -75,9 +75,16 @@ struct Params {
   unsigned flags;
   int atomic;               // accumulate with atomicAdd (split-K)
   uint8_t* pool_idx;        // EPI_POOL4_BF16: routing record (nullable)
+  // E4M3 operands (ELT = 1): acc[row][col] * rs[row / rs_div] * cs[col] before bias / activation (rs == nullptr: none).
+  // Convolutions: rs = per-image activation scales (rs_div = P*Q rows per image), cs = per-filter weight scales; dense
+  // layers (weights are the row operand): rs = weight scales (rs_div = 1), cs = per-image activation scales.
+  const float* rs = nullptr;
+  int rs_div = 1;
+  const float* cs = nullptr;
 };
 
-// ELT_ = operand element size in bytes: 2 = bf16 (kind::f16), 4 = f32 consumed as TF32 (kind::tf32).  All shared-memory
+// ELT_ = operand element size in bytes: 2 = bf16 (kind::f16), 4 = f32 consumed as TF32 (kind::tf32), 1 = E4M3
+// (kind::f8f6f4; K-major swizzled operands and 128-row tiles only, 32 elements per UMMA K step).  All shared-memory
 // geometry below is in BYTES, so the two differ only in elements per row: a UMMA K step is always 32 bytes (16 bf16 /
 // 8 tf32), an MN-major row always 128 bytes (64 bf16 / 32 tf32 elements), and an MN-major stage holds 128 / ELT K-rows.
 template <int BN_, int KCB_, bool A_MN_, bool B_MN_, int B_BW_ = 64, int MIN_STAGES_ = A3D_MIN_STAGES, bool ADAM_ = false,
@@ -88,7 +95,9 @@ struct Cfg {
   static constexpr int A_MN_BLOCKS = ELT_;                // MN-major A: 128-byte-wide blocks per 128 rows (2 / 4)
   static constexpr int A_MN_BLK_BYTES = KROWS * 128;      // one block: KROWS rows x 128 bytes (8 KB / 4 KB)
   static constexpr int A_MN_BLK_ELEMS = 128 / ELT_;       // M elements per block (64 / 32)
-  static_assert(ELT_ == 2 || (ELT_ == 4 && KCB_ != 16 && !ADAM_ && BM_ == 128), "tf32: swizzled operands, plain epilogues");
+  static_assert(ELT_ == 2 || ((ELT_ == 4 || ELT_ == 1) && KCB_ != 16 && !ADAM_ && BM_ == 128),
+                "tf32 / e4m3: swizzled operands, plain epilogues");
+  static_assert(ELT_ != 1 || (!A_MN_ && !B_MN_), "e4m3: K-major operands only");
   static_assert(ELT_ == 2 || !B_MN_ || B_BW_ == 32, "tf32 MN-major B: 128-byte rows only (32-byte-atom swizzle)");
   // BM = 256: the CTA owns TWO 128-row accumulators (TMEM columns [0,BN) and [BN,2BN)) that share every B stage:
   // operand traffic per FLOP drops from (128+BN) to (256+BN)/2 rows per k-block -- the 5x5 layers are bound by
@@ -122,6 +131,18 @@ struct Cfg {
   static_assert(B_BW_ * ELT_ == 128 || B_BW_ * ELT_ == 64 || B_BW_ * ELT_ == 32, "MN-major block width: 128/64/32-byte rows");
   static_assert(BN_ % 16 == 0 && BN_ >= 16 && BN_ <= 256, "UMMA N");
 };
+
+// E4M3 tiles: v[j] (row `row`, columns col0 + j) *= row scale x column scale (Params::rs / cs)
+template <class C, int NV>
+__device__ __forceinline__ void scale_acc(const Params& p, int row, int col0, float* v) {
+  if constexpr (C::ELT == 1) {
+    if (p.rs) {
+      const float r = row < p.M ? __ldg(p.rs + row / p.rs_div) : 0.f;
+#pragma unroll
+      for (int j = 0; j < NV; ++j) v[j] *= r * (col0 + j < p.N ? __ldg(p.cs + col0 + j) : 0.f);
+    }
+  }
+}
 
 template <class C>
 __global__ void __launch_bounds__(192, 2)
@@ -264,8 +285,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
     if (lane == 0) {
-      constexpr uint32_t idesc = C::ELT == 4 ? ptx::make_idesc_tf32(128, C::BN, C::A_MN ? 1 : 0, C::B_MN ? 1 : 0)
-                                             : ptx::make_idesc_bf16(128, C::BN, C::A_MN ? 1 : 0, C::B_MN ? 1 : 0);
+      constexpr uint32_t idesc = C::ELT == 4   ? ptx::make_idesc_tf32(128, C::BN, C::A_MN ? 1 : 0, C::B_MN ? 1 : 0)
+                                 : C::ELT == 1 ? ptx::make_idesc_f8f6f4(128, C::BN, 0, 0)
+                                               : ptx::make_idesc_bf16(128, C::BN, C::A_MN ? 1 : 0, C::B_MN ? 1 : 0);
       constexpr uint32_t k_layout =
           C::KCB == 128 ? ptx::LAYOUT_SW128 : C::KCB == 64 ? ptx::LAYOUT_SW64 : ptx::LAYOUT_SW32;
       for (int i = 0; i < nkb; ++i) {
@@ -294,7 +316,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const uint64_t b_desc = C::B_MN      ? ptx::make_smem_desc(sB, C::B_BLK_BYTES, b_mn_sbo, b_mn_layout)
                                 : C::CHUNKED ? ptx::make_smem_desc(sB, C::BN * 16, 128, ptx::LAYOUT_NONE)
                                              : ptx::make_smem_desc(sB, 16, 8 * C::KCB, k_layout);
-        // one UMMA covers 32 bytes of K: 16 bf16 / 8 tf32 elements.  K-major: 32 bytes along the swizzled row;
+        // one UMMA covers 32 bytes of K: 16 bf16 / 8 tf32 / 32 e4m3 elements.  K-major: 32 bytes along the swizzled row;
         // MN-major: 32 / ELT K-rows of 128 (A) or B_BW * ELT (B) bytes
         constexpr int KSTEP = 32 / C::ELT;
         constexpr uint32_t a_step = C::A_MN ? ((KSTEP * 128) >> 4) : C::CHUNKED ? ((2 * C::BM * 16) >> 4) : (32 >> 4);
@@ -305,6 +327,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           if constexpr (C::ELT == 4) {
             ptx::umma_tf32(tmem_base, a_desc + (uint64_t)(k * a_step), b_desc + (uint64_t)(k * b_step), idesc,
                            (uint32_t)((i | k) != 0));
+          } else if constexpr (C::ELT == 1) {
+            ptx::umma_f8(tmem_base, a_desc + (uint64_t)(k * a_step), b_desc + (uint64_t)(k * b_step), idesc,
+                         (uint32_t)((i | k) != 0));
           } else {
             ptx::umma_bf16(tmem_base, a_desc + (uint64_t)(k * a_step), b_desc + (uint64_t)(k * b_step), idesc,
                            (uint32_t)((i | k) != 0));
@@ -359,6 +384,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           float v[32];
 #pragma unroll
           for (int j = 0; j < 16; ++j) { v[j] = __uint_as_float(ra[j]); v[16 + j] = __uint_as_float(rb[j]); }
+          scale_acc<C, 32>(p, row, col0, v);
           if (p.bias) {
 #pragma unroll
             for (int j = 0; j < 32; ++j)
@@ -412,6 +438,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 #pragma unroll
             for (int j = 0; j < 16; ++j) { v[j] = __uint_as_float(ra[j]); v[16 + j] = __uint_as_float(rb[j]); }
             const int cbase = col0 + half * 32;
+            scale_acc<C, 32>(p, row, cbase, v);
             if (p.bias) {
 #pragma unroll
               for (int j = 0; j < 32; ++j)
@@ -447,6 +474,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const int row0 = m0 + quarter * 32;
         if (row0 < p.M) {
           const uint32_t srow = ptx::smem_u32(slab) + (uint32_t)lane * 128u;
+          float rsc = 1.f;                         // E4M3: row scale; the column scales apply before the max
+          if constexpr (C::ELT == 1) {
+            if (p.rs) rsc = row_ok ? __ldg(p.rs + row / p.rs_div) : 0.f;
+          }
 #pragma unroll 1
           for (int cc = 0; cc < 4; ++cc) {
             uint32_t r0[16], r1[16], r2[16], r3[16];
@@ -463,7 +494,16 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             for (int j = 0; j < 16; ++j) {
               float m = __uint_as_float(r0[j]);
               uint32_t g = 0;
-              const float a1 = __uint_as_float(r1[j]), a2 = __uint_as_float(r2[j]), a3 = __uint_as_float(r3[j]);
+              float a1 = __uint_as_float(r1[j]), a2 = __uint_as_float(r2[j]), a3 = __uint_as_float(r3[j]);
+              if constexpr (C::ELT == 1) {
+                if (p.rs) {
+                  const int c = cc * 16 + j;
+                  m *= rsc * __ldg(p.cs + c);
+                  a1 *= rsc * __ldg(p.cs + 64 + c);
+                  a2 *= rsc * __ldg(p.cs + 128 + c);
+                  a3 *= rsc * __ldg(p.cs + 192 + c);
+                }
+              }
               if (a1 > m) { m = a1; g = 1; }       // strict '>' keeps the FIRST arg-max (TF MaxPoolGrad)
               if (a2 > m) { m = a2; g = 2; }
               if (a3 > m) { m = a3; g = 3; }
@@ -505,6 +545,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       float v[16];
 #pragma unroll
       for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(r[j]);
+      scale_acc<C, 16>(p, row, col0, v);
       if (p.epi == EPI_COL_F32) {
         float* o = reinterpret_cast<float*>(p.out);
         if (row_ok) {

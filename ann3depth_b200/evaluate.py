@@ -10,11 +10,13 @@ averaged over the images with a valid pixel.  The defaults suit the reference's 
 relative depths k/255 (tools/data_tf_converter.py), so min_depth = 1e-3 excludes exactly the zeros.
 
     python -m ann3depth_b200.evaluate nyu --model msdn --ckptdir checkpoints --id run1 --batchsize 32 --datadir data
-                                          [--scale median] [--json metrics.json]
+                                          [--scale median] [--dtype fp8] [--json metrics.json]
 
 restores `<ckptdir>/<model>[_<id>]/model.ckpt` into the inference net and reads `<datadir>/<dataset>/test.tfrecords`
 once.  MSDN reports its two outputs `fine` (the reference's prediction) and `coarse`; DCNF its `output`.  Under
-`torchrun` the ranks evaluate disjoint shards of the file and the chief logs / writes the reduced result.
+`torchrun` the ranks evaluate disjoint shards of the file and the chief logs / writes the reduced result.  `--dtype fp8`
+evaluates MSDN in its FP8 inference mode (E4M3 products; include/a3d.h "FP8 inference"), so the metrics show what FP8
+costs on the user's own model.
 """
 from __future__ import annotations
 
@@ -135,8 +137,11 @@ def main(argv=None):
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("gloo")
+    if args.dtype == "fp8" and args.model != "msdn":
+        raise SystemExit(f"evaluate: {args.model.upper()} has no FP8 mode (--dtype fp8 runs MSDN only)")
     inp = data.inputs(args.datadir, args.dataset, args.batchsize, "test", epochs=1, shard=(rank, world))
-    op = getattr(models, args.model)(inp.images, inp.depths, train=False)
+    op = getattr(models, args.model)(inp.images, inp.depths, train=False,
+                                     **({"dtype": "fp8"} if args.dtype == "fp8" else {}))
     if not restore_checkpoint(op, ckptdir):
         raise SystemExit(f"evaluate: no checkpoint in {ckptdir}")
     meters = evaluate_split(op, inp, make_meters(op, op.net.ctx, args.scale, args.min_depth, args.max_depth))
@@ -145,7 +150,7 @@ def main(argv=None):
         m.reduce()
     results = {name: m.result() for name, m in meters.items()}
     first = next(iter(results.values()))
-    out = {"model": args.model, "global_step": op.global_step, "scale": args.scale, "images": first["images"],
+    out = {"model": args.model, "dtype": args.dtype, "global_step": op.global_step, "scale": args.scale, "images": first["images"],
            "pixels": first["pixels"], "metrics": {name: {k: r[k] for k in ("nonfinite",) + METRICS}
                                                   for name, r in results.items()}}
     if rank == 0:
@@ -172,6 +177,9 @@ def parse_args(argv=None):
     p.add_argument("--scale", default="none", choices=("none", "median"), help="Median-scale each prediction first.")
     p.add_argument("--min-depth", default=1e-3, type=float, help="Valid pixels: min_depth < gt <= max_depth.")
     p.add_argument("--max-depth", default=1.0, type=float)
+    p.add_argument("--dtype", default="bf16", choices=("bf16", "fp8"),
+                   help="Inference precision: bf16, or fp8 (MSDN only: E4M3 products with per-channel weight and "
+                        "per-image activation scales).")
     p.add_argument("--json", default="", help="Write the result to this file.")
     return p.parse_args(argv)
 

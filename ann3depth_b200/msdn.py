@@ -45,6 +45,17 @@ class MSDNNet:
                  beta2=ADAM_BETA2_REFERENCE, impl=L.IMPL_AUTO, dropout_seed=2, comm=None, grad_dtype=torch.float32,
                  overlap=True, fuse_dense_adam=True, dtype="bf16", augment=None, augment_seed=3):
         self.ctx, self.B, self.train, self.beta2, self.impl = ctx, batch, train, beta2, impl
+        # dtype = "fp8": inference only.  Every convolution and dense product runs on E4M3 codes (tcgen05 kind::f8f6f4)
+        # with one scale per weight row and one per image (include/a3d.h "FP8 inference"); the bf16 buffers below stay as
+        # the quantisers' sources, and fine/third, the maps and the losses are computed as in the bf16 mode.
+        self.fp8 = dtype == "fp8"
+        if self.fp8:
+            if train:
+                raise ValueError("dtype='fp8' is an inference mode: build the net with train=False")
+            if augment is not None:
+                raise ValueError("dtype='fp8' is an inference mode and takes no augment=")
+            if comm is not None:
+                raise ValueError("dtype='fp8' is a single-GPU inference mode (no comm)")
         if augment is not None and not train:
             raise ValueError("augment is a training option: an inference net (train=False) sees its inputs unchanged")
         # dtype = "bf16" (default): BF16 storage of activations / activation gradients / the weight mirror, tcgen05
@@ -55,8 +66,8 @@ class MSDNNet:
         # dtype = "tf32x3": as "tf32", with every forward contraction as a 3xTF32 sum over hi/lo-split operands
         # (a3d_conv2d_fwd_tf32x3 / a3d_dense_fwd_tf32x3): float32-grade products, which is what the 1e-4 worst-pixel
         # bound needs (plain TF32 reaches 2.6e-4, profiles/tf32_parity_r02.log).  The backward pass stays plain TF32.
-        if dtype not in ("bf16", "tf32", "tf32x3"):
-            raise ValueError("dtype must be 'bf16', 'tf32' or 'tf32x3'")
+        if dtype not in ("bf16", "tf32", "tf32x3", "fp8"):
+            raise ValueError("dtype must be 'bf16', 'tf32', 'tf32x3' or 'fp8'")
         self.tf32 = dtype in ("tf32", "tf32x3")
         self.x3 = dtype == "tf32x3"
         if self.tf32:
@@ -161,6 +172,20 @@ class MSDNNet:
             self.g_cat = z(B, 55, 74, 64, **bf)
             self.g_f1big = None                          # [B*4070, 256] bf16, allocated on first use (phase 2 only)
             self.g_wbig = None
+        if self.fp8:
+            def e4(*shape):                                   # E4M3 codes, zero-filled as bytes
+                return torch.zeros(*shape, dtype=torch.uint8, device=self.dev).view(torch.float8_e4m3fn)
+            self.img4q = e4(B, IN_H // 4, IN_W // 4, 64)
+            self.p0q, self.p1q = e4(B, 27, 37, 128), e4(B, 13, 18, 256)
+            self.c2q, self.c3q = e4(B, 13, 18, 384), e4(B, 13, 18, 384)
+            self.c4q, self.d0q, self.catq = e4(B, 12288), e4(B, 4096), e4(B, 55, 74, 64)
+            self.s_img = torch.full((B,), 2.0 ** -8, **f32)            # the resized image lies in [0, 1]: fixed scale
+            self.s_p0, self.s_p1, self.s_c2, self.s_c3, self.s_c4, self.s_d0, self.s_cat = (z(B, **f32) for _ in range(7))
+            # E4M3 weights and their row scales, rebuilt from the bf16 mirror by refresh_derived (outside the arena)
+            self.wq = {}
+            for name, t in self._fp8_weight_sources().items():
+                self.wq[name] = (e4(*t.shape), z(t.shape[0], **f32))
+            self.refresh_derived()
         self._graphs = {}
         if os.environ.get("A3D_TIMELINE") == "1" and ctx.timeline is None:
             ctx.timeline = ops.StepTimeline(self.dev)
@@ -193,6 +218,17 @@ class MSDNNet:
         a = self.arena
         s = a.specs["fine/first/conv2d/kernel"]
         self.ctx.scatter_cast_bf16(a.w[s.offset:s.offset + s.numel], self.emb_k, self.wbig)
+        if self.fp8:
+            for name, t in self._fp8_weight_sources().items():
+                self.ctx.quantize_rows_e4m3(t, *self.wq[name])
+
+    def _fp8_weight_sources(self):
+        """The bf16 operand matrices the FP8 mode quantises per output row (name -> [rows, ...] bf16)."""
+        K = "/kernel"
+        src = {n: self.w(n + K) for n in ["coarse/conv/conv2d_%d" % i for i in range(5)] +
+               ["coarse/dense/dense_0", "coarse/dense/dense_1", "fine/second/conv2d"]}
+        src["fine/first/conv2d"] = self.wbig
+        return src
 
     def flush(self):
         """Data parallel: make the bf16 weight mirror current on this rank (rows other ranks updated in the last step are
@@ -238,6 +274,8 @@ class MSDNNet:
     # ------------------------------------------------------------------ forward
     def forward(self):
         """src/models.py:281-290.  Reads self.images / self.depths, fills self.coarse / self.fine / losses."""
+        if self.fp8:
+            return self._forward_fp8()
         self.ctx.tf32x3 = self.x3
         try:
             self._forward()
@@ -289,6 +327,39 @@ class MSDNNet:
                      loss=self.loss_coarse, dout_ld=4096, **{gk: self.g_coarse if self.train else None})
         c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
                      dout_ld=N_PIX, **{gk: self.g_fine if self.train else None})
+
+    def _forward_fp8(self):
+        """The inference forward on E4M3 operands.  Storage points (oracle/fp8.py restates them): the resized image with
+        the fixed scale 2^-8; max-pool of the bf16 conv2d_0 / conv2d_1 outputs, conv2d_2..4, dense_0 and the concat
+        (bf16) with one scale per image; `coarse` f32, `f2` bf16 and fine/third as in the bf16 mode."""
+        c, B, wq = self.ctx, self.B, self.wq
+        c.resize_bilinear_tf1_s2d_e4m3(self.images, IN_H, IN_W, out=self.img4q)
+        self._resize_target()
+        n = "coarse/conv/conv2d_"
+        c.conv2d_fwd_fp8(self.d_c0, self.img4q, self.s_img, *wq[n + "0"], self.bias(n + "0"), relu=True, out=self.c0)
+        c.maxpool2x2_quantize_e4m3(self.c0, out=self.p0q, scale=self.s_p0)
+        c.conv2d_fwd_fp8(self.d_c1, self.p0q, self.s_p0, *wq[n + "1"], self.bias(n + "1"), relu=True, out=self.c1)
+        c.maxpool2x2_quantize_e4m3(self.c1, out=self.p1q, scale=self.s_p1)
+        c.conv2d_fwd_fp8(self.d_c2, self.p1q, self.s_p1, *wq[n + "2"], self.bias(n + "2"), relu=True, out=self.c2)
+        c.quantize_e4m3(self.c2, out=self.c2q, scale=self.s_c2)
+        c.conv2d_fwd_fp8(self.d_c3, self.c2q, self.s_c2, *wq[n + "3"], self.bias(n + "3"), relu=True, out=self.c3)
+        c.quantize_e4m3(self.c3, out=self.c3q, scale=self.s_c3)
+        c.conv2d_fwd_fp8(self.d_c4, self.c3q, self.s_c3, *wq[n + "4"], self.bias(n + "4"), relu=True, out=self.c4)
+        c.quantize_e4m3(self.c4.view(B, 12288), out=self.c4q, scale=self.s_c4)
+        n = "coarse/dense/dense_"
+        c.dense_fwd_fp8(self.c4q, self.s_c4, *wq[n + "0"], self.bias(n + "0"), flags=L.EPI_RELU, out=self.d0)
+        c.quantize_e4m3(self.d0, out=self.d0q, scale=self.s_d0)
+        c.dense_fwd_fp8(self.d0q, self.s_d0, *wq[n + "1"], self.bias(n + "1"), flags=0, out=self.coarse)
+        c.conv2d_pool4_fwd_fp8(self.d_f1, self.img4q, self.s_img, *wq["fine/first/conv2d"], self.bias("fine/first/conv2d"),
+                               relu=True, out=self.cat)
+        c.scatter_channel_bf16(self.coarse, self.cat, 63)
+        c.quantize_e4m3(self.cat, out=self.catq, scale=self.s_cat)
+        c.conv2d_fwd_fp8(self.d_f2, self.catq, self.s_cat, *wq["fine/second/conv2d"], self.bias("fine/second/conv2d"),
+                         relu=True, out=self.f2)
+        c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third/kernel"), self.bias("fine/third"), relu=False,
+                     out=self.fine.view(B, 55, 74, 1))
+        c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse, loss=self.loss_coarse)
+        c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine)
 
     # ------------------------------------------------------------------ backward
     def _dense_wgrad_adam(self, layer, x, dy):

@@ -537,6 +537,94 @@ class Context:
                                                 splits, _stream()), "debug_tc_gemm_tf32")
         return D
 
+    def debug_tc_gemm_fp8(self, A, B, M, N, K, bn, kcb=128, splits=1, rs=None, rs_div=1, cs=None):
+        """E4M3 operands (tcgen05.mma kind::f8f6f4), A [M,K] and B [N,K] codes: D[M,N] = A . B^T (x rs[m // rs_div] x cs[n])"""
+        D = torch.empty(M, N, dtype=torch.float32, device=A.device)
+        L.check(self.lib.a3d_debug_tc_gemm_fp8(self.h, _ptr(A), _ptr(B), _ptr(D), M, N, K, bn, kcb, splits, _ptr(rs), rs_div,
+                                               _ptr(cs), _stream()), "debug_tc_gemm_fp8")
+        return D
+
+    # ------------------------------------------------------------------ FP8 inference (include/a3d.h "FP8 inference")
+    def quantize_rows_e4m3(self, x, q=None, scale=None):
+        """Per-row E4M3 codes of a bf16 matrix (rows = x.shape[0], the rest flattened): (q float8_e4m3fn, scale f32 [rows])."""
+        rows = x.shape[0]
+        cols = x.numel() // rows
+        if q is None:
+            q = torch.empty(x.shape, dtype=torch.float8_e4m3fn, device=x.device)
+        if scale is None:
+            scale = torch.empty(rows, dtype=torch.float32, device=x.device)
+        L.check(self.lib.a3d_quantize_rows_e4m3(self.h, _ptr(x), rows, cols, cols, _ptr(q), _ptr(scale), _stream()),
+                "quantize_rows_e4m3")
+        return q, scale
+
+    def _quant_ws(self, B, n):
+        return self.workspace(("quant_e4m3",), self.lib.a3d_quantize_ws_bytes_e4m3(B, n))
+
+    def quantize_e4m3(self, x, out=None, scale=None):
+        """Per-image E4M3 codes of a bf16 tensor [B, ...]: (out float8_e4m3fn, scale f32 [B])."""
+        B = x.shape[0]
+        n = x.numel() // B
+        if out is None:
+            out = torch.empty(x.shape, dtype=torch.float8_e4m3fn, device=x.device)
+        if scale is None:
+            scale = torch.empty(B, dtype=torch.float32, device=x.device)
+        ws = self._quant_ws(B, n)
+        L.check(self.lib.a3d_quantize_e4m3(self.h, _ptr(x), B, n, _ptr(out), _ptr(scale), _ptr(ws), ws.numel(), _stream()),
+                "quantize_e4m3")
+        return out, scale
+
+    def maxpool2x2_quantize_e4m3(self, x, out=None, scale=None, ldy=None):
+        """2x2/2 max-pool of bf16 [B,H,W,C] into per-image E4M3 codes [B,H/2,W/2,ldy] (channels >= C zero)."""
+        B, H, W, Cc = x.shape
+        ldy = ldy or (out.shape[-1] if out is not None else Cc)
+        if out is None:
+            out = torch.empty(B, H // 2, W // 2, ldy, dtype=torch.float8_e4m3fn, device=x.device)
+        if scale is None:
+            scale = torch.empty(B, dtype=torch.float32, device=x.device)
+        ws = self._quant_ws(B, (H // 2) * (W // 2) * ldy)
+        L.check(self.lib.a3d_maxpool2x2_quantize_e4m3(self.h, _ptr(x), B, H, W, Cc, _ptr(out), ldy, _ptr(scale), _ptr(ws),
+                                                      ws.numel(), _stream()), "maxpool2x2_quantize_e4m3")
+        return out, scale
+
+    def resize_bilinear_tf1_s2d_e4m3(self, src, OH, OW, out=None):
+        """Resize + space-to-depth(4) of f32 or uint8 images [B,H,W,3] into E4M3 codes of 256 * value [B,OH/4,OW/4,64]."""
+        B, H, W, Cc = src.shape
+        if out is None:
+            out = torch.empty(B, OH // 4, OW // 4, 64, dtype=torch.float8_e4m3fn, device=src.device)
+        sd = L.A3D_U8 if src.dtype == torch.uint8 else L.A3D_F32
+        L.check(self.lib.a3d_resize_bilinear_tf1_s2d_e4m3(self.h, _ptr(src), sd, B, H, W, Cc, _ptr(out), OH, OW, 4,
+                                                          out.shape[-1], _stream()), "resize_s2d_e4m3")
+        return out
+
+    def conv2d_fwd_fp8(self, d, x, x_scale, w, w_scale, bias, relu=False, out=None, out_dtype=torch.bfloat16):
+        if out is None:
+            out = torch.empty(d.N, d.P, d.Q, d.ldy, dtype=out_dtype, device=x.device)
+        ws, nb = self.conv_ws(d, L.OP_FWD)
+        code = L.A3D_BF16 if out.dtype == torch.bfloat16 else L.A3D_F32
+        L.check(self.lib.a3d_conv2d_fwd_fp8(self.h, C.byref(d), _ptr(x), _ptr(x_scale), _ptr(w), _ptr(w_scale), _ptr(bias),
+                                            _ptr(out), code, L.EPI_RELU if relu else 0, _ptr(ws), ws.numel(), _stream()),
+                "conv2d_fwd_fp8")
+        return out
+
+    def conv2d_pool4_fwd_fp8(self, d, x, x_scale, w, w_scale, bias, relu=True, out=None):
+        if out is None:
+            out = torch.empty(d.N, d.P, d.Q, d.ldy, dtype=torch.bfloat16, device=x.device)
+        L.check(self.lib.a3d_conv2d_pool4_fwd_fp8(self.h, C.byref(d), _ptr(x), _ptr(x_scale), _ptr(w), _ptr(w_scale),
+                                                  _ptr(bias), _ptr(out), L.EPI_RELU if relu else 0, _stream()),
+                "conv2d_pool4_fwd_fp8")
+        return out
+
+    def dense_fwd_fp8(self, x, x_scale, w, w_scale, bias, flags=0, out=None, out_dtype=torch.bfloat16):
+        M, K = x.shape[0], x.shape[1]
+        N = w.shape[0]
+        if out is None:
+            out = torch.empty(M, N, dtype=out_dtype, device=x.device)
+        acc = self.workspace(("dense_acc", M, N), M * N * 4)
+        code = L.A3D_BF16 if out.dtype == torch.bfloat16 else L.A3D_F32
+        L.check(self.lib.a3d_dense_fwd_fp8(self.h, _ptr(x), x.stride(0), _ptr(x_scale), _ptr(w), _ptr(w_scale), _ptr(bias),
+                                           _ptr(out), code, _ptr(acc), M, N, K, flags, _stream()), "dense_fwd_fp8")
+        return out
+
     # ------------------------------------------------------------------ DCNF
     def pairwise_dense(self, sims, w2, b1, out=None):
         n = sims.numel() // 2

@@ -41,6 +41,7 @@ extern "C" {
 /* element types */
 #define A3D_F32  0
 #define A3D_BF16 1
+#define A3D_E4M3 3          /* E4M3 codes (e4m3fn: max 448, no infinities), one byte each: the FP8 inference mode */
 
 /* conv / gemm implementation selector */
 #define A3D_IMPL_AUTO 0     /* tcgen05 tensor-core kernels wherever the shape allows */
@@ -549,6 +550,48 @@ int a3d_dcnf_step(a3d_dcnf*, const float* images, const float* depths, float* lo
 int a3d_dcnf_infer(a3d_dcnf*, const float* images, float* output, float* z, float* r, void* stream);
 /* device pointers into the net: CRF MAP estimate y* = A^-1 z [B,48], per-graph Cholesky status, the loss scalar */
 int a3d_dcnf_state(a3d_dcnf*, const float** ystar, const int32_t** status, const float** loss);
+
+/* ---- FP8 inference (E4M3 operands, tcgen05.mma kind::f8f6f4, f32 accumulation) -------------------------------------
+ * The MSDN forward (src/models.py:208-253) with every convolution and dense product on E4M3 codes.  Numerics:
+ *   quantiser   amax = max |x|, s = amax / 448, code = e4m3_rn_satfinite(x * (448 / amax)); amax == 0: s = 0, codes 0
+ *   weights     one scale per output row of the operand matrix the kernels read (a3d_quantize_rows_e4m3 of the bf16
+ *               mirror: [K][R][S][C] filters, [N][K] dense kernels) -- the TF variable's per-output-channel scale
+ *   activations one scale per image (a3d_quantize_e4m3 / a3d_maxpool2x2_quantize_e4m3); the image itself has the fixed
+ *               scale 2^-8 (a3d_resize_bilinear_tf1_s2d_e4m3)
+ *   products    y[m][n] = act(acc[m][n] * x_scale[image(m)] * w_scale[n] + bias[n]), image(m) = m / (P*Q) for a
+ *               convolution and m for a dense layer: an image's result never depends on its batch-mates
+ * Every call is asynchronous on `stream` and capturable in a CUDA graph. */
+/* Weight rows: q[r][0..cols) = codes of x[r*ldx + 0..cols) (bf16), scale[r].  cols % 8 == 0. */
+int a3d_quantize_rows_e4m3(a3d_ctx*, const uint16_t* x, int rows, int cols, long long ldx, uint8_t* q, float* scale,
+                           void* stream);
+/* Per image: y[b][0..n) = codes of x[b][0..n) (bf16, n % 8 == 0), y_scale[b].  ws: a3d_quantize_ws_bytes_e4m3(B, n) bytes
+ * (per-image partial maxima).  Replaces the bf16 storage of conv2d_2 / conv2d_3 / conv2d_4 / dense_0 outputs and of the
+ * fine stack's concat (src/models.py:217-229, 246) as operands of the next layer. */
+size_t a3d_quantize_ws_bytes_e4m3(int B, size_t n);
+int a3d_quantize_e4m3(a3d_ctx*, const uint16_t* x, int B, size_t n, uint8_t* y, float* y_scale, void* ws, size_t ws_bytes,
+                      void* stream);
+/* 2x2/2 max-pool of x bf16 [B,H,W,C] quantised per image: y [B,H/2,W/2,ldy] (channels C..ldy-1 zero), y_scale[b];
+ * src/models.py:212,215.  ws: a3d_quantize_ws_bytes_e4m3(B, (H/2)*(W/2)*ldy) bytes. */
+int a3d_maxpool2x2_quantize_e4m3(a3d_ctx*, const uint16_t* x, int B, int H, int W, int C, uint8_t* y, int ldy,
+                                 float* y_scale, void* ws, size_t ws_bytes, void* stream);
+/* Resize (src/models.py:282) + space-to-depth(4) into E4M3 codes of 256 * value: dst [B,OH/4,OW/4,64] (channels 48..63
+ * zero).  src_dtype A3D_F32 or A3D_U8 (pixel / 255), C == 3. */
+int a3d_resize_bilinear_tf1_s2d_e4m3(a3d_ctx*, const void* src, int src_dtype, int B, int H, int W, int C, uint8_t* dst,
+                                     int OH, int OW, int s, int dstC, void* stream);
+/* Convolution forward (src/models.py:211-223, 247): x E4M3 NHWC (C % 64 == 0), w E4M3 [K][R][S][C]; y bf16 or f32
+ * (y_dtype) [N,P,Q,ldy].  ws: a3d_conv2d_ws_bytes(.., A3D_OP_FWD) bytes enable split-K (nullable). */
+int a3d_conv2d_fwd_fp8(a3d_ctx*, const a3d_conv_desc*, const uint8_t* x, const float* x_scale, const uint8_t* w,
+                       const float* w_scale, const float* bias, void* y, int y_dtype, unsigned flags, void* ws,
+                       size_t ws_bytes, void* stream);
+/* conv + bias + act + 2x2 max-pool over the pool-embedded filter (as a3d_conv2d_pool4_fwd; src/models.py:241-245):
+ * K = 256 = 4 window positions x 64 filters, y bf16 [N,P,Q,ldy] (64 pooled channels). */
+int a3d_conv2d_pool4_fwd_fp8(a3d_ctx*, const a3d_conv_desc*, const uint8_t* x, const float* x_scale, const uint8_t* w,
+                             const float* w_scale, const float* bias, uint16_t* y, unsigned flags, void* stream);
+/* Dense forward (src/models.py:228, 231): y[M][N] = act(x[M][K] . w[N][K]^T * x_scale[m] * w_scale[n] + bias[n]), y bf16 or
+ * f32; K % 128 == 0; acc_ws f32 [M][N]. */
+int a3d_dense_fwd_fp8(a3d_ctx*, const uint8_t* x, int ldx, const float* x_scale, const uint8_t* w, const float* w_scale,
+                      const float* bias, void* y, int y_dtype, float* acc_ws, int M, int N, int K, unsigned flags,
+                      void* stream);
 
 #ifdef __cplusplus
 }
