@@ -436,9 +436,20 @@ void tune_cache_store(const TuneKey& key, int ncand, int choice) {
   fclose(f);
 }
 
-// run(c) launches candidate c on `st`; returns the index of the fastest candidate (0 when tuning is unavailable)
+// run(c) launches candidate c on `st`; returns the index of the fastest candidate (0 when tuning is unavailable).
+// A3D_TUNE_PICK=i (read on every call, for tests that run every candidate of a shape): return i without timing, and
+// neither read nor write the in-process or file cache.  i outside [0, ncand) returns -1 with the error set; the call
+// site returns A3D_EINVAL.
 template <class F>
 int autotune(const TuneKey& key, int ncand, F run, cudaStream_t st) {
+  if (const char* pick = getenv("A3D_TUNE_PICK")) {
+    const int i = atoi(pick);
+    if (i < 0 || i >= ncand) {
+      a3d_set_error("A3D_TUNE_PICK=%d out of range: tuner kind %d has %d candidates for this shape", i, key.v[0], ncand);
+      return -1;
+    }
+    return i;
+  }
   tune_cache_load();
   for (int i = 0; i < g_tune_n; ++i)
     if (memcmp(&g_tune[i].key, &key, sizeof(TuneKey)) == 0) return g_tune[i].choice < ncand ? g_tune[i].choice : 0;
@@ -555,7 +566,9 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
     for (int c = 0; c < 4; ++c) cands[nc++] = c;
     if (pair_mode() >= 2) cands[nc++] = 6;
     if (pair_mode() >= 1) cands[nc++] = 7;
-    return run(cands[autotune(key, nc, [&](int i) { return run(cands[i]); }, st)]);
+    const int best = autotune(key, nc, [&](int i) { return run(cands[i]); }, st);
+    if (best < 0) return A3D_EINVAL;
+    return run(cands[best]);
   }
   if (!a3d_tc_conv_fwd_supported(d)) {
     a3d_set_error("tc conv fwd: unsupported shape (C=%d must be a multiple of 16)", d->C);
@@ -577,6 +590,10 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
   p.PQ = d->P * d->Q; p.Q = d->Q; p.sh = d->stride_h; p.sw = d->stride_w; p.lower_h = -d->pad_t; p.lower_w = -d->pad_l;
   p.S = d->S; p.cblocks = cblocks;
   const bool can_split = ws && ws_bytes >= (size_t)M * d->K * sizeof(float);
+  // whether an unsplit launch stores y through the TMA epilogue (maybe_tma_out): the CTA-pair kernel has no other one,
+  // so its candidates exist only for such outputs, and the tuner key tells the two cases apart
+  const bool out_tma = y_dtype == A3D_F32 ? epi_tma_ok(y, d->ldy)
+                                          : epi_tma_enabled() && (reinterpret_cast<uintptr_t>(y) & 15) == 0 && d->ldy % 8 == 0;
 
   auto launch = [&](int bn, int splits, int variant) -> int {
     CUtensorMap tmB;
@@ -629,8 +646,8 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
         if (!variant_exists(bn, kcb, variant)) continue;
         // 256-row tiles only unsplit and when they still give every SM about one CTA
         if ((variant == V_BM256 || variant == V_BM256_DEEP) && (sp != 1 || tiles / 2 < ctx->sm_count * 3 / 4)) continue;
-        // pair kernel: unsplit, at least one full pair of M tiles
-        if ((variant == V_PAIR || variant == V_PAIR_DEEP) && (sp != 1 || ceil_div(M, 128) < 2)) continue;
+        // pair kernel: unsplit, at least one full pair of M tiles, TMA-stored output
+        if ((variant == V_PAIR || variant == V_PAIR_DEEP) && (sp != 1 || ceil_div(M, 128) < 2 || !out_tma)) continue;
         // pair kernel with an f32 output: 32-column slabs, any BN; with a bf16 output BN % 64 (checked at launch)
         if ((variant == V_PAIR || variant == V_PAIR_DEEP) && y_dtype != A3D_F32 && bn % 64) continue;
         bool dup = false;
@@ -645,9 +662,10 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
   }
   TuneKey key{};
   const int kv[16] = {2, d->N, d->H, d->W, d->C, d->K, d->R, d->S, d->stride_h, d->stride_w, d->pad_t, d->pad_l,
-                      d->P, d->Q, d->ldy, y_dtype * 2 + (can_split ? 1 : 0)};
+                      d->P, d->Q, d->ldy, y_dtype * 2 + (can_split ? 1 : 0) + (out_tma ? 0 : 4)};
   memcpy(key.v, kv, sizeof(kv));
   const int best = autotune(key, nc, [&](int c) { return launch(cand[c].bn, cand[c].splits, cand[c].variant); }, st);
+  if (best < 0) return A3D_EINVAL;
   return launch(cand[best].bn, cand[best].splits, cand[best].variant);
 }
 
@@ -709,7 +727,9 @@ int a3d_tc_dense_fwd(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t* w
   TuneKey key{};
   const int kv[16] = {3, M, N, K, ldx, y_dtype, (int)flags, mask != nullptr, s_ok};
   memcpy(key.v, kv, sizeof(kv));
-  return run(cand[autotune(key, nc, [&](int c) { return run(cand[c]); }, st)]);
+  const int best = autotune(key, nc, [&](int c) { return run(cand[c]); }, st);
+  if (best < 0) return A3D_EINVAL;
+  return run(cand[best]);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -835,6 +855,7 @@ int a3d_tc_conv_wgrad(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, c
                       d->P, d->Q, d->ldy, d->dil_w * 4096 + d->pix_pitch};
   memcpy(key.v, kv, sizeof(kv));
   const int best = autotune(key, nc, [&](int c) { return launch(cand[c].nblk, cand[c].splits, cand[c].bm); }, st);
+  if (best < 0) return A3D_EINVAL;
   return launch(cand[best].nblk, cand[best].splits, cand[best].bm);
 }
 
@@ -952,7 +973,9 @@ int a3d_tc_dense_dgrad(a3d_ctx* ctx, const uint16_t* dy, int lddy, const uint16_
   TuneKey key{};
   const int kv[16] = {4, M, N, K, lddy, s_ok};
   memcpy(key.v, kv, sizeof(kv));
-  return run(cand[autotune(key, nc, [&](int c) { return run(cand[c]); }, st)]);
+  const int best = autotune(key, nc, [&](int c) { return run(cand[c]); }, st);
+  if (best < 0) return A3D_EINVAL;
+  return run(cand[best]);
 }
 
 // wgrad: dw[n][k] = sum_b dy[b][n] x[b][k]; both operands MN-major with the batch as the reduction index.
@@ -1337,7 +1360,9 @@ int a3d_tc_conv_fwd_fp8(a3d_ctx* ctx, const a3d_conv_desc* d, const uint8_t* x, 
     const int kv[16] = {7, d->N, d->H, d->W, d->C, d->K, d->R, d->S, d->stride_h, d->stride_w, d->pad_t, d->pad_l,
                         d->P, d->Q, d->ldy};
     memcpy(key.v, kv, sizeof(kv));
-    return run(autotune(key, 2, run, st));
+    const int best = autotune(key, 2, run, st);
+    if (best < 0) return A3D_EINVAL;
+    return run(best);
   }
   const bool can_split = ws && ws_bytes >= (size_t)M * d->K * sizeof(float);
   auto launch = [&](int bn, int splits, int deep) -> int {
@@ -1398,6 +1423,7 @@ int a3d_tc_conv_fwd_fp8(a3d_ctx* ctx, const a3d_conv_desc* d, const uint8_t* x, 
                       d->P, d->Q, d->ldy, y_dtype * 2 + (can_split ? 1 : 0)};
   memcpy(key.v, kv, sizeof(kv));
   const int best = autotune(key, nc, [&](int c) { return launch(cand[c].bn, cand[c].splits, cand[c].deep); }, st);
+  if (best < 0) return A3D_EINVAL;
   return launch(cand[best].bn, cand[best].splits, cand[best].deep);
 }
 
@@ -1442,7 +1468,9 @@ int a3d_tc_dense_fwd_fp8(a3d_ctx* ctx, const uint8_t* x, int ldx, const float* x
   TuneKey key{};
   const int kv[16] = {8, M, N, K, ldx, y_dtype, (int)flags};
   memcpy(key.v, kv, sizeof(kv));
-  return launch(cand[autotune(key, nc, [&](int c) { return launch(cand[c]); }, st)]);
+  const int best = autotune(key, nc, [&](int c) { return launch(cand[c]); }, st);
+  if (best < 0) return A3D_EINVAL;
+  return launch(cand[best]);
 }
 
 // ---- E4M3 (kind::f8f6f4) engine test hook: D[M][N] (f32) = A * B^T with A [M][K], B [N][K] E4M3 codes, K-major,
