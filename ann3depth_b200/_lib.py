@@ -26,7 +26,7 @@ class A3DError(RuntimeError):
     pass
 
 
-ABI_VERSION = 200          # include/a3d.h A3D_VERSION
+ABI_VERSION = 201          # include/a3d.h A3D_VERSION
 
 
 class ConvDesc(C.Structure):
@@ -129,8 +129,6 @@ SIGNATURES = {
     "a3d_dense_dgrad_act": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _f, _u, _vp]),
     "a3d_dense_wgrad": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp, _i, _i, _i, _i, _vp]),
     "a3d_dense_wgrad_adam": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _f, _f, _f, _vp, _vp]),
-    "a3d_dense_wgrad_adam_rows": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _f, _f, _f, _f,
-                                       _vp, _i, _sz, _sz, _vp]),
     "a3d_bias_grad_bf16": (_i, [_vp, _vp, _sz, _i, _i, _vp, _i, _sz, _vp]),
     "a3d_dense_epilogue_bwd": (_i, [_vp, _vp, _vp, _vp, _f, _vp, _sz, _u, _vp]),
     "a3d_maxpool2x2_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),

@@ -129,7 +129,6 @@ int a3d_simt_dense_wgrad(a3d_ctx*, const uint16_t* x, int ldx, const uint16_t* d
                          int K, cudaStream_t st);
 
 // dense_stream.cu: weight-streaming mma.sync kernels (batch <= 32 dense layers, single-filter convolution)
-int a3d_stream_mode();
 bool a3d_stream_dense_fwd_ok(int M, int N, int K, int ldx);
 bool a3d_stream_dense_dgrad_ok(int M, int N, int K, int lddy);
 int a3d_stream_dense_fwd(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t* w, float* acc, int M, int N, int K,

@@ -195,13 +195,7 @@ extern "C" int a3d_conv2d_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16
   if (d->impl == A3D_IMPL_SIMT) return a3d_simt_conv_fwd(ctx, d, x, w, bias, y, y_dtype, flags, st);
   // single-filter 64-channel convolution (MSDN fine/third): tap products on mma.sync + stencil sum reads the
   // input once; as a BN = 16 tcgen05 GEMM the im2col operand traffic is 25x redundant (49 us vs the input's 17 MB).
-  // A3D_K1_TILED=0 keeps the GEMM.
-  {
-    static int k1 = -1;
-    if (k1 < 0) { const char* ev = getenv("A3D_K1_TILED"); k1 = ev ? atoi(ev) : 1; }
-    if (k1 && d->impl == A3D_IMPL_AUTO && a3d_conv_k1_tiled_ok(d))
-      return a3d_conv_k1_tiled(ctx, d, x, w, bias, y, y_dtype, flags, st);
-  }
+  if (d->impl == A3D_IMPL_AUTO && a3d_conv_k1_tiled_ok(d)) return a3d_conv_k1_tiled(ctx, d, x, w, bias, y, y_dtype, flags, st);
   a3d_conv_desc v;
   const a3d_conv_desc* e = virtualize(d, &v) ? &v : d;
   if (a3d_tc_conv_fwd_supported(e)) return a3d_tc_conv_fwd(ctx, e, x, w, bias, y, y_dtype, flags, ws, ws_bytes, st);

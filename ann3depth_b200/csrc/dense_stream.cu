@@ -357,14 +357,7 @@ conv_k1_tiled_kernel(const uint16_t* __restrict__ x, const uint16_t* __restrict_
   }
 }
 
-int stream_mode() {                                                // A3D_DENSE_STREAM: 0 off, 1 autotuned (default), 2 forced
-  const char* e = getenv("A3D_DENSE_STREAM");
-  return e ? atoi(e) : 1;
-}
-
 }  // namespace
-
-int a3d_stream_mode() { return stream_mode(); }
 
 bool a3d_stream_dense_fwd_ok(int M, int N, int K, int ldx) { return M <= 32 && K % 64 == 0 && ldx % 8 == 0 && N >= 1; }
 bool a3d_stream_dense_dgrad_ok(int M, int N, int K, int lddy) { return M <= 32 && K % 64 == 0 && N >= 1 && lddy >= N; }

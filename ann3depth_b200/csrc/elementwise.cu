@@ -752,62 +752,12 @@ __global__ void resize_bilinear_tf1_s2d4c3_kernel(const float* __restrict__ src,
   }
 }
 
-// Row-staged variant (default when two source rows fit in shared memory): one block per resized output row.  The two
-// source rows the row interpolates between are loaded ONCE with coalesced float4 loads (every source byte crosses
-// HBM -> SM a single time: 118 MB for the MSDN batch), then 228 threads each produce one 8-byte piece (4 bf16) of
-// the space-to-depth output.
-__global__ void __launch_bounds__(256)
-resize_bilinear_tf1_s2d4c3_rows_kernel(const float* __restrict__ src, int H, int W, uint16_t* __restrict__ dst, int OH,
-                                       int OWs, int dstC, float sy, float sx) {
-  extern __shared__ float rows_sm[];                    // [2][W*3]
-  const int oy = blockIdx.x % OH, b = blockIdx.x / OH;
-  const float fy = oy * sy;
-  const int y0 = (int)floorf(fy);
-  const int y1 = min(y0 + 1, H - 1);
-  const float ly = fy - y0;
-  const int row_f4 = W * 3 / 4;
-  const float4* r0 = reinterpret_cast<const float4*>(src + ((size_t)b * H + y0) * W * 3);
-  const float4* r1 = reinterpret_cast<const float4*>(src + ((size_t)b * H + y1) * W * 3);
-  float4* s0 = reinterpret_cast<float4*>(rows_sm);
-  float4* s1 = s0 + row_f4;
-  for (int i = threadIdx.x; i < row_f4; i += blockDim.x) { s0[i] = __ldg(r0 + i); s1[i] = __ldg(r1 + i); }
-  __syncthreads();
-  const float* a0 = rows_sm;
-  const float* a1 = rows_sm + W * 3;
-  const int Y = oy >> 2, dy = oy & 3;
-  uint16_t* orow = dst + ((size_t)b * (OH >> 2) + Y) * OWs * dstC;
-  for (int t = threadIdx.x; t < OWs * 3; t += blockDim.x) {
-    const int X = t / 3, p = t - X * 3;               // piece p = values 4p .. 4p+3 of the 12 (dx, c) values
-    float v[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int k = p * 4 + j;
-      const int dx = k / 3, c = k - dx * 3;
-      const float fx = (X * 4 + dx) * sx;
-      const int x0 = (int)floorf(fx);
-      const int x1 = min(x0 + 1, W - 1);
-      const float lx = fx - x0;
-      const float tl = a0[x0 * 3 + c], tr = a0[x1 * 3 + c], bl = a1[x0 * 3 + c], br = a1[x1 * 3 + c];
-      const float top = tl + (tr - tl) * lx;
-      const float bot = bl + (br - bl) * lx;
-      v[j] = top + (bot - top) * ly;
-    }
-    *reinterpret_cast<uint2*>(orow + (size_t)X * dstC + dy * 12 + p * 4) =
-        make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
-  }
-  if (dy == 0) {
-    const int padq = (dstC - 48) / 4;                  // uint2 pieces of zero padding per pixel
-    for (int t = threadIdx.x; t < OWs * padq; t += blockDim.x) {
-      const int X = t / padq, q = t - X * padq;
-      *reinterpret_cast<uint2*>(orow + (size_t)X * dstC + 48 + q * 4) = make_uint2(0u, 0u);
-    }
-  }
-}
-
-// Pipelined variant of the row-staged kernel: persistent blocks, each walks over output rows and copies the two
-// source rows of its NEXT output row into the other half of shared memory (cp.async, 16 bytes per thread and
-// instruction) while it interpolates the current one, so every resident block always has loads in flight
-// (the one-shot kernel above spends half of each block's life in its compute/store phase: 2.9 TB/s).
+// Row-staged resize (used when two pairs of source rows fit in shared memory): the two source rows an output row
+// interpolates between are loaded ONCE with coalesced 16-byte copies (every source byte crosses HBM -> SM a single time:
+// 118 MB for the MSDN batch).  Persistent blocks, each walks over output rows and copies the two source rows of its
+// NEXT output row into the other half of shared memory (cp.async, 16 bytes per thread and instruction) while it
+// interpolates the current one, so every resident block always has loads in flight (a one-shot kernel with one block
+// per output row spent half of each block's life in its compute/store phase: 2.9 TB/s).
 // T = float (the reference's tensor contract, src/data.py:82-86) or uint8_t (8-bit wire format: value / 255,
 // i.e. the pixels before tools/data_tf_converter.py:36-37 turned them into floats; `scale` = 1/255).
 template <typename T>
@@ -922,18 +872,9 @@ extern "C" int a3d_resize_bilinear_tf1_s2d(a3d_ctx* ctx, const float* src, int B
                   dstC >= s * s * C && (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
               "resize_s2d: bad shape (OH, OW multiples of s; dstC %% 8 == 0 and >= s*s*C)");
   float sy = (float)H / (float)OH, sx = (float)W / (float)OW;
-  static int pipelined = -1;                       // A3D_RESIZE_PIPELINED=0: the one-shot row-staged kernel
-  if (pipelined < 0) { const char* e = getenv("A3D_RESIZE_PIPELINED"); pipelined = e ? atoi(e) : 1; }
-  if (pipelined && s == 4 && C == 3 && (W * 3) % 4 == 0 && (size_t)W * 3 * 4 * sizeof(float) <= 100 * 1024 &&
-      dstC % 4 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0)
+  if (s == 4 && C == 3 && (W * 3) % 4 == 0 && (size_t)W * 3 * 4 * sizeof(float) <= 100 * 1024 && dstC % 4 == 0 &&
+      (reinterpret_cast<uintptr_t>(src) & 15) == 0)
     return launch_resize_pipelined<float>(ctx, src, B, H, W, dst, OH, OW, dstC, 1.f, as_stream(stream));
-  if (s == 4 && C == 3 && (W * 3) % 4 == 0 && (size_t)W * 3 * 2 * sizeof(float) <= 48 * 1024 && dstC % 4 == 0 &&
-      (reinterpret_cast<uintptr_t>(src) & 15) == 0) {
-    resize_bilinear_tf1_s2d4c3_rows_kernel<<<B * OH, 256, (size_t)W * 3 * 2 * sizeof(float), as_stream(stream)>>>(
-        src, H, W, dst, OH, OW / 4, dstC, sy, sx);
-    A3D_LAUNCH_OK(ctx);
-    return 0;
-  }
   if (s == 4 && C == 3) {
     const size_t rows = (size_t)B * OH * (OW / 4);
     int block = 256, grid = grid_for(ctx, rows, block);
@@ -1049,10 +990,11 @@ __device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
 }
 
-// QN = column groups of 16 per warp (warp tile 16 rows x 16*QN columns), BPS = resident blocks per SM the register
-// budget is compiled for, PF = prefetch the next row tile's w/m/v lines into L2 while this one is being updated.
-template <int QN, int BPS, bool PF>
-__global__ void __launch_bounds__(256, BPS)
+// kAdamQN = column groups of 16 per warp (warp tile 16 rows x 16*QN columns), kAdamBPS = resident blocks per SM the
+// register budget is compiled for, kAdamPF = prefetch the next row tile's w/m/v lines into L2 while this one is updated.
+constexpr int kAdamQN = 2, kAdamBPS = 3;
+constexpr bool kAdamPF = true;
+__global__ void __launch_bounds__(256, kAdamBPS)
 dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint16_t* __restrict__ dy, int lddy,
                             float* __restrict__ w, float* __restrict__ m, float* __restrict__ v, uint16_t* __restrict__ wb,
                             int M, int N, int K, float lr_t, float b1, float b2, float eps, float gs,
@@ -1060,11 +1002,11 @@ dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint1
   if (lr_dev) lr_t = __ldg(lr_dev);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int g = lane >> 2, t = lane & 3;
-  const int kc0 = blockIdx.x * (128 * QN) + warp * (16 * QN);          // first weight column of this warp
+  const int kc0 = blockIdx.x * (128 * kAdamQN) + warp * (16 * kAdamQN);          // first weight column of this warp
   // B fragments: bfrag[j][kb][0/1], tile j = 2q + h
-  uint32_t bfrag[2 * QN][2][2];
+  uint32_t bfrag[2 * kAdamQN][2][2];
 #pragma unroll
-  for (int j = 0; j < 2 * QN; ++j) {
+  for (int j = 0; j < 2 * kAdamQN; ++j) {
     const int col = kc0 + 16 * (j >> 1) + 4 * (g >> 1) + 2 * (j & 1) + (g & 1);
 #pragma unroll
     for (int kb = 0; kb < 2; ++kb)
@@ -1079,14 +1021,14 @@ dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint1
   const int nstep = gridDim.y * 16;
   for (int n0 = blockIdx.y * 16; n0 < N; n0 += nstep) {
     const int r0 = n0 + g, r1 = n0 + g + 8;
-    if (PF && t == 0) {
+    if (kAdamPF && t == 0) {
       // the 4 lanes of a quad cover 64 contiguous bytes per (row, column group): one prefetch per quad
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         const int row = (half ? r1 : r0) + nstep;
         if (row < N) {
 #pragma unroll
-          for (int q = 0; q < QN; ++q) {
+          for (int q = 0; q < kAdamQN; ++q) {
             const size_t off = (size_t)row * K + kc0 + 16 * q;
             asm volatile("prefetch.global.L2 [%0];" ::"l"(w + off));
             asm volatile("prefetch.global.L2 [%0];" ::"l"(m + off));
@@ -1107,9 +1049,9 @@ dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint1
         const uint32_t hi = (row < N && b0 + 1 < M) ? __ldg(dy + (size_t)(b0 + 1) * lddy + row) : 0u;
         afrag[kb][i] = lo | (hi << 16);
       }
-    float acc[2 * QN][4];
+    float acc[2 * kAdamQN][4];
 #pragma unroll
-    for (int j = 0; j < 2 * QN; ++j) {
+    for (int j = 0; j < 2 * kAdamQN; ++j) {
       acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
       mma_bf16_16816(acc[j], afrag[0], bfrag[j][0]);
       mma_bf16_16816(acc[j], afrag[1], bfrag[j][1]);
@@ -1119,16 +1061,16 @@ dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint1
     for (int half = 0; half < 2; ++half) {
       const int row = half ? r1 : r0;
       if (row < N) {
-        float4 W[QN], Mo[QN], V[QN];
+        float4 W[kAdamQN], Mo[kAdamQN], V[kAdamQN];
 #pragma unroll
-        for (int q = 0; q < QN; ++q) {
+        for (int q = 0; q < kAdamQN; ++q) {
           const size_t off = (size_t)row * K + kc0 + 16 * q + 4 * t;
           W[q] = *reinterpret_cast<const float4*>(w + off);
           Mo[q] = *reinterpret_cast<const float4*>(m + off);
           V[q] = *reinterpret_cast<const float4*>(v + off);
         }
 #pragma unroll
-        for (int q = 0; q < QN; ++q) {
+        for (int q = 0; q < kAdamQN; ++q) {
           const float gr[4] = {acc[2 * q][half * 2], acc[2 * q][half * 2 + 1], acc[2 * q + 1][half * 2],
                                acc[2 * q + 1][half * 2 + 1]};
           float* pw = &W[q].x; float* pm = &Mo[q].x; float* pv = &V[q].x;
@@ -1155,155 +1097,18 @@ int a3d_mma_dense_wgrad_adam(a3d_ctx* ctx, const uint16_t* x, int ldx, const uin
                              float grad_scale, const float* lr_t_dev, cudaStream_t st) {
   if (M > 32 || K % 256 || !aligned16(w) || !aligned16(m) || !aligned16(v) || (wb && (reinterpret_cast<uintptr_t>(wb) & 7)))
     return A3D_ENOTSUP;
-  // A3D_FUSED_ADAM_CFG = <QN><BPS><PF> digits, e.g. "241" = 32-column warp tiles, 4 blocks/SM, prefetch
-  static int cfg = -1;
-  if (cfg < 0) { const char* e = getenv("A3D_FUSED_ADAM_CFG"); cfg = e ? atoi(e) : 231; }
-  const int qn = cfg / 100, bps = (cfg / 10) % 10, pf = cfg % 10;
-  const int kblocks = K / (128 * qn);
-  int gy = bps * ctx->sm_count / kblocks;            // one resident wave
+  const int kblocks = K / (128 * kAdamQN);
+  int gy = kAdamBPS * ctx->sm_count / kblocks;       // one resident wave
   if (gy < 1) gy = 1;
-  // A3D_FUSED_ADAM_TILES = t > 0: NON-persistent grid, every CTA updates t row tiles and retires.  A resident wave of
-  // this kernel holds ~61 k of the SM's 64 k registers for its whole life, so no tensor-core CTA of the concurrently
-  // running backward GEMMs can start next to it (measured with tools/ablate_step.py: the update costs 0.33 ms of the
-  // 0.99 ms step, almost its stand-alone duration).  Short-lived CTAs hand their SM back every few microseconds and the
-  // pending CTAs of the high-priority main stream take it first.
-  static int tiles_per_cta = -1;
-  if (tiles_per_cta < 0) { const char* e = getenv("A3D_FUSED_ADAM_TILES"); tiles_per_cta = e ? atoi(e) : 0; }
-  if (tiles_per_cta > 0) gy = ceil_div(ceil_div(N, 16), tiles_per_cta);
   if (gy > ceil_div(N, 16)) gy = ceil_div(N, 16);
-  dim3 grid(kblocks, gy);
-#define A3D_MMA_ADAM(QN, BPS, PF)                                                                                     \
-  if (qn == QN && bps == BPS && pf == PF)                                                                             \
-    dense_wgrad_adam_mma_kernel<QN, BPS, PF != 0><<<grid, 256, 0, st>>>(x, ldx, dy, lddy, w, m, v, wb, M, N, K, lr_t, \
-                                                                       beta1, beta2, eps, grad_scale, lr_t_dev);
-  A3D_MMA_ADAM(2, 3, 0) A3D_MMA_ADAM(2, 3, 1) A3D_MMA_ADAM(2, 2, 0) A3D_MMA_ADAM(2, 2, 1)
-  A3D_MMA_ADAM(1, 4, 0) A3D_MMA_ADAM(1, 4, 1) A3D_MMA_ADAM(1, 3, 0) A3D_MMA_ADAM(1, 3, 1)
-  A3D_MMA_ADAM(1, 6, 0) A3D_MMA_ADAM(1, 6, 1)
-  A3D_MMA_ADAM(2, 1, 0) A3D_MMA_ADAM(2, 1, 1) A3D_MMA_ADAM(1, 2, 0) A3D_MMA_ADAM(1, 2, 1) A3D_MMA_ADAM(1, 1, 1)
-#undef A3D_MMA_ADAM
+  dense_wgrad_adam_mma_kernel<<<dim3(kblocks, gy), 256, 0, st>>>(x, ldx, dy, lddy, w, m, v, wb, M, N, K, lr_t, beta1, beta2,
+                                                                 eps, grad_scale, lr_t_dev);
   A3D_LAUNCH_OK(ctx);
   return 0;
 }
 
-// ------------------------------------------------------------------------------------ data-parallel dense update
-// Data parallelism for the dense layers WITHOUT a gradient all-reduce: the weight gradient of a dense layer is the
-// rank-B outer product dy^T x, so instead of reducing N*K gradients (134 MB in bf16 for MSDN) the ranks all-gather
-// the two small activation matrices (x_all [n*B, K], dy_all [n*B, N]: ~1 MB per rank) and every rank updates ITS OWN
-// rows [row_lo, row_hi) of the weight matrix from the gathered batch, gradient formed by mma.sync and consumed by
-// TF-Adam in the same pass (grad_scale = 1/n).  The updated bf16 rows are then all-gathered (dp.py).
-// Same warp tiling as dense_wgrad_adam_mma_kernel<2,...>; the batch loop runs over M/16 MMA k-steps and reloads the
-// B fragments from L1/L2 (x_all is small and shared by every warp of the column strip).
-__global__ void __launch_bounds__(256, 3)
-dense_wgrad_adam_mma_rows_kernel(const uint16_t* __restrict__ x, int ldx, const uint16_t* __restrict__ dy, int lddy,
-                                 float* __restrict__ w, float* __restrict__ m, float* __restrict__ v,
-                                 uint16_t* __restrict__ wb, int M, int K, int row_lo, int row_hi, float lr_t, float b1,
-                                 float b2, float eps, float gs, const float* __restrict__ lr_dev, int gb, size_t xgs,
-                                 size_t dygs) {
-  if (lr_dev) lr_t = __ldg(lr_dev);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  const int kc0 = blockIdx.x * 256 + warp * 32;
-  int colj[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) colj[j] = kc0 + 16 * (j >> 1) + 4 * (g >> 1) + 2 * (j & 1) + (g & 1);
-  const int ksteps = (M + 15) >> 4;
-  for (int n0 = row_lo + blockIdx.y * 16; n0 < row_hi; n0 += gridDim.y * 16) {
-    const int r0 = n0 + g, r1 = n0 + g + 8;
-    float acc[4][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
-#pragma unroll 2
-    for (int kb = 0; kb < ksteps; ++kb) {
-      // gb is a multiple of 16: the 16 batch rows of an MMA k-step lie in ONE rank block (one division per k-step)
-      const int grp = (kb * 16) / gb, rin = kb * 16 - grp * gb;
-      const uint16_t* xk = x + (size_t)grp * xgs + (size_t)rin * ldx;
-      const uint16_t* dyk = dy + (size_t)grp * dygs + (size_t)rin * lddy;
-      uint32_t afrag[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int row = (i & 1) ? r1 : r0;
-        const int bl = (i >> 1) * 8 + 2 * t, b0 = kb * 16 + bl;
-        const uint32_t lo = (row < row_hi && b0 < M) ? __ldg(dyk + (size_t)bl * lddy + row) : 0u;
-        const uint32_t hi = (row < row_hi && b0 + 1 < M) ? __ldg(dyk + (size_t)(bl + 1) * lddy + row) : 0u;
-        afrag[i] = lo | (hi << 16);
-      }
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        uint32_t bfrag[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int bl = h * 8 + 2 * t, b0 = kb * 16 + bl;
-          const uint32_t lo = b0 < M ? __ldg(xk + (size_t)bl * ldx + colj[j]) : 0u;
-          const uint32_t hi = b0 + 1 < M ? __ldg(xk + (size_t)(bl + 1) * ldx + colj[j]) : 0u;
-          bfrag[h] = lo | (hi << 16);
-        }
-        mma_bf16_16816(acc[j], afrag, bfrag);
-      }
-    }
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      const int row = half ? r1 : r0;
-      if (row < row_hi) {
-        float4 W[2], Mo[2], V[2];
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          const size_t off = (size_t)row * K + kc0 + 16 * q + 4 * t;
-          W[q] = *reinterpret_cast<const float4*>(w + off);
-          Mo[q] = *reinterpret_cast<const float4*>(m + off);
-          V[q] = *reinterpret_cast<const float4*>(v + off);
-        }
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          const float gr[4] = {acc[2 * q][half * 2], acc[2 * q][half * 2 + 1], acc[2 * q + 1][half * 2],
-                               acc[2 * q + 1][half * 2 + 1]};
-          float* pw = &W[q].x; float* pm = &Mo[q].x; float* pv = &V[q].x;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float gk = gr[j] * gs;
-            pm[j] = b1 * pm[j] + (1.f - b1) * gk;
-            pv[j] = b2 * pv[j] + (1.f - b2) * gk * gk;
-            pw[j] = pw[j] - lr_t * pm[j] / (sqrtf(pv[j]) + eps);
-          }
-          const size_t off = (size_t)row * K + kc0 + 16 * q + 4 * t;
-          *reinterpret_cast<float4*>(w + off) = W[q];
-          *reinterpret_cast<float4*>(m + off) = Mo[q];
-          *reinterpret_cast<float4*>(v + off) = V[q];
-          if (wb) *reinterpret_cast<uint2*>(wb + off) = make_uint2(pack_bf16x2(W[q].x, W[q].y), pack_bf16x2(W[q].z, W[q].w));
-        }
-      }
-    }
-  }
-}
-
-extern "C" int a3d_dense_wgrad_adam_rows(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t* dy, int lddy, float* w,
-                                         float* m, float* v, uint16_t* w_bf16, int M, int N, int K, int row_lo, int row_hi,
-                                         float lr_t, float beta1, float beta2, float eps, float grad_scale,
-                                         const float* lr_t_dev, int group_rows, size_t x_group_stride,
-                                         size_t dy_group_stride, void* stream) {
-  A3D_REQUIRE(ctx && x && dy && w && m && v && M > 0 && N > 0 && K > 0 && lddy >= N && ldx >= K,
-              "dense wgrad+adam rows: bad argument");
-  A3D_REQUIRE(K % 256 == 0 && aligned16(w) && aligned16(m) && aligned16(v) &&
-                  (!w_bf16 || (reinterpret_cast<uintptr_t>(w_bf16) & 7) == 0),
-              "dense wgrad+adam rows: needs K %% 256 == 0 and 16-byte aligned w/m/v");
-  if (row_hi > N) row_hi = N;
-  if (row_lo >= row_hi) return 0;
-  if (group_rows <= 0) {                       // plain [M, ld] matrices = one block of (M rounded up to 16) rows
-    group_rows = (M + 15) / 16 * 16;
-    x_group_stride = dy_group_stride = 0;
-  }
-  A3D_REQUIRE(group_rows % 16 == 0, "dense wgrad+adam rows: group_rows must be a multiple of 16");
-  const int kblocks = K / 256;
-  int gy = 3 * ctx->sm_count / kblocks;
-  if (gy < 1) gy = 1;
-  if (gy > ceil_div(row_hi - row_lo, 16)) gy = ceil_div(row_hi - row_lo, 16);
-  dense_wgrad_adam_mma_rows_kernel<<<dim3(kblocks, gy), 256, 0, as_stream(stream)>>>(
-      x, ldx, dy, lddy, w, m, v, w_bf16, M, K, row_lo, row_hi, lr_t, beta1, beta2, eps, grad_scale, lr_t_dev, group_rows,
-      x_group_stride, dy_group_stride);
-  A3D_LAUNCH_OK(ctx);
-  return 0;
-}
-
-// BiasAddGrad alone: db[c] = sum_rows dy[row][c]  (dy bf16 [rows][ld]; group_rows > 0: rank blocks as above)
+// BiasAddGrad alone: db[c] = sum_rows dy[row][c]  (dy bf16 [rows][ld]; group_rows > 0: rows in blocks of group_rows,
+// block i at dy + i * group_stride)
 extern "C" int a3d_bias_grad_bf16(a3d_ctx* ctx, const uint16_t* dy, size_t rows, int C, int ld, float* db, int group_rows,
                                   size_t group_stride, void* stream) {
   A3D_REQUIRE(ctx && dy && db && rows > 0 && C > 0 && ld >= C, "bias grad: bad argument");

@@ -25,13 +25,11 @@ CUtensorMapSwizzle swizzle_for(int row_bytes) {
 
 // Operand element type of a tensor map: 2 = bf16; 1 = E4M3; 4 = f32 read as TFLOAT32 -- the TMA unit rounds the low 13 mantissa
 // bits away (round to nearest) on the way into shared memory, so kind::tf32 MMAs see properly rounded TF32 values
-// instead of truncated ones.  A3D_TF32_TMAP=0 selects plain FLOAT32 maps (the MMA then truncates).
+// instead of truncated ones.
 CUtensorMapDataType tmap_dtype(int elt) {
   if (elt == 2) return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
   if (elt == 1) return CU_TENSOR_MAP_DATA_TYPE_UINT8;       // E4M3 codes: the TMA unit only moves the bytes
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("A3D_TF32_TMAP"); v = e ? atoi(e) : 1; }
-  return v ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  return CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
 }
 
 // 2-D operand tensor [rows][cols] (cols contiguous, row pitch ld elements of `elt` bytes); box = box_cols x box_rows.
@@ -163,15 +161,10 @@ int make_tmap_out_bf16(a3d_ctx* ctx, CUtensorMap* tm, const void* base, uint64_t
   return 0;
 }
 
-// A3D_EPI_TMA=0 keeps the per-thread register epilogue (A/B measurements); default: TMA wherever the
-// output is an f32 row-major matrix with 16-byte aligned rows.
-bool epi_tma_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("A3D_EPI_TMA"); v = e ? atoi(e) : 1; }
-  return v != 0;
-}
+// The TMA epilogue wherever the output is an f32 row-major matrix with 16-byte aligned rows; the per-thread register
+// epilogue otherwise.
 bool epi_tma_ok(const void* out, long long ldo) {
-  return epi_tma_enabled() && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (ldo % 4) == 0;
+  return (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (ldo % 4) == 0;
 }
 // switch a row-major f32 epilogue to the TMA epilogue when possible; builds the output map
 int maybe_tma_out(a3d_ctx* ctx, tc::Params& p, CUtensorMap* tmC, bool* use) {
@@ -187,7 +180,7 @@ int maybe_tma_out(a3d_ctx* ctx, tc::Params& p, CUtensorMap* tmC, bool* use) {
     if (rc) return rc;
     p.epi = tc::EPI_TMA_F32;
     *use = true;
-  } else if (p.epi == tc::EPI_ROW_BF16 && epi_tma_enabled() && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 &&
+  } else if (p.epi == tc::EPI_ROW_BF16 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 &&
              (p.ldo % 8) == 0) {
     int rc = make_tmap_out_bf16(ctx, tmC, p.out, (uint64_t)p.M, (uint64_t)p.N, (uint64_t)p.ldo);
     if (rc) return rc;
@@ -229,12 +222,6 @@ int launch_cfg(a3d_ctx* ctx, const CUtensorMap& tmA, const CUtensorMap& tmB, con
 enum { V_BASE = 0, V_DEEP = 1, V_BM256 = 2, V_BM256_DEEP = 3, V_PAIR = 11, V_PAIR_DEEP = 12, V_COUNT = 13 };
 // CTAs that share one B tile: the pair kernel's tensor map for B has a box of BN / 2 rows
 int mcast_cl(int variant) { return variant == V_PAIR || variant == V_PAIR_DEEP ? 2 : 1; }
-// A3D_PAIR: 0 off, 1 deep ring only, 2 (default) both pair variants are tuner candidates
-int pair_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("A3D_PAIR"); v = e ? atoi(e) : 2; }
-  return v;
-}
 template <class C>
 int launch_pair(a3d_ctx* ctx, const CUtensorMap& tmA, const CUtensorMap& tmB_half, const tc::Params& p_in, cudaStream_t st) {
   static bool attr_set = false;
@@ -305,8 +292,7 @@ bool variant_exists(int bn, int kcb, int variant) {
   if (variant == V_BASE) return true;
   if (kcb != 128) return false;
   if (variant == V_DEEP) return bn == 64 || bn == 96 || bn == 128 || bn == 192 || bn == 256;
-  if (variant == V_PAIR) return pair_mode() >= 2 && (bn == 64 || bn == 96 || bn == 128 || bn == 192 || bn == 256);
-  if (variant == V_PAIR_DEEP) return pair_mode() >= 1 && (bn == 64 || bn == 96 || bn == 128 || bn == 192 || bn == 256);
+  if (variant == V_PAIR || variant == V_PAIR_DEEP) return bn == 64 || bn == 96 || bn == 128 || bn == 192 || bn == 256;
   if (variant > V_BM256_DEEP) return false;
   return bn == 64 || bn == 96 || bn == 128 || bn == 256;
 }
@@ -390,18 +376,11 @@ int a3d_tc_finish_f32(a3d_ctx* ctx, const float* acc, const float* bias, const u
 // The first launch of a shape (outside stream capture) therefore times every candidate configuration with CUDA
 // events on the launching stream and caches the winner; later launches -- including the captured ones of the
 // CUDA graph -- reuse it.  Candidate runs overwrite the same output, so tuning has no side effects.
-// A3D_AUTOTUNE=0 keeps the heuristic choice (candidate 0).
 namespace {
 struct TuneKey { int v[16]; };
 struct TuneEntry { TuneKey key; int choice; };
 TuneEntry g_tune[256];
 int g_tune_n = 0;
-
-bool autotune_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("A3D_AUTOTUNE"); v = e ? atoi(e) : 1; }
-  return v != 0;
-}
 
 // A3D_TUNE_CACHE=<file>: choices are appended to the file and read back by later processes, so that a run under a
 // profiler (whose launch overhead distorts the candidate timings) uses exactly the configuration of the plain run.
@@ -453,7 +432,7 @@ int autotune(const TuneKey& key, int ncand, F run, cudaStream_t st) {
   tune_cache_load();
   for (int i = 0; i < g_tune_n; ++i)
     if (memcmp(&g_tune[i].key, &key, sizeof(TuneKey)) == 0) return g_tune[i].choice < ncand ? g_tune[i].choice : 0;
-  if (!autotune_enabled() || ncand <= 1) return 0;
+  if (ncand <= 1) return 0;
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) return 0;
   cudaEvent_t e0, e1;
@@ -564,8 +543,8 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
     // candidates 0..3 one-CTA tiles, 6..7 CTA pairs
     int cands[8], nc = 0;
     for (int c = 0; c < 4; ++c) cands[nc++] = c;
-    if (pair_mode() >= 2) cands[nc++] = 6;
-    if (pair_mode() >= 1) cands[nc++] = 7;
+    cands[nc++] = 6;
+    cands[nc++] = 7;
     const int best = autotune(key, nc, [&](int i) { return run(cands[i]); }, st);
     if (best < 0) return A3D_EINVAL;
     return run(cands[best]);
@@ -593,7 +572,7 @@ int a3d_tc_conv_fwd(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, con
   // whether an unsplit launch stores y through the TMA epilogue (maybe_tma_out): the CTA-pair kernel has no other one,
   // so its candidates exist only for such outputs, and the tuner key tells the two cases apart
   const bool out_tma = y_dtype == A3D_F32 ? epi_tma_ok(y, d->ldy)
-                                          : epi_tma_enabled() && (reinterpret_cast<uintptr_t>(y) & 15) == 0 && d->ldy % 8 == 0;
+                                          : (reinterpret_cast<uintptr_t>(y) & 15) == 0 && d->ldy % 8 == 0;
 
   auto launch = [&](int bn, int splits, int variant) -> int {
     CUtensorMap tmB;
@@ -706,14 +685,12 @@ int a3d_tc_dense_fwd(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t* w
   };
   // batch <= 32: the weight-streaming mma.sync kernel (dense_stream.cu) competes with the tcgen05 tiles;
   // candidates >= 100 are stream launches with 1x / 2x / 3x the resident CTA slots
-  const int smode = a3d_stream_mode();
-  const bool s_ok = smode != 0 && a3d_stream_dense_fwd_ok(M, N, K, ldx);
+  const bool s_ok = a3d_stream_dense_fwd_ok(M, N, K, ldx);
   auto launch_stream = [&](int ctas) -> int {
     int r = a3d_stream_dense_fwd(ctx, x, ldx, w, acc_ws, M, N, K, ctas, st);
     if (r) return r;
     return finish(ctx, acc_ws, bias, mask, drop_rate, y, y_dtype == A3D_F32, (size_t)M, N, N, flags, st);
   };
-  if (s_ok && smode == 2) return launch_stream(2 * ctx->sm_count);
   int cand[24];
   int nc = split_candidates(ctx, tiles, p.num_kb, splits0, cand);
   for (int i = 0, n0 = nc; i < n0; ++i)
@@ -771,9 +748,6 @@ int a3d_tc_conv_wgrad(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, c
   const int cblocks = d->C / bw;
   const int RS = d->R * d->S;
   const int total_blocks = RS * cblocks;
-  static int nblk_env = -1, splits_env = -1;       // experiment knobs: force one configuration
-  if (nblk_env < 0) { const char* e = getenv("A3D_WGRAD_NBLK"); nblk_env = e ? atoi(e) : 0; }
-  if (splits_env < 0) { const char* e = getenv("A3D_WGRAD_SPLITS"); splits_env = e ? atoi(e) : 0; }
   const long long Mpix = (long long)d->N * d->P * d->Q;
   CUtensorMap tmA, tmB;
   int rc = make_tmap_2d(ctx, &tmA, dy, Mpix, d->K, d->ldy, 64, 64);
@@ -812,16 +786,9 @@ int a3d_tc_conv_wgrad(a3d_ctx* ctx, const a3d_conv_desc* d, const uint16_t* x, c
     return A3D_ENOTSUP;
   };
   auto tiles_of = [&](int nblk, int bm = 128) { return ceil_div(d->K, bm) * ceil_div(total_blocks, nblk); };
-  static int bm_env = -1;
-  if (bm_env < 0) { const char* e = getenv("A3D_WGRAD_BM"); bm_env = e ? atoi(e) : 0; }
   if (const char* force = getenv("A3D_WGRAD_FORCE")) {           // "nblk,splits,bm": tests and A/B runs
     int fn = 0, fs = 1, fb = 128;
     if (sscanf(force, "%d,%d,%d", &fn, &fs, &fb) >= 1 && fn > 0) return launch(fn, fs, fb);
-  }
-  if (nblk_env > 0 || splits_env > 0) {
-    const int nblk = nblk_env > 0 ? nblk_env : pick_nblk(bw, total_blocks);
-    const int bm = bm_env == 256 && bw == 64 && nblk <= 4 ? 256 : 128;
-    return launch(nblk, splits_env > 0 ? splits_env : pick_splits(ctx, tiles_of(nblk, bm), p.num_kb, 4), bm);
   }
   // candidates: candidate 0 is the heuristic; then every tile width x {1, 1.5, 2, 3} waves' worth of CTAs,
   // with 128 and (layers with > 128 filters, 64-channel blocks) 256 filters per CTA
@@ -952,14 +919,12 @@ int a3d_tc_dense_dgrad(a3d_ctx* ctx, const uint16_t* dy, int lddy, const uint16_
     if (r) return r;
     return finish_dx();
   };
-  const int smode = a3d_stream_mode();
-  const bool s_ok = smode != 0 && a3d_stream_dense_dgrad_ok(M, N, K, lddy);
+  const bool s_ok = a3d_stream_dense_dgrad_ok(M, N, K, lddy);
   auto launch_stream = [&](int ctas) -> int {
     int r = a3d_stream_dense_dgrad(ctx, dy, lddy, w, acc_ws, M, N, K, ctas, st);
     if (r) return r;
     return finish_dx();
   };
-  if (s_ok && smode == 2) return launch_stream(2 * ctx->sm_count);
   int cand[24];
   int nc = split_candidates(ctx, tiles, p.num_kb, splits0, cand);
   for (int i = 0, n0 = nc; i < n0; ++i)
@@ -994,11 +959,8 @@ int a3d_tc_dense_wgrad(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t*
   p.M = N; p.N = K; p.num_kb = ceil_div(M, 64); p.kb_per_split = p.num_kb; p.a_mode = tc::A_TILED;
   p.epi = tc::EPI_ROW_F32; p.out = dw; p.ldo = K; p.atomic = 0;
   // One k-block per CTA: the kernel is all prologue + epilogue.  N tiles of 128 keep the stage ring under
-  // 104 KB so that two CTAs share an SM and one's epilogue hides the other's prologue (A3D_DWGRAD_BN overrides).
-  static int bn_pref = -1;
-  if (bn_pref < 0) { const char* e = getenv("A3D_DWGRAD_BN"); bn_pref = e ? atoi(e) : 128; }
-  if (bn_pref == 256 && K % 256 == 0) return launch_cfg<tc::Cfg<256, 128, true, true, 64>>(ctx, tmA, tmB, p, 1, st);
-  if (bn_pref >= 128 && K % 128 == 0) return launch_cfg<tc::Cfg<128, 128, true, true, 64>>(ctx, tmA, tmB, p, 1, st);
+  // 104 KB so that two CTAs share an SM and one's epilogue hides the other's prologue.
+  if (K % 128 == 0) return launch_cfg<tc::Cfg<128, 128, true, true, 64>>(ctx, tmA, tmB, p, 1, st);
   return launch_cfg<tc::Cfg<64, 128, true, true, 64>>(ctx, tmA, tmB, p, 1, st);
 }
 

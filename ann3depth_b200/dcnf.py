@@ -14,7 +14,6 @@ src/models.py:138-141): only the unary CNN trains.
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 
@@ -121,10 +120,8 @@ class DCNFNet:
         # patches of 50 x 50 cells) on the same kernels; kept as the cross-check of the fully convolutional form.
         # First layer (:64-66: 11x11x3 -> 64, ReLU, 2x2 max-pool) in both forms: ONE pool-fused convolution over
         # space-to-depth(2) cells of 16 channels, read 4 cells (128 bytes) per tap through an overlapped-pixel view
-        # (params.dcnf_first_embedded; a3d_conv_desc dil_w = 4, pix_pitch = 16).  `first_fold` = 4 materialises the view.
+        # (params.dcnf_first_embedded; a3d_conv_desc dil_w = 4, pix_pitch = 16).
         self.unary = unary
-        self.first_fold = int(os.environ.get("A3D_DCNF_FIRST_FOLD", "1"))
-        assert self.first_fold in (1, 4) and (self.first_fold == 1 or unary == "patches")
         if unary == "fullconv":
             N0, ch, cw = B, (H + 2 * PATCH_PAD) // 2, (W + 2 * PATCH_PAD) // 2
         else:
@@ -139,14 +136,14 @@ class DCNFNet:
         q4 = (s4[0] // 2, s4[1] // 2)
         self.s1, self.s4, self.q4 = s1, s4, q4
         assert q4 == (((rows - 1) * 5 + 7, (cols - 1) * 5 + 7) if unary == "fullconv" else (7, 7))
-        ncell = N0 * ch * cw * 16 * self.first_fold
+        ncell = N0 * ch * cw * 16
         self._cells = z(ncell + 128, **bf)             # + slack: the last positions of the last row read past the end
-        self.cells = self._cells[:ncell].view(N0, ch, cw, 16 * self.first_fold)
+        self.cells = self._cells[:ncell].view(N0, ch, cw, 16)
         cd = ops.conv_desc
         d0 = cd(N0, ch, cw, 64, 256, 6, 2, 1, "valid", ldy=64, impl=impl)
         d0.P, d0.Q = s0
         d0.dil_w = 4
-        d0.pix_pitch = 16 if self.first_fold == 1 else 0
+        d0.pix_pitch = 16
         self.d0 = d0
         self.d0w = L.ConvDesc.from_buffer_copy(d0)     # the weight gradient sees the 4 x 64 GEMM columns
         self.d0w.ldy = 256
@@ -248,7 +245,7 @@ class DCNFNet:
         if self.unary == "fullconv":
             c.image_cells_s2d(self.im, PATCH_PAD, self.cells)
         else:
-            c.extract_patches_s2d(self.im, self.cells, self.first_fold)
+            c.extract_patches_s2d(self.im, self.cells)
         c.conv2d_pool4_fwd(self.d0, self.cells, self.wbig0, self.wf(U + "conv2d/bias"), relu=True, out=self.p0, idx=self.i0)
         c.conv2d_fwd(self.d1, self.p0, self.w(U + "conv2d_1" + K), self.wf(U + "conv2d_1/bias"), relu=True, out=self.c1)
         if self.train:

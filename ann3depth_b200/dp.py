@@ -9,8 +9,6 @@ rank x batch n*B (gradients averaged: sum-allreduce, 1/n folded into the optimiz
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import ops
@@ -23,7 +21,7 @@ class DataParallel:
         # The communication stream outranks the compute streams: its kernels are few and short (NCCL CTAs, the row-sharded
         # dense update) but sit on the step's critical chain; at normal priority the 13 / 35 us row updates of an 8-GPU
         # step waited ~170 / 200 us for a free SM slot among the backward GEMMs' CTAs (profiles/step_timeline_r02_n8*).
-        self.stream = torch.cuda.Stream(device=ctx.device, priority=int(os.environ.get("A3D_DP_COMM_PRIORITY", "-3")))
+        self.stream = torch.cuda.Stream(device=ctx.device, priority=-3)
         self._done = []
         self.bytes_per_step = 0
 
@@ -34,12 +32,6 @@ class DataParallel:
             return a.group_range(name)
         if name == "coarse_conv":
             return a.group_range("CoarseConv")
-        if name in ("coarse_conv_early", "coarse_conv_late"):
-            # the conv stack in two buckets (arena order = backward order conv2d_4 .. conv2d_0): the early one is
-            # exchanged under the remaining backward pass, only conv2d_1/conv2d_0 are left for the end of the step
-            lo, hi = a.group_range("CoarseConv")
-            cut = a.specs["coarse/conv/conv2d_1/kernel"].offset
-            return (lo, cut) if name == "coarse_conv_early" else (cut, hi)
         if name in ("coarse_conv_main", "coarse_conv_0"):
             # conv2d_4 .. conv2d_1 (99 % of the group; exchanged under the rest of the backward pass) | conv2d_0
             # (55 k parameters: the only exchange left in the step's tail)
@@ -155,184 +147,83 @@ class DataParallel:
         rows = s.packed_shape[0]
         return rows % (self.world * 16) == 0 and batch * self.world <= 256 and s.packed_shape[1] % 256 == 0
 
-    def dense_gather_adam(self, net, kernel_name, bias_name, x, dy, group, lr, beta1, eps, after=None):
-        """Data-parallel step of ONE dense layer without a gradient all-reduce (a3d_dense_wgrad_adam_rows):
-             all-gather x [B,K] and dy [B,N] (MBs)  |  this rank updates its row slice of the kernel from the gathered
-             batch, gradient and TF-Adam in one pass (grad_scale 1/n)  |  every rank updates the (replicated) bias
-             from the gathered dy  |  all-gather of the updated bf16 kernel rows.
-        NVLink traffic per rank: the bf16 weights once (no reduce-scatter of gradients); HBM traffic: 26 B/param on
-        1/n of the kernel.  `after`: event of the last reader of the weights (the layer's dgrad)."""
-        a, c, n = net.arena, self.ctx, self.world
-        ks, bs = a.specs[kernel_name], a.specs[bias_name]
-        rows, K = ks.packed_shape
-        N = ks.tf_shape[1]
-        B = x.shape[0]
-        lddy = dy.shape[1]
-        blk = B * (K + lddy)                  # one rank block: x [B,K] followed by dy [B,lddy] -> ONE all-gather
-        key = ("gather", kernel_name)
-        bufs = getattr(self, "_gbufs", None)
-        if bufs is None:
-            bufs = self._gbufs = {}
-        if key not in bufs:
-            bufs[key] = torch.zeros(n, blk, dtype=torch.bfloat16, device=x.device)
-        gbuf = bufs[key]
-        xg, dyg = gbuf.view(-1), gbuf.view(-1)[B * K:]
-        ready = torch.cuda.Event()
-        ready.record(torch.cuda.current_stream())
-        with torch.cuda.stream(self.stream):
-            self.stream.wait_event(ready)
-            gbuf[self.rank, :B * K].view(B, K).copy_(x)
-            gbuf[self.rank, B * K:].view(B, lddy).copy_(dy)
-            c.stamp(f"comm: allgather x,dy {kernel_name.split('/')[-2]} begin")
-            ops.allgather(c, gbuf.view(-1), blk)
-            c.stamp(f"comm: allgather x,dy {kernel_name.split('/')[-2]} end")
-            if after is not None:
-                self.stream.wait_event(after)
-            t = max(net.adam_t[group], 1)
-            r = rows // n
-            c.dense_wgrad_adam_rows(xg, dyg, a.view(a.w, kernel_name), a.view(a.m, kernel_name), a.view(a.v, kernel_name),
-                                    a.view(a.wb, kernel_name), self.rank * r, (self.rank + 1) * r, lr, beta1, net.beta2,
-                                    eps, t, 1.0 / n, lr_t_dev=net.lr_dev[group], N=N, M=n * B, ldx=K, lddy=lddy,
-                                    group_rows=B, x_group_stride=blk, dy_group_stride=blk)
-            # bias: replicated update from the gathered dy
-            sl = slice(bs.offset, bs.offset + bs.size)
-            c.bias_grad_bf16(dyg, N, a.g[bs.offset:bs.offset + N], rows=n * B, ld=lddy, group_rows=B, group_stride=blk)
-            c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], lr, beta1, net.beta2, eps, t, 1.0 / n,
-                      lr_t_dev=net.lr_dev[group])
-            c.stamp(f"comm: rows update {kernel_name.split('/')[-2]} end")
-            ops.allgather(c, a.view(a.wb, kernel_name).view(-1), r * K)
-            c.stamp(f"comm: allgather bf16 rows {kernel_name.split('/')[-2]} end")
-            done = torch.cuda.Event()
-            done.record(self.stream)
-        self._done.append(done)
-        self.bytes_per_step += (n * blk + rows * K) * 2
-        self._row_sharded = getattr(self, "_row_sharded", set()) | {kernel_name}
-
     def dense_gather_adam_merged(self, net, layers, group, lr, beta1, eps, ready):
-        """dense_gather_adam for SEVERAL dense layers with one activation all-gather and a DEFERRED weight publish:
+        """Data-parallel step of the dense layers without a gradient all-reduce: ranks exchange activations, not gradients.
              ONE all-gather of every layer's x [B,K] and dy [B,N] (one latency-bound collective instead of one per layer)
-             |  per layer: this rank updates its row slice from the gathered batch (a3d_dense_wgrad_adam_rows) and the
+             |  per layer: this rank updates its row slice of the kernel from the gathered batch (grad_scale 1/n) and the
                 replicated bias, behind that layer's `after` event (its dgrad: the last reader of the old weights).
-           The all-gather of the updated bf16 rows is NOT enqueued here: nobody reads those weights before the next step's
-           dense forward, so `publish_rows` runs at the START of the next step on the comm stream, under the next step's
+           NVLink traffic per rank: the bf16 weights once (no reduce-scatter of gradients).
+           The all-gather of the updated bf16 rows of dense_0 is NOT enqueued here: nobody reads those weights before the
+           next step's dense forward, so `publish_rows` runs at the START of the next step on the comm stream, under the next step's
            resize + convolution forward (the 134 MB weight exchange was ~330 us of serial NCCL time at the end of the
            8-GPU step; profiles/step_timeline_r02_n8_rank0.json).  `flush` publishes outside a step (checkpoint, export,
            end of a timed loop).
         layers: [(kernel_name, bias_name, x, dy, after_event)]; ready: event after which every x / dy is final."""
         a, c, n = net.arena, self.ctx, self.world
-        publish_now = set(os.environ.get("A3D_DP_PUBLISH_NOW", "dense_1").split(","))
         B = layers[0][2].shape[0]
         # The slice's gradient comes from the tcgen05 wgrad GEMM (f32) followed by the streaming TF-Adam pass (34 B/param;
-        # 0.77-0.91 of the HBM roofline at 8 / 4 / 2 GPUs).  The mma.sync row kernel that forms the gradient in registers
-        # and applies TF-Adam in the same pass (a3d_dense_wgrad_adam_rows, 26 B/param) reloads x per row tile: 0.49 of the
-        # roofline at a gathered batch of 64, 0.22 at 256 -- measured slower in the step at every world size (2 GPUs: 1.096 vs
-        # 1.047 ms); A3D_DP_ROWS_MAX_BATCH=<rows> selects it for gathered batches up to that size.
-        use_gemm = n * B > int(os.environ.get("A3D_DP_ROWS_MAX_BATCH", "0"))
+        # 0.77-0.91 of the HBM roofline at 8 / 4 / 2 GPUs).  An mma.sync row kernel that formed the gradient in registers
+        # and applied TF-Adam in the same pass (26 B/param) reloaded x per row tile: 0.49 of the roofline at a gathered
+        # batch of 64, 0.22 at 256 -- measured slower in the step at every world size (2 GPUs: 1.096 vs 1.047 ms).
         bufs = getattr(self, "_gbufs", None)
         if bufs is None:
             bufs = self._gbufs = {}
         t = max(net.adam_t[group], 1)
-
-        def finish_layer(kn, bn_, dy_all, N, lddy, rows, K, r, group_rows=0, group_stride=0):
-            bs = a.specs[bn_]
-            sl = slice(bs.offset, bs.offset + bs.size)
-            c.bias_grad_bf16(dy_all, N, a.g[bs.offset:bs.offset + N], rows=n * B, ld=lddy, group_rows=group_rows,
-                             group_stride=group_stride)
-            c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], lr, beta1, net.beta2, eps, t, 1.0 / n,
-                      lr_t_dev=net.lr_dev[group])
-            c.stamp(f"comm: rows update {kn.split('/')[-2]} end")
-            self.bytes_per_step += rows * K * 2
-            self._row_sharded = getattr(self, "_row_sharded", set()) | {kn}
-            if kn.split("/")[-2] in publish_now:
-                # a layer updated early in the backward pass is published right away: the comm stream is idle until
-                # the conv gradients exist, and the next step's start then only carries the rest
-                ops.allgather(c, a.view(a.wb, kn).view(-1), r * K)
-                c.stamp(f"comm: publish bf16 rows {kn.split('/')[-2]} (in step) end")
-            else:
-                self._unpublished = getattr(self, "_unpublished", set()) | {kn}
-
         self.rows_launches = getattr(self, "rows_launches", {})
-        if use_gemm:
-            key = ("gather_plain",) + tuple(l[0] for l in layers)
-            if key not in bufs:
-                bufs[key] = [(torch.zeros(n * B, x.shape[1], dtype=torch.bfloat16, device=x.device),
-                              torch.zeros(n * B, dy.shape[1], dtype=torch.bfloat16, device=x.device))
-                             for _, _, x, dy, _ in layers]
-            mats = bufs[key]
-            with torch.cuda.stream(self.stream):
-                self.stream.wait_event(ready)
-                for (kn, bn_, x, dy, after), (xg, dyg) in zip(layers, mats):
-                    xg[self.rank * B:(self.rank + 1) * B].copy_(x)
-                    dyg[self.rank * B:(self.rank + 1) * B].copy_(dy)
-                c.stamp("comm: allgather x,dy (all dense layers) begin")
-                c.allgather_multi([m_.view(-1) for pair in mats for m_ in pair])
-                c.stamp("comm: allgather x,dy (all dense layers) end")
-                for (kn, bn_, x, dy, after), (xg, dyg) in zip(layers, mats):
-                    ks = a.specs[kn]
-                    rows, K = ks.packed_shape
-                    N, lddy = ks.tf_shape[1], dy.shape[1]
-                    r = rows // n
-                    lo_r = self.rank * r
-                    s0_ = ks.offset + lo_r * K
-                    if after is not None:
-                        self.stream.wait_event(after)
-
-                    def rows_launch(kn=kn, xg=xg, dyg=dyg, lo_r=lo_r, r=r, K=K, s0_=s0_):
-                        c.dense_wgrad(xg, dyg[:, lo_r:lo_r + r], dw=a.view(a.g, kn)[lo_r:lo_r + r], db=None, N=r)
-                        sl = slice(s0_, s0_ + r * K)
-                        c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], lr, beta1, net.beta2, eps, t, 1.0 / n,
-                                  lr_t_dev=net.lr_dev[group])
-                    rows_launch()
-                    self.rows_launches[kn] = (rows_launch, dict(M=n * B, rows=r, rows_all=rows, K=K, lddy=lddy,
-                                                                kernel="a3d_dense_wgrad (row slice, tcgen05) + a3d_adam_tf",
-                                                                bytes_per_param=34.0))
-                    finish_layer(kn, bn_, dyg, N, lddy, rows, K, r)
-                done = torch.cuda.Event()
-                done.record(self.stream)
-            self._done.append(done)
-            self.bytes_per_step += sum(m_.numel() for pair in mats for m_ in pair) * 2
-            return
-        offs, blk = [], 0
-        for kn, bn_, x, dy, after in layers:
-            K, lddy = x.shape[1], dy.shape[1]
-            offs.append((blk, blk + B * K))
-            blk += B * (K + lddy)
-        key = ("gather_merged",) + tuple(l[0] for l in layers)
+        key = ("gather_plain",) + tuple(l[0] for l in layers)
         if key not in bufs:
-            bufs[key] = torch.zeros(n, blk, dtype=torch.bfloat16, device=layers[0][2].device)
-        gbuf = bufs[key]
-        flat = gbuf.view(-1)
+            bufs[key] = [(torch.zeros(n * B, x.shape[1], dtype=torch.bfloat16, device=x.device),
+                          torch.zeros(n * B, dy.shape[1], dtype=torch.bfloat16, device=x.device))
+                         for _, _, x, dy, _ in layers]
+        mats = bufs[key]
         with torch.cuda.stream(self.stream):
             self.stream.wait_event(ready)
-            for (kn, bn_, x, dy, after), (ox, ody) in zip(layers, offs):
-                K, lddy = x.shape[1], dy.shape[1]
-                gbuf[self.rank, ox:ox + B * K].view(B, K).copy_(x)
-                gbuf[self.rank, ody:ody + B * lddy].view(B, lddy).copy_(dy)
+            for (kn, bn_, x, dy, after), (xg, dyg) in zip(layers, mats):
+                xg[self.rank * B:(self.rank + 1) * B].copy_(x)
+                dyg[self.rank * B:(self.rank + 1) * B].copy_(dy)
             c.stamp("comm: allgather x,dy (all dense layers) begin")
-            ops.allgather(c, flat, blk)
+            c.allgather_multi([m_.view(-1) for pair in mats for m_ in pair])
             c.stamp("comm: allgather x,dy (all dense layers) end")
-            for (kn, bn_, x, dy, after), (ox, ody) in zip(layers, offs):
+            for (kn, bn_, x, dy, after), (xg, dyg) in zip(layers, mats):
                 ks = a.specs[kn]
                 rows, K = ks.packed_shape
                 N, lddy = ks.tf_shape[1], dy.shape[1]
                 r = rows // n
+                lo_r = self.rank * r
+                s0_ = ks.offset + lo_r * K
                 if after is not None:
                     self.stream.wait_event(after)
 
-                def rows_launch(ox=ox, ody=ody, kn=kn, r=r, N=N, K=K, lddy=lddy):
-                    c.dense_wgrad_adam_rows(flat[ox:], flat[ody:], a.view(a.w, kn), a.view(a.m, kn), a.view(a.v, kn),
-                                            a.view(a.wb, kn), self.rank * r, (self.rank + 1) * r, lr, beta1, net.beta2, eps,
-                                            t, 1.0 / n, lr_t_dev=net.lr_dev[group], N=N, M=n * B, ldx=K, lddy=lddy,
-                                            group_rows=B, x_group_stride=blk, dy_group_stride=blk)
+                def rows_launch(kn=kn, xg=xg, dyg=dyg, lo_r=lo_r, r=r, K=K, s0_=s0_):
+                    c.dense_wgrad(xg, dyg[:, lo_r:lo_r + r], dw=a.view(a.g, kn)[lo_r:lo_r + r], db=None, N=r)
+                    sl = slice(s0_, s0_ + r * K)
+                    c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], lr, beta1, net.beta2, eps, t, 1.0 / n,
+                              lr_t_dev=net.lr_dev[group])
                 rows_launch()
                 # bench.py times exactly this launch for the data-parallel roofline line
                 self.rows_launches[kn] = (rows_launch, dict(M=n * B, rows=r, rows_all=rows, K=K, lddy=lddy,
-                                                            kernel="a3d_dense_wgrad_adam_rows", bytes_per_param=26.0))
-                finish_layer(kn, bn_, flat[ody:], N, lddy, rows, K, r, group_rows=B, group_stride=blk)
+                                                            kernel="a3d_dense_wgrad (row slice, tcgen05) + a3d_adam_tf",
+                                                            bytes_per_param=34.0))
+                # bias: replicated update from the gathered dy
+                bs = a.specs[bn_]
+                sl = slice(bs.offset, bs.offset + bs.size)
+                c.bias_grad_bf16(dyg, N, a.g[bs.offset:bs.offset + N], rows=n * B, ld=lddy)
+                c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], lr, beta1, net.beta2, eps, t, 1.0 / n,
+                          lr_t_dev=net.lr_dev[group])
+                c.stamp(f"comm: rows update {kn.split('/')[-2]} end")
+                self.bytes_per_step += rows * K * 2
+                self._row_sharded = getattr(self, "_row_sharded", set()) | {kn}
+                if kn.split("/")[-2] == "dense_1":
+                    # a layer updated early in the backward pass is published right away: the comm stream is idle until
+                    # the conv gradients exist, and the next step's start then only carries the rest
+                    ops.allgather(c, a.view(a.wb, kn).view(-1), r * K)
+                    c.stamp(f"comm: publish bf16 rows {kn.split('/')[-2]} (in step) end")
+                else:
+                    self._unpublished = getattr(self, "_unpublished", set()) | {kn}
             done = torch.cuda.Event()
             done.record(self.stream)
         self._done.append(done)
-        self.bytes_per_step += n * blk * 2
+        self.bytes_per_step += sum(m_.numel() for pair in mats for m_ in pair) * 2
 
     def publish_rows(self, net):
         """All-gather of the bf16 rows updated by the previous step's dense_gather_adam_merged; enqueued on the comm stream

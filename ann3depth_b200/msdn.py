@@ -79,8 +79,6 @@ class MSDNNet:
         # inside the HBM-bound TF-Adam pass (a3d_dense_wgrad_adam), so the 67 M-element f32 gradient is never written
         # or re-read: 26 instead of 38 bytes per dense parameter and step.  Data parallel runs need the gradient in
         # memory for the reduce-scatter and keep the separate kernels (dp.py shards the optimizer instead).
-        if os.environ.get("A3D_FUSE_DENSE_ADAM"):          # A/B measurements
-            fuse_dense_adam = os.environ["A3D_FUSE_DENSE_ADAM"] != "0"
         self.fuse_dense_adam = fuse_dense_adam
         self._s_fine = self._s_wgrad = self._s_cwgrad = None
         self._wflip = None            # flipped filters of the stride-1 dgrads (refreshed at the start of every step)
@@ -465,323 +463,267 @@ class MSDNNet:
         self.ctx.adam_tf(a.w[lo:hi], a.g[lo:hi], a.m[lo:hi], a.v[lo:hi], a.wb[lo:hi], ADAM_LR[group], ADAM_BETA1,
                          self.beta2, ADAM_EPS, max(self.adam_t[group], 1), grad_scale, lr_t_dev=self.lr_dev[group])
 
-    # ------------------------------------------------------------------ phase-1 step on three streams
+    # ------------------------------------------------------------------ phase-1 step on four streams
     def _enqueue_phase1_overlapped(self):
-        """The multi-stream phase-1 step with its critical path (resize, coarse forward, loss, dgrad chain) on a
-        HIGH-PRIORITY stream: whenever an SM slot frees up, pending CTAs of the chain are placed before those of the
-        fine / wgrad / optimizer streams, which fill the remaining slots.  (CUDA graph capture keeps the priority as
-        a kernel-node attribute.)  A3D_MAIN_PRIORITY=0 disables."""
-        if os.environ.get("A3D_MAIN_PRIORITY", "-1") == "0":
-            return self._enqueue_phase1_streams()
-        if getattr(self, "_s_main", None) is None:
-            self._s_main = torch.cuda.Stream(device=self.dev, priority=-1)
-        cur = torch.cuda.current_stream()
-        e_in = torch.cuda.Event()
-        e_in.record(cur)
-        with torch.cuda.stream(self._s_main):
-            self._s_main.wait_event(e_in)
-            self._enqueue_phase1_streams()
-            e_out = torch.cuda.Event()
-            e_out.record(self._s_main)
-        cur.wait_event(e_out)
-
-    def _enqueue_phase1_streams(self):
         """Same launches as forward() + backward_coarse() + apply_adam(), arranged by data dependence:
              main stream : resize, coarse forward, coarse loss, the dgrad chain (the critical path)
              fine stream : fine forward + fine loss (needs only the image and the coarse map)
              wgrad stream: every weight/bias gradient as soon as its dY exists, each optimizer group's
                            gradient allreduce hand-off and TF-Adam right behind its last wgrad
            so the HBM-bound Adam of the 67 M dense parameters and the small-grid wgrad kernels run under the
-           tensor-bound dgrad chain instead of after it.  Joins back before global_step += 1."""
+           tensor-bound dgrad chain instead of after it.  Joins back before global_step += 1.
+        The main stream has HIGH PRIORITY: whenever an SM slot frees up, pending CTAs of the chain are placed before those
+        of the fine / wgrad / optimizer streams, which fill the remaining slots.  (CUDA graph capture keeps the priority
+        as a kernel-node attribute.)"""
         c, B, K = self.ctx, self.B, "/kernel"
         dev = self.dev
         if self._s_fine is None:
+            self._s_main = torch.cuda.Stream(device=dev, priority=-1)
             self._s_fine, self._s_wgrad = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
             self._s_cwgrad = torch.cuda.Stream(device=dev)
+        cur = torch.cuda.current_stream()
+        e_in = torch.cuda.Event()
+        e_in.record(cur)
         # s2: dense wgrads + dense Adam (HBM-bound) ; s3: conv wgrads + conv Adam (tensor / L2-bound)
-        s0, s1, s2, s3 = torch.cuda.current_stream(), self._s_fine, self._s_wgrad, self._s_cwgrad
-        if isinstance(self.overlap, str):            # debugging knob: "fine" or "wgrad" overlaps only that part
-            s1 = s1 if "fine" in self.overlap else s0
-            s2 = s2 if "wgrad" in self.overlap else s0
-            s3 = s3 if "wgrad" in self.overlap else s0
-        inv_world = 1.0 / self.comm.world if self.comm else 1.0
-        if c.timeline is not None:
-            c.timeline.begin()
-        c.stamp("step begin")
-        # data parallel: the dense rows other ranks updated in the PREVIOUS step arrive now, under this step's resize and
-        # convolution forward (dp.dense_gather_adam_merged / publish_rows); the dense forward waits for them
-        e_pub = self.comm.publish_rows(self) if self.comm else None
+        s0, s1, s2, s3 = self._s_main, self._s_fine, self._s_wgrad, self._s_cwgrad
+        with torch.cuda.stream(s0):
+            s0.wait_event(e_in)
+            inv_world = 1.0 / self.comm.world if self.comm else 1.0
+            if c.timeline is not None:
+                c.timeline.begin()
+            c.stamp("step begin")
+            # data parallel: the dense rows other ranks updated in the PREVIOUS step arrive now, under this step's resize and
+            # convolution forward (dp.dense_gather_adam_merged / publish_rows); the dense forward waits for them
+            e_pub = self.comm.publish_rows(self) if self.comm else None
 
-        def dp_update(bucket, group, after=None):     # DP: reduce-scatter -> sharded TF-Adam -> all-gather (dp.py)
-            self.comm.sharded_adam(self, bucket, group, ADAM_LR[group], ADAM_BETA1, ADAM_EPS, after)
-        hook = self.comm.bucket_ready if self.comm else (lambda *_: None)
+            def dp_update(bucket, group, after=None):     # DP: reduce-scatter -> sharded TF-Adam -> all-gather (dp.py)
+                self.comm.sharded_adam(self, bucket, group, ADAM_LR[group], ADAM_BETA1, ADAM_EPS, after)
+            hook = self.comm.bucket_ready if self.comm else (lambda *_: None)
 
-        def mark(stream):
-            e = torch.cuda.Event()
-            e.record(stream)
-            return e
+            def mark(stream):
+                e = torch.cuda.Event()
+                e.record(stream)
+                return e
 
-        # ---- fine stream, part 0: what the critical path needs only later (depth target, dropout mask)
-        n0 = "coarse/conv/conv2d_"
-        prep = os.environ.get("A3D_DGRAD_PREPARE", "1") != "0"
-        e_start = mark(s0)
-        e_draw = None
-        if self.augment is not None:             # the transform both resizes apply
-            self._augment_draw()
-            e_draw = mark(s0)
-        for side in (s2, s3):                 # every side stream forks from the step's start (a stream that happens to
-            if side is not s0:                # get no work in some mode must still be part of the capture to be joined)
-                side.wait_event(e_start)
-        with torch.cuda.stream(s1):
-            s1.wait_event(e_start)
-            if e_draw is not None:
-                s1.wait_event(e_draw)
-            self._resize_target()
-            if not self.external_mask:
-                c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
-            e_aux = mark(s1)
-            # flipped filters of the stride-1 dgrads (weights are final since the previous step's Adam): three small
-            # transposes that used to sit inside the dgrad chain
-            if self._wflip is None:
-                self._wflip = {}
+            # ---- fine stream, part 0: what the critical path needs only later (depth target, dropout mask)
+            n0 = "coarse/conv/conv2d_"
+            e_start = mark(s0)
+            e_draw = None
+            if self.augment is not None:             # the transform both resizes apply
+                self._augment_draw()
+                e_draw = mark(s0)
+            for side in (s2, s3):                 # every side stream forks from the step's start (a stream that happens to
+                side.wait_event(e_start)          # get no work in some mode must still be part of the capture to be joined)
+            with torch.cuda.stream(s1):
+                s1.wait_event(e_start)
+                if e_draw is not None:
+                    s1.wait_event(e_draw)
+                self._resize_target()
+                if not self.external_mask:
+                    c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
+                e_aux = mark(s1)
+                # flipped filters of the stride-1 dgrads (weights are final since the previous step's Adam): three small
+                # transposes that used to sit inside the dgrad chain
+                if self._wflip is None:
+                    self._wflip = {}
+                    for i, dsc in (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1)):
+                        self._wflip[i] = c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K))
                 for i, dsc in (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1)):
-                    self._wflip[i] = c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K)) if prep else None
-            for i, dsc in (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1)):
-                if self._wflip[i] is not None:
                     c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K), out=self._wflip[i])
-            e_flip = mark(s1)
-        # ---- main: preprocessing
-        self._resize_image()
-        c.stamp("resize done")
-        e_img = mark(s0)
-        # ---- fine stream, part 1: first conv + pool need only the image
-        with torch.cuda.stream(s1):
-            c.ws_tag = "fine"
-            s1.wait_event(e_img)
-            c.conv2d_pool4_fwd(self.d_f1, self.img4, self.wbig, self.bias("fine/first/conv2d"), relu=True, out=self.cat,
-                               idx=self.if1)
-            c.stamp("fine/first done")
-            c.ws_tag = ""
-        # ---- main: coarse forward
-        n = "coarse/conv/conv2d_"
-        c.conv2d_fwd(self.d_c0, self.img4, self.w(n + "0" + K), self.bias(n + "0"), relu=True, out=self.c0)
-        c.maxpool2x2_fwd_f32(self.c0, out=self.p0, idx=self.i0)
-        c.conv2d_fwd(self.d_c1, self.p0, self.w(n + "1" + K), self.bias(n + "1"), relu=True, out=self.c1)
-        c.maxpool2x2_fwd_f32(self.c1, out=self.p1, idx=self.i1)
-        c.conv2d_fwd(self.d_c2, self.p1, self.w(n + "2" + K), self.bias(n + "2"), relu=True, out=self.c2)
-        c.conv2d_fwd(self.d_c3, self.c2, self.w(n + "3" + K), self.bias(n + "3"), relu=True, out=self.c3)
-        c.conv2d_fwd(self.d_c4, self.c3, self.w(n + "4" + K), self.bias(n + "4"), relu=True, out=self.c4)
-        c.stamp("coarse conv fwd done")
-        s0.wait_event(e_aux)
-        if e_pub is not None:
-            s0.wait_event(e_pub)
-        nd = "coarse/dense/dense_"
-        c.dense_fwd(self.c4.view(B, 12288), self.w(nd + "0" + K), self.bias(nd + "0"), flags=L.EPI_RELU,
-                    keep_mask=self.keep_mask, drop_rate=0.5, out=self.d0, impl=self.impl)
-        c.dense_fwd(self.d0, self.w(nd + "1" + K), self.bias(nd + "1"), flags=0, out=self.coarse, impl=self.impl)
-        c.stamp("dense fwd done")
-        e_coarse = mark(s0)
-        # ---- fine stream, part 2
-        with torch.cuda.stream(s1):
-            c.ws_tag = "fine"
-            s1.wait_event(e_coarse)
-            c.scatter_channel_bf16(self.coarse, self.cat, 63)
-            c.conv2d_fwd(self.d_f2, self.cat, self.w("fine/second/conv2d" + K), self.bias("fine/second/conv2d"),
-                         relu=True, out=self.f2)
-            c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third" + K), self.bias("fine/third"), relu=False,
-                         out=self.fine.view(B, 55, 74, 1))
-            c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
-                         dout_bf16=self.g_fine)
-            c.stamp("fine fwd + loss done")
-            c.ws_tag = ""
-            e_fine = mark(s1)
-        # ---- main: coarse loss, then the dgrad chain; wgrad stream follows each dY
-        c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse,
-                     loss=self.loss_coarse, dout_bf16=self.g_coarse, dout_ld=4096)
-        e_g = mark(s0)
-
-        def on_wgrad(event, fn, stream=None, label=None):
-            stream = stream or s2
-            with torch.cuda.stream(stream):
-                c.ws_tag = "wgrad" if stream is s2 else "cwgrad"
-                stream.wait_event(event)
-                if label:
-                    c.stamp(label + " begin")
-                fn()
-                if label:
-                    c.stamp(label + " end")
+                e_flip = mark(s1)
+            # ---- main: preprocessing
+            self._resize_image()
+            c.stamp("resize done")
+            e_img = mark(s0)
+            # ---- fine stream, part 1: first conv + pool need only the image
+            with torch.cuda.stream(s1):
+                c.ws_tag = "fine"
+                s1.wait_event(e_img)
+                c.conv2d_pool4_fwd(self.d_f1, self.img4, self.wbig, self.bias("fine/first/conv2d"), relu=True, out=self.cat,
+                                   idx=self.if1)
+                c.stamp("fine/first done")
                 c.ws_tag = ""
+            # ---- main: coarse forward
+            n = "coarse/conv/conv2d_"
+            c.conv2d_fwd(self.d_c0, self.img4, self.w(n + "0" + K), self.bias(n + "0"), relu=True, out=self.c0)
+            c.maxpool2x2_fwd_f32(self.c0, out=self.p0, idx=self.i0)
+            c.conv2d_fwd(self.d_c1, self.p0, self.w(n + "1" + K), self.bias(n + "1"), relu=True, out=self.c1)
+            c.maxpool2x2_fwd_f32(self.c1, out=self.p1, idx=self.i1)
+            c.conv2d_fwd(self.d_c2, self.p1, self.w(n + "2" + K), self.bias(n + "2"), relu=True, out=self.c2)
+            c.conv2d_fwd(self.d_c3, self.c2, self.w(n + "3" + K), self.bias(n + "3"), relu=True, out=self.c3)
+            c.conv2d_fwd(self.d_c4, self.c3, self.w(n + "4" + K), self.bias(n + "4"), relu=True, out=self.c4)
+            c.stamp("coarse conv fwd done")
+            s0.wait_event(e_aux)
+            if e_pub is not None:
+                s0.wait_event(e_pub)
+            nd = "coarse/dense/dense_"
+            c.dense_fwd(self.c4.view(B, 12288), self.w(nd + "0" + K), self.bias(nd + "0"), flags=L.EPI_RELU,
+                        keep_mask=self.keep_mask, drop_rate=0.5, out=self.d0, impl=self.impl)
+            c.dense_fwd(self.d0, self.w(nd + "1" + K), self.bias(nd + "1"), flags=0, out=self.coarse, impl=self.impl)
+            c.stamp("dense fwd done")
+            e_coarse = mark(s0)
+            # ---- fine stream, part 2
+            with torch.cuda.stream(s1):
+                c.ws_tag = "fine"
+                s1.wait_event(e_coarse)
+                c.scatter_channel_bf16(self.coarse, self.cat, 63)
+                c.conv2d_fwd(self.d_f2, self.cat, self.w("fine/second/conv2d" + K), self.bias("fine/second/conv2d"),
+                             relu=True, out=self.f2)
+                c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third" + K), self.bias("fine/third"), relu=False,
+                             out=self.fine.view(B, 55, 74, 1))
+                c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
+                             dout_bf16=self.g_fine)
+                c.stamp("fine fwd + loss done")
+                c.ws_tag = ""
+                e_fine = mark(s1)
+            # ---- main: coarse loss, then the dgrad chain; wgrad stream follows each dY
+            c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse,
+                         loss=self.loss_coarse, dout_bf16=self.g_coarse, dout_ld=4096)
+            e_g = mark(s0)
 
-        fused = self.fuse_dense_adam and not self.comm
-        a = self.arena
-        # The bias gradients (latency-bound column sums of dY, 7-10 us each) leave the conv-wgrad stream
-        # for the fine stream, whose forward work is long done by then: they run next to the wgrad GEMMs, not before them.
-        # (Data parallel: measured slower at 2 GPUs, 1.184 vs 1.144 ms -- the comm stream's NCCL kernels already fill
-        # those gaps -- so there A3D_SIDE_BIAS must be set to 2 to enable it.)
-        sb_env = os.environ.get("A3D_SIDE_BIAS", "1")
-        side_bias = s1 is not s0 and (sb_env == "2" or (sb_env != "0" and not self.comm))
-        e_bias = {}
+            def on_wgrad(event, fn, stream=None, label=None):
+                stream = stream or s2
+                with torch.cuda.stream(stream):
+                    c.ws_tag = "wgrad" if stream is s2 else "cwgrad"
+                    stream.wait_event(event)
+                    if label:
+                        c.stamp(label + " begin")
+                    fn()
+                    if label:
+                        c.stamp(label + " end")
+                    c.ws_tag = ""
 
-        def conv_wgrad(desc, x, dy, name, event):
+            fused = self.fuse_dense_adam and not self.comm
+            a = self.arena
+            # The bias gradients (latency-bound column sums of dY, 7-10 us each) leave the conv-wgrad stream
+            # for the fine stream, whose forward work is long done by then: they run next to the wgrad GEMMs, not before them.
+            # (Data parallel: measured slower at 2 GPUs, 1.184 vs 1.144 ms -- the comm stream's NCCL kernels already fill
+            # those gaps -- so there the conv wgrads keep their bias gradients.)
+            side_bias = not self.comm
+
+            def conv_wgrad(desc, x, dy, name, event):
+                if side_bias:
+                    with torch.cuda.stream(s1):
+                        s1.wait_event(event)
+                        c.bias_grad_bf16(dy.view(-1, dy.shape[-1]), dy.shape[-1], self.gw(name + "/bias"))
+                    on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=None), s3)
+                else:
+                    on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=self.gw(name + "/bias")), s3)
+
+            dense_wgrad_adam = self._dense_wgrad_adam
+            nd = "coarse/dense/dense_"
+
+            e_loss = e_g
+            c.dense_dgrad_act(self.g_coarse, self.w(nd + "1" + K), self.d0, self.keep_mask, 0.5, L.EPI_RELU, out=self.g_d0,
+                              impl=self.impl)
+            e_g = mark(s0)
+            # data parallel, dense layers: exchange activations instead of gradients (dp.dense_gather_adam_merged)
+            gather = bool(self.comm) and all(self.comm.can_gather_dense(self, nd + l + K, B) for l in "01")
+            e_g1 = e_g
+            if not fused and not gather:
+                # the bucket's Adam overwrites dense_1's weights: it waits for e_g (dense_1's dgrad has read them)
+                on_wgrad(e_loss, lambda: (c.dense_wgrad(self.d0, self.g_coarse, dw=self.gw(nd + "1" + K),
+                                                        db=self.gw(nd + "1/bias"), impl=self.impl),
+                                          self.comm and dp_update("dense_1", "CoarseDense", e_g)))
+            if fused:       # updates dense_1's weights: must follow dense_1's dgrad, their last reader
+                on_wgrad(e_g, lambda: dense_wgrad_adam("1", self.d0, self.g_coarse), label="dense_1 wgrad+adam")
+            e_d0 = e_g
+            c.dense_dgrad_act(self.g_d0, self.w(nd + "0" + K), self.c4.view(B, 12288), None, 0.0, L.EPI_RELU,
+                              out=self.g_c4.view(B, 12288), impl=self.impl)
+            e_g = mark(s0)
+            if gather:
+                # one activation all-gather for both layers as soon as g_d0 exists (e_d0); each layer's row update waits for
+                # its own dgrad; the updated rows are published at the start of the next step
+                g_ = "CoarseDense"
+                self.comm.dense_gather_adam_merged(
+                    self, [(nd + "1" + K, nd + "1/bias", self.d0, self.g_coarse, e_g1),
+                           (nd + "0" + K, nd + "0/bias", self.c4.view(B, 12288), self.g_d0, e_g)],
+                    g_, ADAM_LR[g_], ADAM_BETA1, ADAM_EPS, ready=e_d0)
+            elif not fused:
+                on_wgrad(e_d0, lambda: (c.dense_wgrad(self.c4.view(B, 12288), self.g_d0, dw=self.gw(nd + "0" + K),
+                                                      db=self.gw(nd + "0/bias"), impl=self.impl),
+                                        self.comm and dp_update("dense_0", "CoarseDense", e_g)))
+            c.stamp("dense dgrad done")
+            if fused:
+                on_wgrad(e_g, lambda: dense_wgrad_adam("0", self.c4.view(B, 12288), self.g_d0), label="dense_0 wgrad+adam")
+            elif not self.comm:
+                # single GPU: the dense group's Adam runs under the conv backward.  It overwrites the dense weight
+                # mirror, so it waits for e_g: both dense dgrads (the last readers of those weights) are done.
+                on_wgrad(e_g, lambda: self.apply_adam(("CoarseDense",)))
+            conv_wgrad(self.d_c4, self.c3, self.g_c4, n + "4", e_g)
+            c.conv2d_dgrad(self.d_c4, self.g_c4, self.w(n + "4" + K), out=self.g_c3, relu_src=self.c3)
+            c.stamp("dgrad conv2d_4 done")
+            e_g = mark(s0)
+            conv_wgrad(self.d_c3, self.c2, self.g_c3, n + "3", e_g)
+            s0.wait_event(e_flip)
+            c.conv2d_dgrad(self.d_c3, self.g_c3, self.w(n + "3" + K), out=self.g_c2, relu_src=self.c2, wflip=self._wflip["3"])
+            e_g = mark(s0)
+            conv_wgrad(self.d_c2, self.p1, self.g_c2, n + "2", e_g)
+            c.conv2d_dgrad(self.d_c2, self.g_c2, self.w(n + "2" + K), out=self.g_p1, wflip=self._wflip["2"])
+            c.maxpool2x2_idx_bwd(self.i1, self.g_p1, (B, 27, 37, 256), out=self.g_c1)
+            c.stamp("dgrad conv2d_3,2 + pool bwd done")
+            e_g = mark(s0)
+            # (DP: exchanging conv2d_4..2 here as an early bucket was measured SLOWER at 2 GPUs, 1.30 vs 1.26 ms: three more
+            # NCCL launches cost more than the shorter tail saves)
+            conv_wgrad(self.d_c1, self.p0, self.g_c1, n + "1", e_g)
+            e_w1 = mark(s3)                                # gradients of conv2d_4 .. conv2d_1 are complete
+            c.conv2d_dgrad(self.d_c1, self.g_c1, self.w(n + "1" + K), out=self.g_p0, wflip=self._wflip["1"])
+            c.maxpool2x2_idx_bwd(self.i0, self.g_p0, (B, 55, 74, 96), out=self.g_c0)
+            c.stamp("dgrad conv2d_1 + pool bwd done")
+            e_g = mark(s0)
+            # Single GPU: TF-Adam of conv2d_4 .. conv2d_1 (99 % of the group) runs on the idle fine stream next to
+            # conv2d_0's weight gradient; only conv2d_0's 55 k parameters are updated in the step's tail.  The group is
+            # one contiguous arena range in backward order, so this is the same update as two launches.
+            # Data parallel, the same cut: conv2d_4 .. conv2d_1 are all-reduced in f32 and updated behind conv2d_1's weight
+            # gradient, under conv2d_1's dgrad, the pool backward and conv2d_0's wgrad; the step's tail exchanges conv2d_0's
+            # 55 k parameters only.  (8 GPUs, profiles/step_timeline_r02_n8_rank0.json: the single 16 MB allreduce + Adam was
+            # ~150 us of exposed tail.)  f32 allreduce + replicated Adam beats cast + reduce-scatter + sharded Adam +
+            # all-gather at every world size (4 GPUs: 1.160 vs 1.185 ms; 2 GPUs, with the split: 0.972 vs 1.015 ms -- the
+            # collectives are latency-bound at 8-16 MB and the sharded form needs three of them); a sharded exchange of the
+            # split measured 1.20 against 1.18 ms unsplit at 2 GPUs (the extra NCCL kernels take SM slots from the GEMMs
+            # they overlap with).
+            lo_cc, hi_cc = a.group_range("CoarseConv")
+            split_cc = a.specs["coarse/conv/conv2d_0/kernel"].offset
+            if self.comm:
+                with torch.cuda.stream(s3):
+                    self.comm.bucket_ready(self, "coarse_conv_main", after=e_g,
+                                           then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
+            else:
+                with torch.cuda.stream(s1):
+                    s1.wait_event(e_fine)
+                    s1.wait_event(e_w1)
+                    s1.wait_event(e_g)                      # conv2d_1's dgrad was the last reader of these weights
+                    self.adam_range("CoarseConv", lo_cc, split_cc)
+                    e_fine = mark(s1)
+
+            e_b0 = None
             if side_bias:
                 with torch.cuda.stream(s1):
-                    s1.wait_event(event)
-                    c.bias_grad_bf16(dy.view(-1, dy.shape[-1]), dy.shape[-1], self.gw(name + "/bias"))
-                    e_bias[name] = mark(s1)
-                on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=None), s3)
-            else:
-                on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=self.gw(name + "/bias")), s3)
+                    s1.wait_event(e_g)
+                    c.bias_grad_bf16(self.g_c0.view(-1, 96), 96, self.gw(n + "0/bias"))
+                    e_b0 = mark(s1)
 
-        dense_wgrad_adam = self._dense_wgrad_adam
-        nd = "coarse/dense/dense_"
-
-        e_loss = e_g
-        c.dense_dgrad_act(self.g_coarse, self.w(nd + "1" + K), self.d0, self.keep_mask, 0.5, L.EPI_RELU, out=self.g_d0,
-                          impl=self.impl)
-        e_g = mark(s0)
-        # data parallel, dense layers: exchange activations instead of gradients (dp.dense_gather_adam)
-        gather = bool(self.comm) and all(self.comm.can_gather_dense(self, nd + l + K, B) for l in "01") and \
-            os.environ.get("A3D_DP_GATHER", "1") != "0"
-
-        def dp_dense(layer, x, dy, after):
-            g = "CoarseDense"
-            self.comm.dense_gather_adam(self, nd + layer + K, nd + layer + "/bias", x, dy, g, ADAM_LR[g], ADAM_BETA1,
-                                        ADAM_EPS, after)
-        merged = gather and os.environ.get("A3D_DP_MERGED", "1") != "0"
-        e_g1 = e_g
-        if gather and not merged:
-            on_wgrad(e_loss, lambda: dp_dense("1", self.d0, self.g_coarse, e_g), label="dp dense_1 enqueue")
-        elif not fused and not gather:
-            # the bucket's Adam overwrites dense_1's weights: it waits for e_g (dense_1's dgrad has read them)
-            on_wgrad(e_loss, lambda: (c.dense_wgrad(self.d0, self.g_coarse, dw=self.gw(nd + "1" + K),
-                                                    db=self.gw(nd + "1/bias"), impl=self.impl),
-                                      self.comm and dp_update("dense_1", "CoarseDense", e_g)))
-        if fused:       # updates dense_1's weights: must follow dense_1's dgrad, their last reader
-            on_wgrad(e_g, lambda: dense_wgrad_adam("1", self.d0, self.g_coarse), label="dense_1 wgrad+adam")
-        e_d0 = e_g
-        c.dense_dgrad_act(self.g_d0, self.w(nd + "0" + K), self.c4.view(B, 12288), None, 0.0, L.EPI_RELU,
-                          out=self.g_c4.view(B, 12288), impl=self.impl)
-        e_g = mark(s0)
-        if merged:
-            # one activation all-gather for both layers as soon as g_d0 exists (e_d0); each layer's row update waits for
-            # its own dgrad; the updated rows are published at the start of the next step
-            g_ = "CoarseDense"
-            self.comm.dense_gather_adam_merged(
-                self, [(nd + "1" + K, nd + "1/bias", self.d0, self.g_coarse, e_g1),
-                       (nd + "0" + K, nd + "0/bias", self.c4.view(B, 12288), self.g_d0, e_g)],
-                g_, ADAM_LR[g_], ADAM_BETA1, ADAM_EPS, ready=e_d0)
-        elif gather:
-            on_wgrad(e_d0, lambda: dp_dense("0", self.c4.view(B, 12288), self.g_d0, e_g), label="dp dense_0 enqueue")
-        elif not fused:
-            on_wgrad(e_d0, lambda: (c.dense_wgrad(self.c4.view(B, 12288), self.g_d0, dw=self.gw(nd + "0" + K),
-                                                  db=self.gw(nd + "0/bias"), impl=self.impl),
-                                    self.comm and dp_update("dense_0", "CoarseDense", e_g)))
-        c.stamp("dense dgrad done")
-        if fused:
-            on_wgrad(e_g, lambda: dense_wgrad_adam("0", self.c4.view(B, 12288), self.g_d0), label="dense_0 wgrad+adam")
-        elif not self.comm:
-            # single GPU: the dense group's Adam runs under the conv backward.  It overwrites the dense weight
-            # mirror, so it waits for e_g: both dense dgrads (the last readers of those weights) are done.
-            on_wgrad(e_g, lambda: self.apply_adam(("CoarseDense",)))
-        conv_wgrad(self.d_c4, self.c3, self.g_c4, n + "4", e_g)
-        c.conv2d_dgrad(self.d_c4, self.g_c4, self.w(n + "4" + K), out=self.g_c3, relu_src=self.c3)
-        c.stamp("dgrad conv2d_4 done")
-        e_g = mark(s0)
-        conv_wgrad(self.d_c3, self.c2, self.g_c3, n + "3", e_g)
-        s0.wait_event(e_flip)
-        c.conv2d_dgrad(self.d_c3, self.g_c3, self.w(n + "3" + K), out=self.g_c2, relu_src=self.c2, wflip=self._wflip["3"])
-        e_g = mark(s0)
-        conv_wgrad(self.d_c2, self.p1, self.g_c2, n + "2", e_g)
-        c.conv2d_dgrad(self.d_c2, self.g_c2, self.w(n + "2" + K), out=self.g_p1, wflip=self._wflip["2"])
-        c.maxpool2x2_idx_bwd(self.i1, self.g_p1, (B, 27, 37, 256), out=self.g_c1)
-        c.stamp("dgrad conv2d_3,2 + pool bwd done")
-        e_g = mark(s0)
-        # (DP: exchanging conv2d_4..2 here as an early bucket was measured SLOWER at 2 GPUs, 1.30 vs 1.26 ms: three more
-        # NCCL launches cost more than the shorter tail saves; dp.bucket_range keeps the early/late split available)
-        conv_wgrad(self.d_c1, self.p0, self.g_c1, n + "1", e_g)
-        e_w1 = mark(s3)                                # gradients of conv2d_4 .. conv2d_1 are complete
-        c.conv2d_dgrad(self.d_c1, self.g_c1, self.w(n + "1" + K), out=self.g_p0, wflip=self._wflip["1"])
-        c.maxpool2x2_idx_bwd(self.i0, self.g_p0, (B, 55, 74, 96), out=self.g_c0)
-        c.stamp("dgrad conv2d_1 + pool bwd done")
-        e_g = mark(s0)
-        # Single GPU: TF-Adam of conv2d_4 .. conv2d_1 (99 % of the group) runs on the idle fine stream next to
-        # conv2d_0's weight gradient; only conv2d_0's 55 k parameters are updated in the step's tail.  The group is
-        # one contiguous arena range in backward order, so this is the same update as two launches.
-        # DP exchange of the conv stack (4 M parameters): f32 allreduce + replicated Adam beats cast + reduce-scatter +
-        # sharded Adam + all-gather at every world size (4 GPUs: 1.160 vs 1.185 ms; 2 GPUs, with the split below:
-        # 0.972 vs 1.015 ms -- the collectives are latency-bound at 8-16 MB and the sharded form needs three of them).
-        # A3D_DP_CONV_ALLREDUCE=0 selects the sharded form (a weight-sharded optimizer, kept for large conv stacks).
-        conv_allreduce = os.environ.get("A3D_DP_CONV_ALLREDUCE", "1" if self.comm else "0") == "1"
-        lo_cc, hi_cc = a.group_range("CoarseConv")
-        split_cc = a.specs["coarse/conv/conv2d_0/kernel"].offset
-        split_ok = (not self.comm) and lo_cc < split_cc < hi_cc and a.specs["coarse/conv/conv2d_0/bias"].offset > split_cc
-        # Data parallel, optional (A3D_DP_CONV_SPLIT=1): the same cut for the exchange.  conv2d_4 .. conv2d_1 go through
-        # reduce-scatter -> sharded Adam -> all-gather right behind conv2d_1's weight gradient, under conv2d_1's dgrad and
-        # conv2d_0's wgrad; the tail keeps ONE small f32 allreduce (conv2d_0) + its replicated Adam instead of three
-        # collectives.  Measured at 2 GPUs: 1.20 ms against 1.18 ms unsplit -- the extra NCCL kernels take SM slots from
-        # the GEMMs they overlap with -- so it is off by default.
-        dp_split = bool(self.comm) and lo_cc < split_cc < hi_cc and (split_cc - lo_cc) % (self.comm.world * 8) == 0 and \
-            os.environ.get("A3D_DP_CONV_SPLIT", "0") == "1" and not conv_allreduce
-        # With the f32-allreduce exchange (the default) the same cut is ON by default: conv2d_4 .. conv2d_1 (99 % of the bucket)
-        # are all-reduced and updated behind conv2d_1's weight gradient, under conv2d_1's dgrad, the pool backward and
-        # conv2d_0's wgrad; the step's tail exchanges conv2d_0's 55 k parameters only.  (8 GPUs, profiles/
-        # step_timeline_r02_n8_rank0.json: the single 16 MB allreduce + Adam was ~150 us of exposed tail.)
-        dp_split_ar = bool(self.comm) and conv_allreduce and lo_cc < split_cc < hi_cc and \
-            os.environ.get("A3D_DP_CONV_SPLIT", "1") == "1"
-        if dp_split_ar:
-            with torch.cuda.stream(s3):
-                if side_bias:
-                    s3.wait_event(e_bias[n + "1"])
-                self.comm.bucket_ready(self, "coarse_conv_main", after=e_g,
-                                       then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
-        if dp_split:
-            with torch.cuda.stream(s3):
-                if side_bias:
-                    s3.wait_event(e_bias[n + "1"])         # s1 is in order: the biases of conv2d_4 .. conv2d_1 are done
-                dp_update("coarse_conv_main", "CoarseConv", e_g)
-        if split_ok:
-            with torch.cuda.stream(s1):
-                s1.wait_event(e_fine)
-                s1.wait_event(e_w1)
-                s1.wait_event(e_g)                      # conv2d_1's dgrad was the last reader of these weights
-                self.adam_range("CoarseConv", lo_cc, split_cc)
-                e_fine = mark(s1)
-
-        e_b0 = None
-        if side_bias:
-            with torch.cuda.stream(s1):
-                s1.wait_event(e_g)
-                c.bias_grad_bf16(self.g_c0.view(-1, 96), 96, self.gw(n + "0/bias"))
-                e_b0 = mark(s1)
-
-        def conv0_and_adam():
-            c.conv2d_wgrad(self.d_c0, self.img4, self.g_c0, dw=self.gw(n + "0" + K), db=None if side_bias else self.gw(n + "0/bias"))
-            if e_b0 is not None:
-                s3.wait_event(e_b0)
-            self._mask_padding("coarse/conv/conv2d_0/kernel")
-            if self.comm and (dp_split or dp_split_ar):
-                self.comm.bucket_ready(self, "coarse_conv_0",
-                                       then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
-                self.comm.wait_all(self)
-            elif self.comm:
-                if conv_allreduce:                                          # f32 allreduce + replicated Adam (1 NCCL op)
-                    self.comm.bucket_ready(self, "coarse_conv",
+            def conv0_and_adam():
+                c.conv2d_wgrad(self.d_c0, self.img4, self.g_c0, dw=self.gw(n + "0" + K), db=None if side_bias else self.gw(n + "0/bias"))
+                if e_b0 is not None:
+                    s3.wait_event(e_b0)
+                self._mask_padding("coarse/conv/conv2d_0/kernel")
+                if self.comm:
+                    self.comm.bucket_ready(self, "coarse_conv_0",
                                            then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
+                    self.comm.wait_all(self)
                 else:
-                    dp_update("coarse_conv", "CoarseConv")
-                self.comm.wait_all(self)
-            elif split_ok:
-                self.adam_range("CoarseConv", split_cc, hi_cc)
-            else:
-                self.apply_adam(("CoarseConv",))
-        on_wgrad(e_g, conv0_and_adam, s3, label="conv2d_0 wgrad + conv exchange/adam")
-        # ---- join
-        s0.wait_event(e_fine)
-        s0.wait_event(mark(s2))
-        if s3 is not s2:
+                    self.adam_range("CoarseConv", split_cc, hi_cc)
+            on_wgrad(e_g, conv0_and_adam, s3, label="conv2d_0 wgrad + conv exchange/adam")
+            # ---- join
+            s0.wait_event(e_fine)
+            s0.wait_event(mark(s2))
             s0.wait_event(mark(s3))
-        c.increment_i64(self.step_dev)
-        c.stamp("step end")
+            c.increment_i64(self.step_dev)
+            c.stamp("step end")
+            e_out = torch.cuda.Event()
+            e_out.record(s0)
+        cur.wait_event(e_out)
 
     # ------------------------------------------------------------------ one session.run(model_op)
     def _enqueue_step(self, phase):

@@ -497,21 +497,6 @@ class Context:
                                               _ptr(v), _ptr(w_bf16), M, N, K, adam_lr_t(lr, beta1, beta2, t), beta1,
                                               beta2, eps, grad_scale, _ptr(lr_t_dev), _stream()), "dense_wgrad_adam")
 
-    def dense_wgrad_adam_rows(self, x, dy, w, m, v, w_bf16, row_lo, row_hi, lr, beta1, beta2, eps, t, grad_scale=1.0,
-                              lr_t_dev=None, N=None, M=None, ldx=None, lddy=None, group_rows=0, x_group_stride=0,
-                              dy_group_stride=0):
-        """Rows [row_lo, row_hi) of a dense kernel updated from the (all-gathered) batch x [M,K], dy [M,lddy];
-        with group_rows the batch is stored in rank blocks (see include/a3d.h)."""
-        if M is None:
-            M, lddy = dy.shape
-            ldx = x.shape[1]
-        Nw, K = w.shape
-        L.check(self.lib.a3d_dense_wgrad_adam_rows(self.h, _ptr(x), ldx, _ptr(dy), lddy, _ptr(w), _ptr(m), _ptr(v),
-                                                   _ptr(w_bf16), M, N if N is not None else Nw, K, row_lo, row_hi,
-                                                   adam_lr_t(lr, beta1, beta2, t), beta1, beta2, eps, grad_scale,
-                                                   _ptr(lr_t_dev), group_rows, x_group_stride, dy_group_stride,
-                                                   _stream()), "dense_wgrad_adam_rows")
-
     def bias_grad_bf16(self, dy, C_, db, rows=None, ld=None, group_rows=0, group_stride=0):
         if rows is None:
             rows, ld = dy.shape

@@ -29,7 +29,8 @@
 extern "C" {
 #endif
 
-#define A3D_VERSION 200   /* 200: a3d_conv_desc gained dil_w / pix_pitch; TF32, model-level and DCNF fully convolutional entry points */
+#define A3D_VERSION 201   /* 201: a3d_dense_wgrad_adam_rows removed.
+                             200: a3d_conv_desc gained dil_w / pix_pitch; TF32, model-level and DCNF fully convolutional entry points */
 
 /* negative error codes */
 #define A3D_EINVAL   (-1)   /* bad argument / unsupported shape */
@@ -185,21 +186,8 @@ int a3d_dense_wgrad_adam(a3d_ctx*, const uint16_t* x, int ldx, const uint16_t* d
                          float* w, float* m, float* v, uint16_t* w_bf16, int M, int N, int K,
                          float lr_t, float beta1, float beta2, float eps, float grad_scale,
                          const float* lr_t_dev, void* stream);
-/* Data-parallel form of the above: updates only rows [row_lo, row_hi) of the [N,K] kernel, from a batch of M
- * samples (M <= any multiple of 16; the ranks' all-gathered activations x_all [M,K], dy_all [M,N]).  With
- * grad_scale = 1/n this is the sharded optimizer step of n ranks x batch B without any gradient all-reduce: a dense
- * layer's gradient is the rank-M product dy_all^T x_all, so the ranks exchange activations (MBs) instead of
- * gradients (100s of MBs) -- replaces the parameter-server gradient push of src/ann3depth.py:78-92 for the dense
- * variables.  Requires K % 256 == 0.
- * group_rows > 0: the gathered batch is stored in rank blocks -- batch row b is row b % group_rows of block
- * b / group_rows, blocks x_group_stride / dy_group_stride elements apart (x and dy of a rank travel in ONE
- * all-gather); group_rows = 0: plain [M, ld] matrices. */
-int a3d_dense_wgrad_adam_rows(a3d_ctx*, const uint16_t* x, int ldx, const uint16_t* dy, int lddy,
-                              float* w, float* m, float* v, uint16_t* w_bf16, int M, int N, int K,
-                              int row_lo, int row_hi, float lr_t, float beta1, float beta2, float eps,
-                              float grad_scale, const float* lr_t_dev, int group_rows,
-                              size_t x_group_stride, size_t dy_group_stride, void* stream);
-/* BiasAddGrad alone: db[c] = sum over rows of dy[row][c] (dy bf16 [rows][ld]; group_rows / group_stride as above). */
+/* BiasAddGrad alone: db[c] = sum over rows of dy[row][c] (dy bf16 [rows][ld]).  group_rows > 0: the rows are stored in
+ * blocks -- row r is row r % group_rows of block r / group_rows, blocks group_stride elements apart. */
 int a3d_bias_grad_bf16(a3d_ctx*, const uint16_t* dy, size_t rows, int C, int ld, float* db, int group_rows,
                        size_t group_stride, void* stream);
 /* Elementwise backward of the dense epilogue: g_pre = g_post * mask/(1-rate) * act'(y).

@@ -29,7 +29,7 @@ def test_ctypes_table_matches_header(repo_root):
     table = {n for n in _lib.SIGNATURES if not n.startswith("a3d_debug_")}
     assert names == table, (names - table, table - names)
     lib = _lib.load()
-    assert lib.a3d_version() == 200 == _lib.ABI_VERSION
+    assert lib.a3d_version() == 201 == _lib.ABI_VERSION
 
 
 def test_no_device_fails_loudly():

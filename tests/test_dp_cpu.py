@@ -117,7 +117,7 @@ def _gather_worker(rank, world, port, out):
     B, K, N = 4, 64, 48
     g = torch.Generator().manual_seed(10 + rank)
     x, dy = torch.randn(B, K, generator=g), torch.randn(B, N, generator=g)
-    # activation-gather protocol of dp.dense_gather_adam: gather the small matrices, update own rows only
+    # activation-gather protocol of dp.dense_gather_adam_merged: gather the small matrices, update own rows only
     xs, dys = [torch.empty_like(x) for _ in range(world)], [torch.empty_like(dy) for _ in range(world)]
     dist.all_gather(xs, x)
     dist.all_gather(dys, dy)
@@ -138,7 +138,7 @@ def _gather_worker(rank, world, port, out):
 
 def test_dense_activation_gather_equals_gradient_allreduce(tmp_path):
     """dW = dy^T x has rank B: all-gathering x and dy and updating one's own rows is the same update as the
-    gradient sum-allreduce it replaces (dp.dense_gather_adam, a3d_dense_wgrad_adam_rows)."""
+    gradient sum-allreduce it replaces (dp.dense_gather_adam_merged)."""
     world, port = 2, 29532
     out = str(tmp_path / "gather.pt")
     mp.spawn(_gather_worker, args=(world, port, out), nprocs=world, join=True)

@@ -377,8 +377,8 @@ def test_dense_bwd(ctx, M, N, K, ld, impl):
 
 @pytest.mark.parametrize("M,N,K", [(32, 4096, 12288), (32, 4070, 4096), (7, 300, 192), (32, 256, 64), (1, 4070, 4096)])
 def test_dense_stream_kernels(ctx, monkeypatch, M, N, K):
-    """csrc/dense_stream.cu (weight-streaming mma.sync path for batch <= 32), forced with A3D_DENSE_STREAM=2,
-    against fp32 evaluation of the same bf16 operands and against the tcgen05 path (A3D_DENSE_STREAM=0)."""
+    """csrc/dense_stream.cu (weight-streaming mma.sync path for batch <= 32), forced with A3D_DENSE_FORCE=101,
+    against fp32 evaluation of the same bf16 operands and against an unsplit tcgen05 tile (A3D_DENSE_FORCE=1)."""
     x = bf16_rand(M, K, seed=40)
     w = bf16_rand(N, K, seed=41, scale=1.0 / math.sqrt(K))
     bias = (torch.rand(N, generator=torch.Generator().manual_seed(42)) - 0.5).to(DEV)
@@ -388,8 +388,8 @@ def test_dense_stream_kernels(ctx, monkeypatch, M, N, K):
     dyp[:, :N] = bf16_rand(M, N, seed=44)
     dy = dyp[:, :N]
     out = {}
-    for mode in ("2", "0"):
-        monkeypatch.setenv("A3D_DENSE_STREAM", mode)
+    for mode in ("101", "1"):
+        monkeypatch.setenv("A3D_DENSE_FORCE", mode)
         n0 = ctx.launches
         y = ctx.dense_fwd(x, w, bias, flags=L.EPI_RELU, keep_mask=mask, drop_rate=0.5, out_dtype=torch.float32, impl=L.IMPL_TC)
         dx = ctx.dense_dgrad(dyp, w, impl=L.IMPL_TC)
@@ -398,10 +398,10 @@ def test_dense_stream_kernels(ctx, monkeypatch, M, N, K):
         out[mode] = (y, dx)
     ref_y = torch.relu(x.float() @ w.float().t() + bias) * mask.float() * 2.0
     ref_dx = dy.float() @ w.float()
-    for mode in ("2", "0"):
+    for mode in ("101", "1"):
         assert rel_err(out[mode][0], ref_y) < 2e-3, mode
         assert rel_err(out[mode][1], ref_dx) < 1e-2, mode
-    assert rel_err(out["2"][0], out["0"][0]) < 1e-3
+    assert rel_err(out["101"][0], out["1"][0]) < 1e-3
 
 
 @pytest.mark.parametrize("H,W,R,pad", [(55, 74, 5, "same"), (9, 13, 3, "same"), (12, 20, 5, "valid"), (3, 150, 5, "same")])
@@ -723,10 +723,10 @@ def test_gather_sum_and_scatter_cast(ctx):
     assert torch.equal(out, exp)
 
 
-@pytest.mark.parametrize("M,N,K,rows", [(32, 100, 512, (0, 100)), (64, 200, 512, (32, 160)), (256, 96, 256, (48, 96))])
-def test_dense_wgrad_adam_fused_and_rows(ctx, M, N, K, rows):
-    """Fused dense wgrad + TF-Adam (mma.sync gradient inside the optimizer pass): whole matrix (M <= 32) and the
-    data-parallel row-slice form with a gathered batch, against f32 torch math on the same bf16 operands."""
+def test_dense_wgrad_adam_fused(ctx):
+    """Fused dense wgrad + TF-Adam (mma.sync gradient inside the optimizer pass) against f32 torch math on the same
+    bf16 operands."""
+    M, N, K = 32, 100, 512
     g = torch.Generator().manual_seed(50)
     x = bf16_rand(M, K, seed=51)
     lddy = (N + 7) // 8 * 8
@@ -739,52 +739,26 @@ def test_dense_wgrad_adam_fused_and_rows(ctx, M, N, K, rows):
     m1 = b1 * m0 + (1 - b1) * grad
     v1 = b2 * v0 + (1 - b2) * grad * grad
     w1 = w0 - ops.adam_lr_t(lr, b1, b2, t) * m1 / (v1.sqrt() + eps)
-    lo, hi = rows
     w, m, v = w0.clone(), m0.clone(), v0.clone()
     wb = torch.zeros(N, K, dtype=torch.bfloat16, device=DEV)
-    ctx.dense_wgrad_adam_rows(x, dy, w, m, v, wb, lo, hi, lr, b1, b2, eps, t, gs, N=N)
-    assert torch.allclose(m[lo:hi], m1[lo:hi], rtol=1e-4, atol=1e-6)
-    assert torch.allclose(v[lo:hi], v1[lo:hi], rtol=1e-4, atol=1e-7)
-    assert torch.allclose(w[lo:hi], w1[lo:hi], rtol=1e-4, atol=1e-5)
-    assert torch.equal(wb[lo:hi], w[lo:hi].bfloat16())
-    keep = torch.ones(N, dtype=torch.bool, device=DEV)
-    keep[lo:hi] = False
-    assert torch.equal(w[keep], w0[keep]) and torch.equal(m[keep], m0[keep]) and float(wb[keep].abs().max() if keep.any() else 0) == 0
-    if M <= 32 and K % 256 == 0:
-        w, m, v = w0.clone(), m0.clone(), v0.clone()
-        db = torch.zeros(N, device=DEV)
-        ctx.dense_wgrad_adam(x, dy, db, w, m, v, wb, lr, b1, b2, eps, t, gs)
-        assert torch.allclose(w, w1, rtol=1e-4, atol=1e-5) and torch.allclose(m, m1, rtol=1e-4, atol=1e-6)
-        assert torch.allclose(db, dy[:, :N].float().sum(0), rtol=1e-3, atol=1e-3)
+    db = torch.zeros(N, device=DEV)
+    ctx.dense_wgrad_adam(x, dy, db, w, m, v, wb, lr, b1, b2, eps, t, gs)
+    assert torch.allclose(w, w1, rtol=1e-4, atol=1e-5) and torch.allclose(m, m1, rtol=1e-4, atol=1e-6)
+    assert torch.allclose(db, dy[:, :N].float().sum(0), rtol=1e-3, atol=1e-3)
 
 
-def test_dense_rows_update_with_rank_blocks(ctx):
-    """The gathered batch stored as rank blocks [x_r | dy_r] (one all-gather per layer, dp.dense_gather_adam) must
-    give the same update and bias gradient as the plain [M, ld] matrices."""
+def test_bias_grad_bf16_rank_blocks(ctx):
+    """a3d_bias_grad_bf16 over a batch stored as rank blocks [x_r | dy_r] (group_rows / group_stride) must give the
+    column sums of the plain [M, ld] matrix."""
     n, B, N, K = 4, 16, 96, 256
     lddy = 96
     x = bf16_rand(n * B, K, seed=60)
     dy = bf16_rand(n * B, lddy, seed=61)
-    g = torch.Generator().manual_seed(62)
-    w0 = torch.rand(N, K, generator=g).to(DEV)
-    m0 = (torch.rand(N, K, generator=g) * 0.1).to(DEV)
-    v0 = (torch.rand(N, K, generator=g) * 0.01).to(DEV)
-    args = (0.01, 0.9, 0.999, 1e-8, 2, 1.0 / n)
-    ref = [t.clone() for t in (w0, m0, v0)]
-    wb_ref = torch.zeros(N, K, dtype=torch.bfloat16, device=DEV)
-    ctx.dense_wgrad_adam_rows(x, dy, *ref, wb_ref, 16, 80, *args, N=N)
     blk = B * (K + lddy)
     gbuf = torch.zeros(n, blk, dtype=torch.bfloat16, device=DEV)
     for r in range(n):
         gbuf[r, :B * K] = x[r * B:(r + 1) * B].reshape(-1)
         gbuf[r, B * K:] = dy[r * B:(r + 1) * B].reshape(-1)
-    got = [t.clone() for t in (w0, m0, v0)]
-    wb = torch.zeros(N, K, dtype=torch.bfloat16, device=DEV)
-    ctx.dense_wgrad_adam_rows(gbuf.view(-1), gbuf.view(-1)[B * K:], *got, wb, 16, 80, *args, N=N, M=n * B, ldx=K, lddy=lddy,
-                              group_rows=B, x_group_stride=blk, dy_group_stride=blk)
-    for a, b in zip(got, ref):
-        assert torch.equal(a, b)
-    assert torch.equal(wb, wb_ref)
     db = torch.zeros(N, device=DEV)
     ctx.bias_grad_bf16(gbuf.view(-1)[B * K:], N, db, rows=n * B, ld=lddy, group_rows=B, group_stride=blk)
     assert torch.allclose(db, dy[:, :N].float().sum(0), rtol=1e-5, atol=1e-4)

@@ -43,8 +43,7 @@ def main():
     sep_a = lambda: ctx.adam_tf(w.view(-1), g.view(-1), m.view(-1), v.view(-1), wb.view(-1), 0.1, 0.9, 0.999, 1e-8, 1)
     sep_w(); sep_a(); torch.cuda.synchronize()
     tw, ta = timed(sep_w), timed(sep_a)
-    print(json.dumps({"cfg": os.environ.get("A3D_FUSED_ADAM_CFG", "default"), "variant": os.environ.get("A3D_FUSED_ADAM", "mma"),
-                      "fused_us": tf, "fused_GBs": 26.0 * N * K / tf / 1e3, "wgrad_us": tw, "adam_us": ta,
+    print(json.dumps({"fused_us": tf, "fused_GBs": 26.0 * N * K / tf / 1e3, "wgrad_us": tw, "adam_us": ta,
                       "adam_GBs": 30.0 * N * K / ta / 1e3}), flush=True)
 
 
