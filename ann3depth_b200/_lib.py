@@ -17,7 +17,7 @@ A3D_ENOTSUP = -5
 IMPL_AUTO, IMPL_SIMT, IMPL_TC = 0, 1, 2
 EPI_RELU, EPI_SIGMOID = 1, 2
 OP_FWD, OP_DGRAD, OP_WGRAD = 0, 1, 2
-DM_SCALE_NONE, DM_SCALE_MEDIAN = 0, 1
+DM_SCALE_NONE, DM_SCALE_MEDIAN, DM_SCALE_AFFINE = 0, 1, 2
 # a3d_depth_metrics slots (A3D_DM_*), in order
 DM_SLOTS = ("n", "abs_rel", "sq_rel", "sq", "log", "log_sq", "log10", "delta1", "delta2", "delta3", "nonfinite")
 

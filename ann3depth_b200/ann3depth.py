@@ -142,7 +142,7 @@ class Validator:
         self.eval_op = getattr(models, args.model)(inp.images, inp.depths, train=False)
         inp.close()
         self.eval_op.net.arena = op.net.arena
-        self.meters = evaluate.make_meters(self.eval_op, self.eval_op.net.ctx)
+        self.meters = evaluate.make_meters(self.eval_op, self.eval_op.net.ctx, getattr(args, "evalscale", "none"))
         self.last_step = None
 
     def _inputs(self):
@@ -288,6 +288,9 @@ def parse_args(argv=None):
     parser.add_argument("--timeout", "-k", default=4200, type=int, help="The time after which the process dies.")
     parser.add_argument("--evalfreq", default=0, type=int,
                         help="Evaluate the test split every N steps and at the last step (0: never; beyond the reference).")
+    parser.add_argument("--evalscale", default="none", choices=["none", "median", "affine"],
+                        help="Alignment of each prediction before the --evalfreq metrics, as evaluate --scale: median "
+                             "scale, or least-squares scale and shift per image (affine).")
     parser.add_argument("--augment", default="none", choices=["none", "eigen"],
                         help="Training-time augmentation: 'eigen' = random scale, rotation, crop, flip and colour of "
                              "Eigen et al. 2014, section 3.3, on the GPU (beyond the reference).")

@@ -14,6 +14,11 @@
 // so one barrier per pass separates the writers of pass p+1 from the readers of pass p.  A last pass applies the scale and
 // reduces the sums: float32 per-thread partials, combined across threads and across the cluster in float64 in a fixed
 // order (no float atomics), so a captured graph replays to identical sums.
+//
+// Affine (scale-and-shift) alignment: one pass of float64 per-thread moments (n, sum p~, sum g, sum p~^2, sum p~ g) and
+// the float32 min / max of p~ (an exact test for a constant p~, which the moments cannot give after rounding), reduced
+// in the same fixed order across warps and, after one cluster barrier, across the cluster: every CTA reads the S
+// partials over DSMEM in rank order, so all CTAs derive the same (s, t) before the final pass.
 #include "common.cuh"
 #include <cooperative_groups.h>
 #include <cmath>
@@ -86,6 +91,15 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
   return v;
 }
 
+__device__ __forceinline__ double warp_max_f64(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+
+// Alignment statistics of the affine mode: sums n, sum p~, sum g, sum p~^2, sum p~ g, then maxima -min p~, max p~.
+constexpr int kAlign = 7, kAlignSums = 5;
+
 // Block-wide exclusive scan of one value per thread; returns the prefix, `total` = the block's sum.
 __device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* warp_tot, uint32_t& total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -108,7 +122,7 @@ __device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* w
   return before + inc - v;
 }
 
-template <bool MEDIAN>
+template <int MODE>
 __global__ void __launch_bounds__(kThreads) depth_metrics_kernel(const float* __restrict__ pred, int ph, int pw,
                                                                  const float* __restrict__ gt, int gh, int gw, float lo,
                                                                  float hi, double* __restrict__ sums,
@@ -124,8 +138,8 @@ __global__ void __launch_bounds__(kThreads) depth_metrics_kernel(const float* __
 
   __shared__ uint32_t warp_tot[kThreads / 32];
   __shared__ double part[A3D_DM_SLOTS];
-  float s = 1.f;
-  if constexpr (MEDIAN) {
+  float s = 1.f, t = 0.f;
+  if constexpr (MODE == A3D_DM_SCALE_MEDIAN) {
     __shared__ uint32_t hist[2][2][kBins];       // [buffer][gt, p~][bin]
     __shared__ uint32_t found[2][2];             // [gt, p~][selected prefix, residual rank]
     uint32_t prefix[2] = {0u, 0u}, want[2] = {0u, 0u};
@@ -179,13 +193,66 @@ __global__ void __launch_bounds__(kThreads) depth_metrics_kernel(const float* __
     // the next cluster.sync (before the partial sums are read) also keeps every CTA's histograms alive until the last
     // remote read of them has finished
   }
+  if constexpr (MODE == A3D_DM_SCALE_AFFINE) {
+    uint32_t c = 0;
+    double sp = 0.0, sg = 0.0, spp = 0.0, spg = 0.0;
+    float pmin = INFINITY, pmax = -INFINITY;
+    for_pixels(begin, end, pred, ph, pw, gt, gw, sy, sx, lo, hi, [&](const Pixel& px) {
+      const double p = px.p, g = px.g;
+      c += 1;
+      sp += p;
+      sg += g;
+      spp += p * p;
+      spg += p * g;
+      pmin = fminf(pmin, px.p);
+      pmax = fmaxf(pmax, px.p);
+    });
+    const double vals[kAlign] = {(double)c, sp, sg, spp, spg, -(double)pmin, (double)pmax};
+    __shared__ double awarp[kThreads / 32][kAlign];
+    __shared__ double apart[kAlign], atot[kAlign];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < kAlign; ++k) {
+      double v = k < kAlignSums ? warp_sum_f64(vals[k]) : warp_max_f64(vals[k]);
+      if (lane == 0) awarp[warp][k] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < kAlign) {
+      const int k = threadIdx.x;
+      double v = awarp[0][k];
+      for (int w = 1; w < kThreads / 32; ++w) v = k < kAlignSums ? v + awarp[w][k] : fmax(v, awarp[w][k]);
+      apart[k] = v;
+    }
+    cluster.sync();                              // every CTA's partials are complete
+    if (threadIdx.x < kAlign) {
+      const int k = threadIdx.x;
+      double v = cluster.map_shared_rank(apart, 0)[k];
+      for (int r = 1; r < S; ++r) {
+        double x = cluster.map_shared_rank(apart, r)[k];
+        v = k < kAlignSums ? v + x : fmax(v, x);
+      }
+      atot[k] = v;
+    }
+    __syncthreads();
+    // the same float64 arithmetic on the same totals in every thread of every CTA; the final pass's cluster.sync keeps
+    // apart alive until the last remote read of it has finished
+    const double n = atot[0];
+    if (n > 0.0) {
+      const double mp = atot[1] / n, mg = atot[2] / n;
+      const double sxx = atot[3] - atot[1] * mp, sxy = atot[4] - atot[1] * mg;
+      const double sd = (-atot[5] < atot[6] && sxx > 0.0) ? sxy / sxx : 1.0;
+      s = (float)sd;
+      t = (float)(mg - sd * mp);
+    }
+  }
 
   // final pass: per-thread float32 partials
   float f_abs = 0.f, f_sqrel = 0.f, f_sq = 0.f, f_d = 0.f, f_d2 = 0.f, f_l10 = 0.f;
   uint32_t c_n = 0, c_d1 = 0, c_d2 = 0, c_d3 = 0, c_nf = 0;
   for_pixels(begin, end, pred, ph, pw, gt, gw, sy, sx, lo, hi, [&](const Pixel& px) {
     float p = px.p, g = px.g;
-    if constexpr (MEDIAN) p = fminf(fmaxf(s * p, lo), hi);
+    if constexpr (MODE == A3D_DM_SCALE_MEDIAN) p = fminf(fmaxf(s * p, lo), hi);
+    if constexpr (MODE == A3D_DM_SCALE_AFFINE) p = fminf(fmaxf(__fadd_rn(__fmul_rn(s, p), t), lo), hi);
     float q = p / g, qi = g / p;
     float diff = p - g, rel = q - 1.f;
     float d = logf(q);
@@ -225,7 +292,14 @@ __global__ void __launch_bounds__(kThreads) depth_metrics_kernel(const float* __
       for (int r = 0; r < S; ++r) v += cluster.map_shared_rank(part, r)[threadIdx.x];
       sums[(size_t)b * A3D_DM_SLOTS + threadIdx.x] = v;
     }
-    if (threadIdx.x == 0 && scale_out) scale_out[b] = s;
+    if (threadIdx.x == 0 && scale_out) {
+      if constexpr (MODE == A3D_DM_SCALE_AFFINE) {
+        scale_out[2 * b] = s;
+        scale_out[2 * b + 1] = t;
+      } else {
+        scale_out[b] = s;
+      }
+    }
   }
   cluster.sync();                                // rank 0's remote reads are done before any CTA exits
 }
@@ -246,7 +320,8 @@ extern "C" int a3d_depth_metrics(a3d_ctx* ctx, const float* pred, int B, int ph,
               "depth_metrics: bad shape");
   A3D_REQUIRE(min_depth > 0.f && min_depth < max_depth && std::isfinite(max_depth),
               "depth_metrics: need 0 < min_depth < max_depth (finite)");
-  A3D_REQUIRE(scale_mode == A3D_DM_SCALE_NONE || scale_mode == A3D_DM_SCALE_MEDIAN, "depth_metrics: bad scale_mode");
+  A3D_REQUIRE(scale_mode == A3D_DM_SCALE_NONE || scale_mode == A3D_DM_SCALE_MEDIAN || scale_mode == A3D_DM_SCALE_AFFINE,
+              "depth_metrics: bad scale_mode");
   const int S = cluster_size_for(ctx, B);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(B * S);
@@ -258,11 +333,14 @@ extern "C" int a3d_depth_metrics(a3d_ctx* ctx, const float* pred, int B, int ph,
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   if (scale_mode == A3D_DM_SCALE_MEDIAN)
-    A3D_CHECK_CUDA(cudaLaunchKernelEx(&cfg, depth_metrics_kernel<true>, pred, ph, pw, gt, gh, gw, min_depth, max_depth,
-                                      sums, scale));
+    A3D_CHECK_CUDA(cudaLaunchKernelEx(&cfg, depth_metrics_kernel<A3D_DM_SCALE_MEDIAN>, pred, ph, pw, gt, gh, gw,
+                                      min_depth, max_depth, sums, scale));
+  else if (scale_mode == A3D_DM_SCALE_AFFINE)
+    A3D_CHECK_CUDA(cudaLaunchKernelEx(&cfg, depth_metrics_kernel<A3D_DM_SCALE_AFFINE>, pred, ph, pw, gt, gh, gw,
+                                      min_depth, max_depth, sums, scale));
   else
-    A3D_CHECK_CUDA(cudaLaunchKernelEx(&cfg, depth_metrics_kernel<false>, pred, ph, pw, gt, gh, gw, min_depth, max_depth,
-                                      sums, scale));
+    A3D_CHECK_CUDA(cudaLaunchKernelEx(&cfg, depth_metrics_kernel<A3D_DM_SCALE_NONE>, pred, ph, pw, gt, gh, gw,
+                                      min_depth, max_depth, sums, scale));
   A3D_LAUNCH_OK(ctx);
   return 0;
 }

@@ -7,10 +7,13 @@ sums (include/a3d.h); `update` adds them to a float64 device vector without a ho
 the ranks (gloo), `result` turns it into the metrics.  Dataset metrics pool all valid pixels of all images (abs_rel,
 sq_rel, rmse, rmse_log, log10, delta1-3); silog = sqrt(mean d^2 - (mean d)^2), d = ln p - ln g, is taken per image and
 averaged over the images with a valid pixel.  The defaults suit the reference's data: its depths are min-max byte-scaled
-relative depths k/255 (tools/data_tf_converter.py), so min_depth = 1e-3 excludes exactly the zeros.
+relative depths k/255 (tools/data_tf_converter.py), so min_depth = 1e-3 excludes exactly the zeros.  Because each
+ground truth is min-max scaled on its own, it is the true depth up to an unknown scale and shift per image:
+`--scale affine` fits both per image (least squares, as MiDaS does for relative depth) before the metrics, so they
+measure the model and not the lost affine map; `--scale median` removes a scale only.
 
     python -m ann3depth_b200.evaluate nyu --model msdn --ckptdir checkpoints --id run1 --batchsize 32 --datadir data
-                                          [--scale median] [--dtype fp8] [--json metrics.json]
+                                          [--scale median|affine] [--dtype fp8] [--json metrics.json]
 
 restores `<ckptdir>/<model>[_<id>]/model.ckpt` into the inference net and reads `<datadir>/<dataset>/test.tfrecords`
 once.  MSDN reports its two outputs `fine` (the reference's prediction) and `coarse`; DCNF its `output`.  Under
@@ -36,15 +39,16 @@ logger = logging.getLogger("ann3depth.evaluate")
 _NS = len(L.DM_SLOTS)
 _SILOG, _SILOG_IMAGES, _IMAGES = _NS, _NS + 1, _NS + 2
 METRICS = ("abs_rel", "sq_rel", "rmse", "rmse_log", "log10", "silog", "delta1", "delta2", "delta3")
+SCALES = ("none", "median", "affine")
 
 
 class DepthMetrics:
     """Accumulator of the metrics of one prediction stream.  ctx: ops.Context (None: `add_sums` only)."""
 
     def __init__(self, ctx, min_depth=1e-3, max_depth=1.0, scale="none", device=None):
-        if scale not in ("none", "median"):
-            raise ValueError("scale must be 'none' or 'median'")
-        self.ctx, self.min_depth, self.max_depth, self.median = ctx, float(min_depth), float(max_depth), scale == "median"
+        if scale not in SCALES:
+            raise ValueError("scale must be 'none', 'median' or 'affine'")
+        self.ctx, self.min_depth, self.max_depth, self.scale = ctx, float(min_depth), float(max_depth), scale
         if device is None:
             device = f"cuda:{ctx.device}" if ctx is not None else "cpu"
         self.acc = torch.zeros(_NS + 3, dtype=torch.float64, device=device)
@@ -60,7 +64,8 @@ class DepthMetrics:
             return
         if self._sums is None or self._sums.shape[0] < n:
             self._sums = torch.empty(pred.shape[0], _NS, dtype=torch.float64, device=pred.device)
-        sums = self.ctx.depth_metrics(pred[:n], gt[:n], self.min_depth, self.max_depth, self.median, sums=self._sums[:n])
+        sums = self.ctx.depth_metrics(pred[:n], gt[:n], self.min_depth, self.max_depth, median=self.scale == "median",
+                                      affine=self.scale == "affine", sums=self._sums[:n])
         self.add_sums(sums)
 
     def add_sums(self, sums):
@@ -174,7 +179,9 @@ def parse_args(argv=None):
     p.add_argument("--id", default="", type=str, help="Checkpoint path suffix (as for training).")
     p.add_argument("--batchsize", "-b", default=32, type=int)
     p.add_argument("--datadir", "-d", default="data", type=str, help="The data directory containing the datasets.")
-    p.add_argument("--scale", default="none", choices=("none", "median"), help="Median-scale each prediction first.")
+    p.add_argument("--scale", default="none", choices=SCALES,
+                   help="Align each prediction to its ground truth first: median = median scaling, affine = "
+                        "least-squares scale and shift (for relative depth known only up to both).")
     p.add_argument("--min-depth", default=1e-3, type=float, help="Valid pixels: min_depth < gt <= max_depth.")
     p.add_argument("--max-depth", default=1.0, type=float)
     p.add_argument("--dtype", default="bf16", choices=("bf16", "fp8"),

@@ -714,9 +714,10 @@ class Context:
         return g_src
 
     # ------------------------------------------------------------------ evaluation
-    def depth_metrics(self, pred, gt, min_depth, max_depth, median=False, sums=None, scale=None):
+    def depth_metrics(self, pred, gt, min_depth, max_depth, median=False, sums=None, scale=None, affine=False):
         """pred f32 [B,ph,pw(,1)], gt f32 [B,gh,gw(,1)] -> sums f64 [B, len(L.DM_SLOTS)] (a3d_depth_metrics);
-        `scale` f32 [B] (optional) receives the median scale."""
+        `median=True`: median scaling, `scale` f32 [B] (optional) receives s.  `affine=True`: per-image least-squares
+        scale and shift, `scale` f32 [B,2] (optional) receives (s, t)."""
         B, ph, pw = pred.shape[:3]
         gh, gw = gt.shape[1:3]
         if gt.shape[0] != B or pred.dim() == 4 and pred.shape[3] != 1 or gt.dim() == 4 and gt.shape[3] != 1:
@@ -724,9 +725,14 @@ class Context:
         for t in (pred, gt):
             if t.dtype != torch.float32 or not t.is_cuda or not t.is_contiguous():
                 raise ValueError("depth_metrics: pred and gt must be contiguous float32 CUDA tensors")
+        if median and affine:
+            raise ValueError("depth_metrics: median and affine are exclusive")
+        if affine and scale is not None and (scale.dtype != torch.float32 or tuple(scale.shape) != (B, 2)
+                                             or not scale.is_contiguous()):
+            raise ValueError("depth_metrics: affine scale must be a contiguous float32 tensor [B, 2]")
         if sums is None:
             sums = torch.empty(B, len(L.DM_SLOTS), dtype=torch.float64, device=pred.device)
-        mode = L.DM_SCALE_MEDIAN if median else L.DM_SCALE_NONE
+        mode = L.DM_SCALE_AFFINE if affine else L.DM_SCALE_MEDIAN if median else L.DM_SCALE_NONE
         L.check(self.lib.a3d_depth_metrics(self.h, _ptr(pred), B, ph, pw, _ptr(gt), gh, gw, min_depth, max_depth, mode,
                                            _ptr(sums), _ptr(scale), _stream()), "depth_metrics")
         return sums

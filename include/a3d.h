@@ -343,11 +343,20 @@ int a3d_window_scatter_sum(a3d_ctx*, const uint16_t* g_out, int B, int Hs, int W
  * (0 < min_depth < max_depth).  p~ = the sampled prediction clamped to [min_depth, max_depth]; a NaN maps to min_depth.
  * scale_mode A3D_DM_SCALE_NONE: p = p~.  A3D_DM_SCALE_MEDIAN: s = median(gt) / median(p~) over the valid pixels (float32
  * division of the two exact lower medians, the elements of rank floor((n-1)/2)), p = clamp(s * p~); s = 1 for an image
- * without a valid pixel.  With d = ln p - ln g, writes sums[b][A3D_DM_*] (float64, overwritten per image) over the
- * valid pixels, and scale[b] = s if `scale` is non-null.  The ratio tests are float32: max(p/g, g/p) < 1.25^k.
+ * without a valid pixel.  A3D_DM_SCALE_AFFINE (for relative depth, known only up to a scale and shift per image):
+ * (s, t) = argmin sum (s * p~ + t - g)^2 over the valid pixels, in float64 from the raw moments:
+ *   n, mp = sum p~ / n, mg = sum g / n, Sxx = sum p~^2 - sum p~ * mp, Sxy = sum p~ g - sum p~ * mg,
+ *   sd = Sxy / Sxx (may be negative), or sd = 1 when min p~ = max p~ or Sxx <= 0 (a constant prediction),
+ *   s = float32(sd), t = float32(mg - sd * mp);  s = 1, t = 0 for an image without a valid pixel;
+ *   p = fminf(fmaxf(float32(float32(s * p~) + t), min_depth), max_depth) (two float32 roundings, no fused
+ *   multiply-add; a NaN maps to min_depth).
+ * With d = ln p - ln g, writes sums[b][A3D_DM_*] (float64, overwritten per image) over the
+ * valid pixels, and if `scale` is non-null: scale[b] = s (NONE, MEDIAN) or scale[b][0..1] = (s, t) (AFFINE, [B][2]).
+ * The ratio tests are float32: max(p/g, g/p) < 1.25^k.
  * No workspace, no host sync, CUDA-graph capturable; the sums do not depend on scheduling (fixed reduction order). */
 #define A3D_DM_SCALE_NONE    0
 #define A3D_DM_SCALE_MEDIAN  1
+#define A3D_DM_SCALE_AFFINE  2
 #define A3D_DM_N          0   /* number of valid pixels */
 #define A3D_DM_ABS_REL    1   /* sum |p - g| / g */
 #define A3D_DM_SQ_REL     2   /* sum (p - g)^2 / g */

@@ -1,16 +1,18 @@
-"""Cost of evaluation: a3d_depth_metrics alone (CUDA events over many launches, both scale modes) at the shapes the two
+"""Cost of evaluation: a3d_depth_metrics alone (CUDA events over many launches, each scale mode) at the shapes the two
 models evaluate, and evaluation throughput with device-resident batches against inference alone.
 
   MSDN: B = 32, prediction 55x74 into 480x640 ground truth;  DCNF: B = 16, 240x320 into 480x640.
 
-Algorithmic bytes = one read of the ground truth and of the prediction plus the sums written (the kernel reads the ground
-truth 1x without and 4x with median scaling; repeated reads of one image come from L2).  The ground truth rotates over
-enough copies (> 126 MB of L2) that every launch reads its image from HBM the first time.  The card's name, power limit
-and maximum SM clock are read in the same run.  Usage: python tools/eval_bench.py [--out PATH]
+Algorithmic bytes = one read of the ground truth and of the prediction plus the sums written (the kernel reads the
+ground truth 1x without scaling, 2x with affine and 4x with median scaling; repeated reads of one image come from L2).
+The ground truth rotates over enough copies (> 126 MB of L2) that every launch reads its image from HBM the first time.
+The kernel modes alternate over --rounds rounds per shape; "us" is the median round, "us_rounds" all of them.  The
+card's name, power limit and maximum SM clock are read in the same run.  Usage: python tools/eval_bench.py [--out PATH]
 """
 import argparse
 import json
 import os
+import statistics
 import subprocess
 import sys
 
@@ -42,19 +44,32 @@ def time_ms(fn, iters):
     return e0.elapsed_time(e1) / iters
 
 
-def kernel_case(ctx, B, ph, pw, gh, gw, median, iters):
+SCALES = ("none", "median", "affine")
+
+
+def kernel_cases(ctx, B, ph, pw, gh, gw, iters, rounds):
     g = torch.Generator(device="cuda").manual_seed(0)
     copies = max(2, -(-160 * 2 ** 20 // (B * gh * gw * 4)))
     gts = [torch.randint(1, 256, (B, gh, gw), device="cuda", generator=g).float() / 255.0 for _ in range(copies)]
     pred = torch.rand(B, ph, pw, device="cuda", generator=g)
     sums = torch.empty(B, 11, dtype=torch.float64, device="cuda")
-    scale = torch.empty(B, device="cuda")
-    ms = time_ms(lambda i: ctx.depth_metrics(pred, gts[i % copies], 1e-3, 1.0, median=median, sums=sums, scale=scale),
-                 iters)
+    scales = {"none": torch.empty(B, device="cuda"), "median": torch.empty(B, device="cuda"),
+              "affine": torch.empty(B, 2, device="cuda")}
+    times = {m: [] for m in SCALES}
+    for _ in range(rounds):
+        for m in SCALES:
+            times[m].append(time_ms(lambda i: ctx.depth_metrics(pred, gts[i % copies], 1e-3, 1.0, median=m == "median",
+                                                                affine=m == "affine", sums=sums, scale=scales[m]),
+                                    iters))
     nbytes = B * (gh * gw + ph * pw) * 4 + sums.numel() * 8
-    return {"B": B, "pred": [ph, pw], "gt": [gh, gw], "scale": "median" if median else "none", "us": ms * 1e3,
-            "algorithmic_bytes": nbytes, "GB_per_s": nbytes / ms / 1e6, "share_of_hbm": nbytes / ms / 1e9 / HBM_TBS,
-            "gt_copies_rotated": copies}
+    out = []
+    for m in SCALES:
+        ms = statistics.median(times[m])
+        out.append({"B": B, "pred": [ph, pw], "gt": [gh, gw], "scale": m, "us": ms * 1e3,
+                    "us_rounds": [t * 1e3 for t in times[m]], "algorithmic_bytes": nbytes,
+                    "GB_per_s": nbytes / ms / 1e6, "share_of_hbm": nbytes / ms / 1e9 / HBM_TBS,
+                    "gt_copies_rotated": copies})
+    return out
 
 
 def throughput(model, B, iters):
@@ -66,7 +81,7 @@ def throughput(model, B, iters):
     outs = {"fine": op.outputs, "coarse": op.coarse} if model == "msdn" else {"output": op.outputs}
     res = {"B": B, "outputs": list(outs)}
     res["infer_ms"] = time_ms(lambda i: op.run(), iters)
-    for scale in ("none", "median"):
+    for scale in SCALES:
         meters = {k: DepthMetrics(op.net.ctx, scale=scale) for k in outs}
 
         def step(i):
@@ -85,14 +100,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="")
     ap.add_argument("--iters", type=int, default=200)
+    ap.add_argument("--rounds", type=int, default=5)
     args = ap.parse_args()
     ctx = models.get_context()
-    res = {"card": card(), "kernel": [], "throughput": {}}
+    res = {"card": card(), "kernel": [], "affine_over_none": {}, "throughput": {}}
     for B, ph, pw in ((32, 55, 74), (16, 240, 320), (1, 55, 74)):
-        for median in (False, True):
-            r = kernel_case(ctx, B, ph, pw, 480, 640, median, args.iters)
+        rs = {r["scale"]: r for r in kernel_cases(ctx, B, ph, pw, 480, 640, args.iters, args.rounds)}
+        for r in rs.values():
             res["kernel"].append(r)
             print(json.dumps(r), flush=True)
+        res["affine_over_none"][f"B{B} {ph}x{pw}"] = rs["affine"]["us"] / rs["none"]["us"]
+    print(json.dumps(res["affine_over_none"]), flush=True)
     for model, B in (("msdn", 32), ("dcnf", 16)):
         res["throughput"][model] = throughput(model, B, max(args.iters // 10, 10))
         print(model, json.dumps(res["throughput"][model]), flush=True)
