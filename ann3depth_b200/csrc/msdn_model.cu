@@ -9,8 +9,8 @@
 // host synchronisation and no allocation, i.e. it is CUDA-graph capturable once the first (autotuning) call is done.
 // Schedule: the sequential single-stream form of ann3depth_b200/msdn.py (forward of both stacks + both losses; backward
 // of the active tf.case branch with the dense weight gradients fused into TF-Adam; TF-Adam of the branch's groups;
-// global_step += 1).  BF16 storage, tcgen05 kernels.  The Python host adds the multi-stream overlap, data parallelism
-// and the TF32 mode on top of the same kernels.
+// global_step += 1).  BF16 storage, tcgen05 kernels.  The Python host adds the multi-stream overlap (stream placement as
+// annotations on the same launch sequence: msdn.py's _Lanes), data parallelism and the TF32 mode on top of the same kernels.
 #include "common.cuh"
 #include <math.h>
 #include <string.h>

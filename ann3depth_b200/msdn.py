@@ -7,6 +7,7 @@ stream; PyTorch only owns the buffers.  The whole step is captured in a CUDA gra
 """
 from __future__ import annotations
 
+import contextlib
 import os
 
 import torch
@@ -35,6 +36,79 @@ def phase_of(global_step: int, batchsize: int) -> int:
     if global_step < steps_coarse + steps_fine:
         return 2
     return 3
+
+
+class _Lanes:
+    """Stream placement of the phase-1 training step with `MSDNNet.overlap`, written as annotations on its one launch
+    sequence.  The main stream (HIGH PRIORITY: freed SM slots go to its pending CTAs first; graph capture keeps the
+    priority as a kernel-node attribute) carries the critical path: resize, coarse forward and loss, the dgrad chain.
+    "fine" takes the depth target, the dropout mask and the fine forward + loss, later the conv bias gradients; "wgrad"
+    the dense weight gradients and updates; "cwgrad" the conv weight gradients.  Each side stream forks from the step's
+    start and joins the main stream before the step counter moves, and sets its own `ctx.ws_tag`: concurrent launches
+    must not share scratch.  `lane(name, *labels)` runs a block on that stream behind the events `mark(label)` recorded
+    (labels never marked are skipped).  _SEQUENTIAL, with all of it a no-op, runs every launch on the current stream."""
+    SIDES = ("fine", "wgrad", "cwgrad")
+
+    def __init__(self, net=None):
+        self.on, self.net, self.events = net is not None, net, {}
+
+    def __enter__(self):
+        if self.on:
+            net = self.net
+            if net._streams is None:
+                net._streams = {"main": torch.cuda.Stream(device=net.dev, priority=-1),
+                                **{k: torch.cuda.Stream(device=net.dev) for k in self.SIDES}}
+            self.caller, start = torch.cuda.current_stream(), self._record()
+            self._main = torch.cuda.stream(net._streams["main"])
+            self._main.__enter__()
+            for st in net._streams.values():
+                st.wait_event(start)
+        return self
+
+    def __exit__(self, *exc):
+        if self.on:
+            end = self._record()
+            self._main.__exit__(*exc)
+            self.caller.wait_event(end)
+
+    @contextlib.contextmanager
+    def lane(self, name, *after):
+        if not self.on:
+            yield
+            return
+        ctx = self.net.ctx
+        tag, ctx.ws_tag = ctx.ws_tag, "" if name == "main" else name
+        try:
+            with torch.cuda.stream(self.net._streams[name]):
+                self.wait(*after)
+                yield
+        finally:
+            ctx.ws_tag = tag
+
+    @staticmethod
+    def _record(stream=None):
+        e = torch.cuda.Event()
+        e.record(stream)
+        return e
+
+    def mark(self, label):
+        if self.on:
+            self.events[label] = self._record()
+
+    def event(self, label):
+        return self.events.get(label)
+
+    def wait(self, *labels):
+        for e in filter(None, map(self.events.get, labels)):
+            torch.cuda.current_stream().wait_event(e)
+
+    def join(self):
+        if self.on:
+            for k in self.SIDES:
+                torch.cuda.current_stream().wait_event(self._record(self.net._streams[k]))
+
+
+_SEQUENTIAL = _Lanes()
 
 
 class MSDNNet:
@@ -74,13 +148,13 @@ class MSDNNet:
             if comm is not None:
                 raise ValueError("dtype='tf32' is a single-GPU precision mode")
             overlap, fuse_dense_adam = False, False
-        self.overlap = overlap                # phase-1 step on several streams (see _enqueue_phase1_overlapped)
+        self.overlap = overlap                # phase-1 step on four streams (see _Lanes)
         # single GPU: the dense weight gradients (32 FMAs per parameter at batch 32) are recomputed on the CUDA cores
         # inside the HBM-bound TF-Adam pass (a3d_dense_wgrad_adam), so the 67 M-element f32 gradient is never written
         # or re-read: 26 instead of 38 bytes per dense parameter and step.  Data parallel runs need the gradient in
         # memory for the reduce-scatter and keep the separate kernels (dp.py shards the optimizer instead).
         self.fuse_dense_adam = fuse_dense_adam
-        self._s_fine = self._s_wgrad = self._s_cwgrad = None
+        self._streams = None          # the phase-1 step's streams (_Lanes), created on first use
         self._wflip = None            # flipped filters of the stride-1 dgrads (refreshed at the start of every step)
         self.dev = torch.device(f"cuda:{ctx.device}")
         self.in_hw, self.depth_hw = in_hw, depth_hw
@@ -270,23 +344,28 @@ class MSDNNet:
             self.ctx.resize_bilinear_tf1(self.depths, OUT_H, OUT_W, out=self.tar)
 
     # ------------------------------------------------------------------ forward
-    def forward(self):
-        """src/models.py:281-290.  Reads self.images / self.depths, fills self.coarse / self.fine / losses."""
+    def forward(self, lanes=None):
+        """src/models.py:281-290.  Reads self.images / self.depths, fills self.coarse / self.fine / losses.  `lanes`: the
+        step's stream placement (_Lanes); by default every launch runs on the current stream."""
         if self.fp8:
             return self._forward_fp8()
         self.ctx.tf32x3 = self.x3
         try:
-            self._forward()
+            self._forward(lanes or _SEQUENTIAL)
         finally:
             self.ctx.tf32x3 = False
 
-    def _forward(self):
+    def _forward(self, s):
         c, B = self.ctx, self.B
         K = "/kernel"
         if self.augment is not None:
-            self._augment_draw()
+            self._augment_draw()                        # the transform both resizes apply
+            s.mark("draw")
         self._resize_image()
-        self._resize_target()
+        c.stamp("resize done")
+        s.mark("img")
+        with s.lane("fine", "draw"):
+            self._resize_target()
         # coarse (src/models.py:208-236)
         n = "coarse/conv/conv2d_"
         c.conv2d_fwd(self.d_c0, self.img4, self.w(n + "0" + K), self.bias(n + "0"), relu=True, out=self.c0)
@@ -302,29 +381,49 @@ class MSDNNet:
         c.conv2d_fwd(self.d_c2, self.p1, self.w(n + "2" + K), self.bias(n + "2"), relu=True, out=self.c2)
         c.conv2d_fwd(self.d_c3, self.c2, self.w(n + "3" + K), self.bias(n + "3"), relu=True, out=self.c3)
         c.conv2d_fwd(self.d_c4, self.c3, self.w(n + "4" + K), self.bias(n + "4"), relu=True, out=self.c4)
+        c.stamp("coarse conv fwd done")
         mask = None
         if self.train:
-            if not self.external_mask:
-                c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
+            with s.lane("fine"):
+                if not self.external_mask:
+                    c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
+                s.mark("aux")
+                if s.on:
+                    # flipped filters of the stride-1 dgrads (weights are final since the previous step's Adam): three
+                    # small transposes that would otherwise sit inside the dgrad chain
+                    flip = (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1))
+                    if self._wflip is None:
+                        self._wflip = {i: c.conv2d_dgrad_prepare(d, self.w(n + i + K)) for i, d in flip}
+                    for i, d in flip:
+                        c.conv2d_dgrad_prepare(d, self.w(n + i + K), out=self._wflip[i])
+                    s.mark("flip")
             mask = self.keep_mask
+        s.wait("aux", "published")
         n = "coarse/dense/dense_"
         c.dense_fwd(self.c4.view(B, 12288), self.w(n + "0" + K), self.bias(n + "0"), flags=L.EPI_RELU, keep_mask=mask,
                     drop_rate=0.5, out=self.d0, impl=self.impl)
         c.dense_fwd(self.d0, self.w(n + "1" + K), self.bias(n + "1"), flags=0, out=self.coarse, impl=self.impl)
-        # fine (src/models.py:238-253)
-        c.conv2d_pool4_fwd(self.d_f1, self.img4, self.wbig, self.bias("fine/first/conv2d"), relu=True, out=self.cat,
-                           idx=self.if1 if self.train else None)
-        c.scatter_channel_bf16(self.coarse, self.cat, 63)
-        c.conv2d_fwd(self.d_f2, self.cat, self.w("fine/second/conv2d" + K), self.bias("fine/second/conv2d"), relu=True,
-                     out=self.f2)
-        c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third" + K), self.bias("fine/third"), relu=False,
-                     out=self.fine.view(B, 55, 74, 1))
+        c.stamp("dense fwd done")
+        s.mark("coarse")
+        # fine (src/models.py:238-253): the first conv + pool needs only the image, the rest the coarse map too
+        with s.lane("fine", "img"):
+            c.conv2d_pool4_fwd(self.d_f1, self.img4, self.wbig, self.bias("fine/first/conv2d"), relu=True, out=self.cat,
+                               idx=self.if1 if self.train else None)
+            c.stamp("fine/first done")
+            s.wait("coarse")
+            c.scatter_channel_bf16(self.coarse, self.cat, 63)
+            c.conv2d_fwd(self.d_f2, self.cat, self.w("fine/second/conv2d" + K), self.bias("fine/second/conv2d"),
+                         relu=True, out=self.f2)
+            c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third" + K), self.bias("fine/third"), relu=False,
+                         out=self.fine.view(B, 55, 74, 1))
         # losses (src/models.py:288-290); the gradient of the active branch is produced in the same pass
         gk = "dout" if self.tf32 else "dout_bf16"          # the gradient w.r.t. the prediction, in the storage type
         c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse,
                      loss=self.loss_coarse, dout_ld=4096, **{gk: self.g_coarse if self.train else None})
-        c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
-                     dout_ld=N_PIX, **{gk: self.g_fine if self.train else None})
+        with s.lane("fine"):
+            c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
+                         dout_ld=N_PIX, **{gk: self.g_fine if self.train else None})
+            c.stamp("fine fwd + loss done")
 
     def _forward_fp8(self):
         """The inference forward on E4M3 operands.  Storage points (oracle/fp8.py restates them): the resized image with
@@ -367,57 +466,146 @@ class MSDNNet:
         c, a, g = self.ctx, self.arena, "CoarseDense"
         kn, bn_ = "coarse/dense/dense_" + layer + "/kernel", "coarse/dense/dense_" + layer + "/bias"
         rr = self._real_rows
+        c.stamp(f"dense_{layer} wgrad+adam begin")
         c.dense_wgrad_adam(x, dy, self.gw(bn_), rr(a.w, kn), rr(a.m, kn), rr(a.v, kn), rr(a.wb, kn),
                            ADAM_LR[g], ADAM_BETA1, self.beta2, ADAM_EPS, max(self.adam_t[g], 1), 1.0,
                            lr_t_dev=self.lr_dev[g])
         s = a.specs[bn_]
-        sl = slice(s.offset, s.offset + s.size)
-        c.adam_tf(a.w[sl], a.g[sl], a.m[sl], a.v[sl], a.wb[sl], ADAM_LR[g], ADAM_BETA1, self.beta2, ADAM_EPS,
-                  max(self.adam_t[g], 1), 1.0, lr_t_dev=self.lr_dev[g])
+        self.adam_range(g, s.offset, s.offset + s.size)
+        c.stamp(f"dense_{layer} wgrad+adam end")
 
-    def backward_coarse(self, fused_dense_adam=False):
+    def backward_coarse(self, fused_dense_adam=False, lanes=None):
         """d loss_coarse / d coarse variables (compute_gradients of src/models.py:319-324).  With
         `fused_dense_adam` the two dense kernels are updated on the spot (see _dense_wgrad_adam) and the caller
-        applies Adam to the CoarseConv group only."""
-        c, B, K = self.ctx, self.B, "/kernel"
-        hook = self.comm.bucket_ready if self.comm else (lambda *_: None)
+        applies Adam to the CoarseConv group only.  On four streams (`lanes`) every weight gradient runs as soon as its dY
+        exists and each optimizer group's update right behind its last weight gradient, so the HBM-bound Adam of the
+        67 M dense parameters and the small-grid wgrad kernels run under the tensor-bound dgrad chain."""
+        c, B, K, comm = self.ctx, self.B, "/kernel", self.comm
+        s = lanes or _SEQUENTIAL
+        hook = comm.bucket_ready if comm and not s.on else (lambda *_: None)   # sequential DP: allreduce now, Adam later
         n = "coarse/dense/dense_"
-        if not fused_dense_adam:
-            c.dense_wgrad(self.d0, self.g_coarse, dw=self.gw(n + "1" + K), db=self.gw(n + "1/bias"), impl=self.impl)
+        # data parallel on four streams, dense layers: exchange activations instead of gradients where the gathered batch
+        # allows it (dp.dense_gather_adam_merged), else reduce-scatter -> sharded TF-Adam -> all-gather (dp.sharded_adam)
+        gather = s.on and comm and all(comm.can_gather_dense(self, n + l + K, B) for l in "01")
+        sharded = s.on and comm and not gather
+        s.mark("loss")
+        if not fused_dense_adam and not gather:
+            with s.lane("wgrad", "loss"):
+                c.dense_wgrad(self.d0, self.g_coarse, dw=self.gw(n + "1" + K), db=self.gw(n + "1/bias"), impl=self.impl)
             hook(self, "dense_1")
         # dropout grad (mask * 1/(1-rate)) and relu grad (d0 > 0) ride in the dgrad's finishing pass
         c.dense_dgrad_act(self.g_coarse, self.w(n + "1" + K), self.d0, self.keep_mask, 0.5, L.EPI_RELU, out=self.g_d0,
                           impl=self.impl)
-        if fused_dense_adam:
-            self._dense_wgrad_adam("1", self.d0, self.g_coarse)
-        else:
-            c.dense_wgrad(self.c4.view(B, 12288), self.g_d0, dw=self.gw(n + "0" + K), db=self.gw(n + "0/bias"),
-                          impl=self.impl)
-            hook(self, "dense_0")
+        s.mark("dgrad dense_1")          # the last reader of dense_1's weights: its update may follow
+        if sharded:
+            with s.lane("wgrad"):
+                self._sharded_adam("1", s.event("dgrad dense_1"))
+        with s.lane("wgrad", "dgrad dense_1"):
+            if fused_dense_adam:
+                self._dense_wgrad_adam("1", self.d0, self.g_coarse)
+            elif not gather:
+                c.dense_wgrad(self.c4.view(B, 12288), self.g_d0, dw=self.gw(n + "0" + K), db=self.gw(n + "0/bias"),
+                              impl=self.impl)
+                hook(self, "dense_0")
         c.dense_dgrad_act(self.g_d0, self.w(n + "0" + K), self.c4.view(B, 12288), None, 0.0, L.EPI_RELU,
                           out=self.g_c4.view(B, 12288), impl=self.impl)
-        if fused_dense_adam:
-            self._dense_wgrad_adam("0", self.c4.view(B, 12288), self.g_d0)
+        s.mark("dgrad dense_0")
+        if gather:       # one all-gather of both layers' activations; each row update waits for its layer's dgrad
+            g_ = "CoarseDense"
+            comm.dense_gather_adam_merged(
+                self, [(n + "1" + K, n + "1/bias", self.d0, self.g_coarse, s.event("dgrad dense_1")),
+                       (n + "0" + K, n + "0/bias", self.c4.view(B, 12288), self.g_d0, s.event("dgrad dense_0"))],
+                g_, ADAM_LR[g_], ADAM_BETA1, ADAM_EPS, ready=s.event("dgrad dense_1"))
+        elif sharded:
+            with s.lane("wgrad"):
+                self._sharded_adam("0", s.event("dgrad dense_0"))
+        c.stamp("dense dgrad done")
+        with s.lane("wgrad", "dgrad dense_0"):
+            if fused_dense_adam:
+                self._dense_wgrad_adam("0", self.c4.view(B, 12288), self.g_d0)
+            elif s.on and not comm:      # under the conv backward, behind the last readers of the dense weights
+                self.apply_adam(("CoarseDense",))
         n = "coarse/conv/conv2d_"
+        # The bias gradients (latency-bound column sums of dY, 7-10 us each) run on the fine stream, whose forward work is
+        # long done by then: next to the wgrad GEMMs, not before them.  (Data parallel on four streams: measured slower at
+        # 2 GPUs, 1.184 vs 1.144 ms -- the comm stream's NCCL kernels already fill those gaps -- so there the conv wgrads
+        # keep their bias gradients.)
+        side_bias = not (s.on and comm)
 
-        def wgrad(desc, x, dy, name):
-            # bias gradient (a column sum of dY, not a tensor-core op) as its own call, like the multi-stream schedule
-            # does: bench.py's per-kernel table then times the wgrad GEMM alone
-            c.bias_grad_bf16(dy.view(-1, dy.shape[-1]), dy.shape[-1], self.gw(name + "/bias"))
-            c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=None)
-        wgrad(self.d_c4, self.c3, self.g_c4, n + "4")
+        def wgrad(desc, x, dy, name, after):
+            if side_bias:
+                with s.lane("fine", after):
+                    c.bias_grad_bf16(dy.view(-1, dy.shape[-1]), dy.shape[-1], self.gw(name + "/bias"))
+            with s.lane("cwgrad", after):
+                c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=None if side_bias else self.gw(name + "/bias"))
+        flip = self._wflip if s.on else {}
+        wgrad(self.d_c4, self.c3, self.g_c4, n + "4", "dgrad dense_0")
         c.conv2d_dgrad(self.d_c4, self.g_c4, self.w(n + "4" + K), out=self.g_c3, relu_src=self.c3)
-        wgrad(self.d_c3, self.c2, self.g_c3, n + "3")
-        c.conv2d_dgrad(self.d_c3, self.g_c3, self.w(n + "3" + K), out=self.g_c2, relu_src=self.c2)
-        wgrad(self.d_c2, self.p1, self.g_c2, n + "2")
-        c.conv2d_dgrad(self.d_c2, self.g_c2, self.w(n + "2" + K), out=self.g_p1)
+        c.stamp("dgrad conv2d_4 done")
+        s.mark("g_c3")
+        wgrad(self.d_c3, self.c2, self.g_c3, n + "3", "g_c3")
+        s.wait("flip")
+        c.conv2d_dgrad(self.d_c3, self.g_c3, self.w(n + "3" + K), out=self.g_c2, relu_src=self.c2, wflip=flip.get("3"))
+        s.mark("g_c2")
+        wgrad(self.d_c2, self.p1, self.g_c2, n + "2", "g_c2")
+        c.conv2d_dgrad(self.d_c2, self.g_c2, self.w(n + "2" + K), out=self.g_p1, wflip=flip.get("2"))
         c.maxpool2x2_idx_bwd(self.i1, self.g_p1, (self.B, 27, 37, 256), out=self.g_c1)
-        wgrad(self.d_c1, self.p0, self.g_c1, n + "1")
-        c.conv2d_dgrad(self.d_c1, self.g_c1, self.w(n + "1" + K), out=self.g_p0)
+        c.stamp("dgrad conv2d_3,2 + pool bwd done")
+        s.mark("g_c1")
+        # (DP: exchanging conv2d_4..2 here as an early bucket was measured SLOWER at 2 GPUs, 1.30 vs 1.26 ms: three more
+        # NCCL launches cost more than the shorter tail saves)
+        wgrad(self.d_c1, self.p0, self.g_c1, n + "1", "g_c1")
+        with s.lane("cwgrad"):
+            s.mark("wgrad conv2d_1")                       # gradients of conv2d_4 .. conv2d_1 are complete
+        c.conv2d_dgrad(self.d_c1, self.g_c1, self.w(n + "1" + K), out=self.g_p0, wflip=flip.get("1"))
         c.maxpool2x2_idx_bwd(self.i0, self.g_p0, (self.B, 55, 74, 96), out=self.g_c0)
-        wgrad(self.d_c0, self.img4, self.g_c0, n + "0")
-        self._mask_padding("coarse/conv/conv2d_0/kernel")
+        c.stamp("dgrad conv2d_1 + pool bwd done")
+        s.mark("g_c0")
+        # On four streams the CoarseConv update is cut at conv2d_0.  Single GPU: TF-Adam of conv2d_4 .. conv2d_1 (99 % of
+        # the group) runs on the idle fine stream next to conv2d_0's weight gradient; only conv2d_0's 55 k parameters are
+        # updated in the step's tail.  The group is one contiguous arena range in backward order, so this is the same
+        # update as one launch.
+        # Data parallel, the same cut: conv2d_4 .. conv2d_1 are all-reduced in f32 and updated behind conv2d_1's weight
+        # gradient, under conv2d_1's dgrad, the pool backward and conv2d_0's wgrad; the step's tail exchanges conv2d_0's
+        # 55 k parameters only.  (8 GPUs, profiles/step_timeline_r02_n8_rank0.json: the single 16 MB allreduce + Adam was
+        # ~150 us of exposed tail.)  f32 allreduce + replicated Adam beats cast + reduce-scatter + sharded Adam +
+        # all-gather at every world size (4 GPUs: 1.160 vs 1.185 ms; 2 GPUs, with the split: 0.972 vs 1.015 ms -- the
+        # collectives are latency-bound at 8-16 MB and the sharded form needs three of them); a sharded exchange of the
+        # split measured 1.20 against 1.18 ms unsplit at 2 GPUs (the extra NCCL kernels take SM slots from the GEMMs
+        # they overlap with).
+        lo, hi = self.arena.group_range("CoarseConv")
+        cut = self.arena.specs["coarse/conv/conv2d_0/kernel"].offset
+        inv_world = 1.0 / comm.world if comm else 1.0
+
+        def adam_cc(lo, hi):
+            self.adam_range("CoarseConv", lo, hi, inv_world)
+        if s.on and comm:
+            with s.lane("cwgrad"):
+                comm.bucket_ready(self, "coarse_conv_main", after=s.event("g_c0"), then=adam_cc)
+        elif s.on:       # conv2d_1's dgrad was the last reader of these weights
+            with s.lane("fine", "wgrad conv2d_1", "g_c0"):
+                adam_cc(lo, cut)
+        if side_bias:
+            with s.lane("fine", "g_c0"):
+                c.bias_grad_bf16(self.g_c0.view(-1, 96), 96, self.gw(n + "0/bias"))
+                s.mark("bias conv2d_0")
+        with s.lane("cwgrad", "g_c0"):
+            c.stamp("conv2d_0 wgrad + conv exchange/adam begin")
+            c.conv2d_wgrad(self.d_c0, self.img4, self.g_c0, dw=self.gw(n + "0" + K),
+                           db=None if side_bias else self.gw(n + "0/bias"))
+            s.wait("bias conv2d_0")
+            self._mask_padding("coarse/conv/conv2d_0/kernel")
+            if s.on and comm:
+                comm.bucket_ready(self, "coarse_conv_0", then=adam_cc)
+                comm.wait_all(self)
+            elif s.on:
+                adam_cc(cut, hi)
+            c.stamp("conv2d_0 wgrad + conv exchange/adam end")
         hook(self, "coarse_conv")
+
+    def _sharded_adam(self, layer, after):
+        g = "CoarseDense"
+        self.comm.sharded_adam(self, "dense_" + layer, g, ADAM_LR[g], ADAM_BETA1, ADAM_EPS, after)
 
     def backward_fine(self):
         """d loss_fine / d fine variables (src/models.py:334-338); the coarse map is a constant input."""
@@ -452,304 +640,49 @@ class MSDNNet:
     # ------------------------------------------------------------------ optimizer
     def apply_adam(self, groups, grad_scale=1.0):
         """apply_gradients of the two Adam instances of the active branch (src/models.py:326-331,340-345)."""
-        a = self.arena
         for g in groups:
-            lo, hi = a.group_range(g)
-            self.ctx.adam_tf(a.w[lo:hi], a.g[lo:hi], a.m[lo:hi], a.v[lo:hi], a.wb[lo:hi], ADAM_LR[g], ADAM_BETA1,
-                             self.beta2, ADAM_EPS, max(self.adam_t[g], 1), grad_scale, lr_t_dev=self.lr_dev[g])
+            self.adam_range(g, *self.arena.group_range(g), grad_scale)
 
     def adam_range(self, group, lo, hi, grad_scale=1.0):
         a = self.arena
         self.ctx.adam_tf(a.w[lo:hi], a.g[lo:hi], a.m[lo:hi], a.v[lo:hi], a.wb[lo:hi], ADAM_LR[group], ADAM_BETA1,
                          self.beta2, ADAM_EPS, max(self.adam_t[group], 1), grad_scale, lr_t_dev=self.lr_dev[group])
 
-    # ------------------------------------------------------------------ phase-1 step on four streams
-    def _enqueue_phase1_overlapped(self):
-        """Same launches as forward() + backward_coarse() + apply_adam(), arranged by data dependence:
-             main stream : resize, coarse forward, coarse loss, the dgrad chain (the critical path)
-             fine stream : fine forward + fine loss (needs only the image and the coarse map)
-             wgrad stream: every weight/bias gradient as soon as its dY exists, each optimizer group's
-                           gradient allreduce hand-off and TF-Adam right behind its last wgrad
-           so the HBM-bound Adam of the 67 M dense parameters and the small-grid wgrad kernels run under the
-           tensor-bound dgrad chain instead of after it.  Joins back before global_step += 1.
-        The main stream has HIGH PRIORITY: whenever an SM slot frees up, pending CTAs of the chain are placed before those
-        of the fine / wgrad / optimizer streams, which fill the remaining slots.  (CUDA graph capture keeps the priority
-        as a kernel-node attribute.)"""
-        c, B, K = self.ctx, self.B, "/kernel"
-        dev = self.dev
-        if self._s_fine is None:
-            self._s_main = torch.cuda.Stream(device=dev, priority=-1)
-            self._s_fine, self._s_wgrad = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
-            self._s_cwgrad = torch.cuda.Stream(device=dev)
-        cur = torch.cuda.current_stream()
-        e_in = torch.cuda.Event()
-        e_in.record(cur)
-        # s2: dense wgrads + dense Adam (HBM-bound) ; s3: conv wgrads + conv Adam (tensor / L2-bound)
-        s0, s1, s2, s3 = self._s_main, self._s_fine, self._s_wgrad, self._s_cwgrad
-        with torch.cuda.stream(s0):
-            s0.wait_event(e_in)
-            inv_world = 1.0 / self.comm.world if self.comm else 1.0
+    # ------------------------------------------------------------------ one session.run(model_op)
+    def _enqueue_step(self, phase):
+        s = _Lanes(self) if phase == 1 and self.overlap else _SEQUENTIAL
+        with s:
+            c = self.ctx
             if c.timeline is not None:
                 c.timeline.begin()
             c.stamp("step begin")
-            # data parallel: the dense rows other ranks updated in the PREVIOUS step arrive now, under this step's resize and
-            # convolution forward (dp.dense_gather_adam_merged / publish_rows); the dense forward waits for them
-            e_pub = self.comm.publish_rows(self) if self.comm else None
-
-            def dp_update(bucket, group, after=None):     # DP: reduce-scatter -> sharded TF-Adam -> all-gather (dp.py)
-                self.comm.sharded_adam(self, bucket, group, ADAM_LR[group], ADAM_BETA1, ADAM_EPS, after)
-            hook = self.comm.bucket_ready if self.comm else (lambda *_: None)
-
-            def mark(stream):
-                e = torch.cuda.Event()
-                e.record(stream)
-                return e
-
-            # ---- fine stream, part 0: what the critical path needs only later (depth target, dropout mask)
-            n0 = "coarse/conv/conv2d_"
-            e_start = mark(s0)
-            e_draw = None
-            if self.augment is not None:             # the transform both resizes apply
-                self._augment_draw()
-                e_draw = mark(s0)
-            for side in (s2, s3):                 # every side stream forks from the step's start (a stream that happens to
-                side.wait_event(e_start)          # get no work in some mode must still be part of the capture to be joined)
-            with torch.cuda.stream(s1):
-                s1.wait_event(e_start)
-                if e_draw is not None:
-                    s1.wait_event(e_draw)
-                self._resize_target()
-                if not self.external_mask:
-                    c.bernoulli_mask(self.keep_mask, 0.5, self.dropout_seed, self.step_dev)
-                e_aux = mark(s1)
-                # flipped filters of the stride-1 dgrads (weights are final since the previous step's Adam): three small
-                # transposes that used to sit inside the dgrad chain
-                if self._wflip is None:
-                    self._wflip = {}
-                    for i, dsc in (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1)):
-                        self._wflip[i] = c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K))
-                for i, dsc in (("3", self.d_c3), ("2", self.d_c2), ("1", self.d_c1)):
-                    c.conv2d_dgrad_prepare(dsc, self.w(n0 + i + K), out=self._wflip[i])
-                e_flip = mark(s1)
-            # ---- main: preprocessing
-            self._resize_image()
-            c.stamp("resize done")
-            e_img = mark(s0)
-            # ---- fine stream, part 1: first conv + pool need only the image
-            with torch.cuda.stream(s1):
-                c.ws_tag = "fine"
-                s1.wait_event(e_img)
-                c.conv2d_pool4_fwd(self.d_f1, self.img4, self.wbig, self.bias("fine/first/conv2d"), relu=True, out=self.cat,
-                                   idx=self.if1)
-                c.stamp("fine/first done")
-                c.ws_tag = ""
-            # ---- main: coarse forward
-            n = "coarse/conv/conv2d_"
-            c.conv2d_fwd(self.d_c0, self.img4, self.w(n + "0" + K), self.bias(n + "0"), relu=True, out=self.c0)
-            c.maxpool2x2_fwd_f32(self.c0, out=self.p0, idx=self.i0)
-            c.conv2d_fwd(self.d_c1, self.p0, self.w(n + "1" + K), self.bias(n + "1"), relu=True, out=self.c1)
-            c.maxpool2x2_fwd_f32(self.c1, out=self.p1, idx=self.i1)
-            c.conv2d_fwd(self.d_c2, self.p1, self.w(n + "2" + K), self.bias(n + "2"), relu=True, out=self.c2)
-            c.conv2d_fwd(self.d_c3, self.c2, self.w(n + "3" + K), self.bias(n + "3"), relu=True, out=self.c3)
-            c.conv2d_fwd(self.d_c4, self.c3, self.w(n + "4" + K), self.bias(n + "4"), relu=True, out=self.c4)
-            c.stamp("coarse conv fwd done")
-            s0.wait_event(e_aux)
-            if e_pub is not None:
-                s0.wait_event(e_pub)
-            nd = "coarse/dense/dense_"
-            c.dense_fwd(self.c4.view(B, 12288), self.w(nd + "0" + K), self.bias(nd + "0"), flags=L.EPI_RELU,
-                        keep_mask=self.keep_mask, drop_rate=0.5, out=self.d0, impl=self.impl)
-            c.dense_fwd(self.d0, self.w(nd + "1" + K), self.bias(nd + "1"), flags=0, out=self.coarse, impl=self.impl)
-            c.stamp("dense fwd done")
-            e_coarse = mark(s0)
-            # ---- fine stream, part 2
-            with torch.cuda.stream(s1):
-                c.ws_tag = "fine"
-                s1.wait_event(e_coarse)
-                c.scatter_channel_bf16(self.coarse, self.cat, 63)
-                c.conv2d_fwd(self.d_f2, self.cat, self.w("fine/second/conv2d" + K), self.bias("fine/second/conv2d"),
-                             relu=True, out=self.f2)
-                c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third" + K), self.bias("fine/third"), relu=False,
-                             out=self.fine.view(B, 55, 74, 1))
-                c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
-                             dout_bf16=self.g_fine)
-                c.stamp("fine fwd + loss done")
-                c.ws_tag = ""
-                e_fine = mark(s1)
-            # ---- main: coarse loss, then the dgrad chain; wgrad stream follows each dY
-            c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse,
-                         loss=self.loss_coarse, dout_bf16=self.g_coarse, dout_ld=4096)
-            e_g = mark(s0)
-
-            def on_wgrad(event, fn, stream=None, label=None):
-                stream = stream or s2
-                with torch.cuda.stream(stream):
-                    c.ws_tag = "wgrad" if stream is s2 else "cwgrad"
-                    stream.wait_event(event)
-                    if label:
-                        c.stamp(label + " begin")
-                    fn()
-                    if label:
-                        c.stamp(label + " end")
-                    c.ws_tag = ""
-
-            fused = self.fuse_dense_adam and not self.comm
-            a = self.arena
-            # The bias gradients (latency-bound column sums of dY, 7-10 us each) leave the conv-wgrad stream
-            # for the fine stream, whose forward work is long done by then: they run next to the wgrad GEMMs, not before them.
-            # (Data parallel: measured slower at 2 GPUs, 1.184 vs 1.144 ms -- the comm stream's NCCL kernels already fill
-            # those gaps -- so there the conv wgrads keep their bias gradients.)
-            side_bias = not self.comm
-
-            def conv_wgrad(desc, x, dy, name, event):
-                if side_bias:
-                    with torch.cuda.stream(s1):
-                        s1.wait_event(event)
-                        c.bias_grad_bf16(dy.view(-1, dy.shape[-1]), dy.shape[-1], self.gw(name + "/bias"))
-                    on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=None), s3)
-                else:
-                    on_wgrad(event, lambda: c.conv2d_wgrad(desc, x, dy, dw=self.gw(name + K), db=self.gw(name + "/bias")), s3)
-
-            dense_wgrad_adam = self._dense_wgrad_adam
-            nd = "coarse/dense/dense_"
-
-            e_loss = e_g
-            c.dense_dgrad_act(self.g_coarse, self.w(nd + "1" + K), self.d0, self.keep_mask, 0.5, L.EPI_RELU, out=self.g_d0,
-                              impl=self.impl)
-            e_g = mark(s0)
-            # data parallel, dense layers: exchange activations instead of gradients (dp.dense_gather_adam_merged)
-            gather = bool(self.comm) and all(self.comm.can_gather_dense(self, nd + l + K, B) for l in "01")
-            e_g1 = e_g
-            if not fused and not gather:
-                # the bucket's Adam overwrites dense_1's weights: it waits for e_g (dense_1's dgrad has read them)
-                on_wgrad(e_loss, lambda: (c.dense_wgrad(self.d0, self.g_coarse, dw=self.gw(nd + "1" + K),
-                                                        db=self.gw(nd + "1/bias"), impl=self.impl),
-                                          self.comm and dp_update("dense_1", "CoarseDense", e_g)))
-            if fused:       # updates dense_1's weights: must follow dense_1's dgrad, their last reader
-                on_wgrad(e_g, lambda: dense_wgrad_adam("1", self.d0, self.g_coarse), label="dense_1 wgrad+adam")
-            e_d0 = e_g
-            c.dense_dgrad_act(self.g_d0, self.w(nd + "0" + K), self.c4.view(B, 12288), None, 0.0, L.EPI_RELU,
-                              out=self.g_c4.view(B, 12288), impl=self.impl)
-            e_g = mark(s0)
-            if gather:
-                # one activation all-gather for both layers as soon as g_d0 exists (e_d0); each layer's row update waits for
-                # its own dgrad; the updated rows are published at the start of the next step
-                g_ = "CoarseDense"
-                self.comm.dense_gather_adam_merged(
-                    self, [(nd + "1" + K, nd + "1/bias", self.d0, self.g_coarse, e_g1),
-                           (nd + "0" + K, nd + "0/bias", self.c4.view(B, 12288), self.g_d0, e_g)],
-                    g_, ADAM_LR[g_], ADAM_BETA1, ADAM_EPS, ready=e_d0)
-            elif not fused:
-                on_wgrad(e_d0, lambda: (c.dense_wgrad(self.c4.view(B, 12288), self.g_d0, dw=self.gw(nd + "0" + K),
-                                                      db=self.gw(nd + "0/bias"), impl=self.impl),
-                                        self.comm and dp_update("dense_0", "CoarseDense", e_g)))
-            c.stamp("dense dgrad done")
-            if fused:
-                on_wgrad(e_g, lambda: dense_wgrad_adam("0", self.c4.view(B, 12288), self.g_d0), label="dense_0 wgrad+adam")
-            elif not self.comm:
-                # single GPU: the dense group's Adam runs under the conv backward.  It overwrites the dense weight
-                # mirror, so it waits for e_g: both dense dgrads (the last readers of those weights) are done.
-                on_wgrad(e_g, lambda: self.apply_adam(("CoarseDense",)))
-            conv_wgrad(self.d_c4, self.c3, self.g_c4, n + "4", e_g)
-            c.conv2d_dgrad(self.d_c4, self.g_c4, self.w(n + "4" + K), out=self.g_c3, relu_src=self.c3)
-            c.stamp("dgrad conv2d_4 done")
-            e_g = mark(s0)
-            conv_wgrad(self.d_c3, self.c2, self.g_c3, n + "3", e_g)
-            s0.wait_event(e_flip)
-            c.conv2d_dgrad(self.d_c3, self.g_c3, self.w(n + "3" + K), out=self.g_c2, relu_src=self.c2, wflip=self._wflip["3"])
-            e_g = mark(s0)
-            conv_wgrad(self.d_c2, self.p1, self.g_c2, n + "2", e_g)
-            c.conv2d_dgrad(self.d_c2, self.g_c2, self.w(n + "2" + K), out=self.g_p1, wflip=self._wflip["2"])
-            c.maxpool2x2_idx_bwd(self.i1, self.g_p1, (B, 27, 37, 256), out=self.g_c1)
-            c.stamp("dgrad conv2d_3,2 + pool bwd done")
-            e_g = mark(s0)
-            # (DP: exchanging conv2d_4..2 here as an early bucket was measured SLOWER at 2 GPUs, 1.30 vs 1.26 ms: three more
-            # NCCL launches cost more than the shorter tail saves)
-            conv_wgrad(self.d_c1, self.p0, self.g_c1, n + "1", e_g)
-            e_w1 = mark(s3)                                # gradients of conv2d_4 .. conv2d_1 are complete
-            c.conv2d_dgrad(self.d_c1, self.g_c1, self.w(n + "1" + K), out=self.g_p0, wflip=self._wflip["1"])
-            c.maxpool2x2_idx_bwd(self.i0, self.g_p0, (B, 55, 74, 96), out=self.g_c0)
-            c.stamp("dgrad conv2d_1 + pool bwd done")
-            e_g = mark(s0)
-            # Single GPU: TF-Adam of conv2d_4 .. conv2d_1 (99 % of the group) runs on the idle fine stream next to
-            # conv2d_0's weight gradient; only conv2d_0's 55 k parameters are updated in the step's tail.  The group is
-            # one contiguous arena range in backward order, so this is the same update as two launches.
-            # Data parallel, the same cut: conv2d_4 .. conv2d_1 are all-reduced in f32 and updated behind conv2d_1's weight
-            # gradient, under conv2d_1's dgrad, the pool backward and conv2d_0's wgrad; the step's tail exchanges conv2d_0's
-            # 55 k parameters only.  (8 GPUs, profiles/step_timeline_r02_n8_rank0.json: the single 16 MB allreduce + Adam was
-            # ~150 us of exposed tail.)  f32 allreduce + replicated Adam beats cast + reduce-scatter + sharded Adam +
-            # all-gather at every world size (4 GPUs: 1.160 vs 1.185 ms; 2 GPUs, with the split: 0.972 vs 1.015 ms -- the
-            # collectives are latency-bound at 8-16 MB and the sharded form needs three of them); a sharded exchange of the
-            # split measured 1.20 against 1.18 ms unsplit at 2 GPUs (the extra NCCL kernels take SM slots from the GEMMs
-            # they overlap with).
-            lo_cc, hi_cc = a.group_range("CoarseConv")
-            split_cc = a.specs["coarse/conv/conv2d_0/kernel"].offset
-            if self.comm:
-                with torch.cuda.stream(s3):
-                    self.comm.bucket_ready(self, "coarse_conv_main", after=e_g,
-                                           then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
-            else:
-                with torch.cuda.stream(s1):
-                    s1.wait_event(e_fine)
-                    s1.wait_event(e_w1)
-                    s1.wait_event(e_g)                      # conv2d_1's dgrad was the last reader of these weights
-                    self.adam_range("CoarseConv", lo_cc, split_cc)
-                    e_fine = mark(s1)
-
-            e_b0 = None
-            if side_bias:
-                with torch.cuda.stream(s1):
-                    s1.wait_event(e_g)
-                    c.bias_grad_bf16(self.g_c0.view(-1, 96), 96, self.gw(n + "0/bias"))
-                    e_b0 = mark(s1)
-
-            def conv0_and_adam():
-                c.conv2d_wgrad(self.d_c0, self.img4, self.g_c0, dw=self.gw(n + "0" + K), db=None if side_bias else self.gw(n + "0/bias"))
-                if e_b0 is not None:
-                    s3.wait_event(e_b0)
-                self._mask_padding("coarse/conv/conv2d_0/kernel")
-                if self.comm:
-                    self.comm.bucket_ready(self, "coarse_conv_0",
-                                           then=lambda lo, hi: self.adam_range("CoarseConv", lo, hi, inv_world))
-                    self.comm.wait_all(self)
-                else:
-                    self.adam_range("CoarseConv", split_cc, hi_cc)
-            on_wgrad(e_g, conv0_and_adam, s3, label="conv2d_0 wgrad + conv exchange/adam")
-            # ---- join
-            s0.wait_event(e_fine)
-            s0.wait_event(mark(s2))
-            s0.wait_event(mark(s3))
-            c.increment_i64(self.step_dev)
-            c.stamp("step end")
-            e_out = torch.cuda.Event()
-            e_out.record(s0)
-        cur.wait_event(e_out)
-
-    # ------------------------------------------------------------------ one session.run(model_op)
-    def _enqueue_step(self, phase):
-        if phase == 1 and self.overlap and self.train:
-            return self._enqueue_phase1_overlapped()
-        if self.comm:
-            self.comm.flush(self)                       # rows updated by a previous (overlapped) step
-        self.forward()
-        if phase == 1:
-            fused = self.fuse_dense_adam and not self.comm
-            self.backward_coarse(fused_dense_adam=fused)
-            groups = ("CoarseConv",) if fused else ("CoarseDense", "CoarseConv")
-        elif phase == 2:
-            self.backward_fine()
-            groups = ("FineA", "FineB")
-        else:
+            if self.comm and s.on:
+                # the dense rows other ranks updated in the PREVIOUS step arrive now, under this step's resize and
+                # convolution forward (dp.dense_gather_adam_merged / publish_rows); the dense forward waits for them
+                s.events["published"] = self.comm.publish_rows(self)
+            elif self.comm:
+                self.comm.flush(self)                   # rows updated by a previous (overlapped) step
+            self.forward(s)
             groups = ()
-        if groups:
-            scale = 1.0
-            if self.comm:
-                self.comm.wait_all(self)
-                scale = 1.0 / self.comm.world
-            self.apply_adam(groups, scale)
-            if "FineA" in groups:
-                self.refresh_derived()                   # fine/first moved: re-embed it into the pool-fused filter
-        self.ctx.increment_i64(self.step_dev)            # global_step += 1 (src/models.py:329,343,356)
+            if phase == 1:
+                fused = self.fuse_dense_adam and not self.comm
+                self.backward_coarse(fused_dense_adam=fused, lanes=s)
+                if not s.on:                            # on four streams each group was updated behind its wgrads
+                    groups = ("CoarseConv",) if fused else ("CoarseDense", "CoarseConv")
+            elif phase == 2:
+                self.backward_fine()
+                groups = ("FineA", "FineB")
+            if groups:
+                scale = 1.0
+                if self.comm:
+                    self.comm.wait_all(self)
+                    scale = 1.0 / self.comm.world
+                self.apply_adam(groups, scale)
+                if "FineA" in groups:
+                    self.refresh_derived()               # fine/first moved: re-embed it into the pool-fused filter
+            s.join()
+            c.increment_i64(self.step_dev)              # global_step += 1 (src/models.py:329,343,356)
+            c.stamp("step end")
 
     def _ensure_graph(self, phase):
         """Warm-up launch outside capture (sets function attributes, allocates workspaces, autotunes first-use shapes;
