@@ -46,6 +46,7 @@ class AugmentDesc(C.Structure):
 A3D_U8 = 2
 AUG_PARAMS = 16                       # A3D_AUG_PARAMS: floats per image in the packed parameter rows
 AUG_VALUE_COLOR, AUG_VALUE_DEPTH = 0, 1
+DENSE_WGRAD_ADAM_MAX_M = 32           # A3D_DENSE_WGRAD_ADAM_MAX_M: largest batch a3d_dense_wgrad_adam takes
 
 _vp, _i, _f, _sz, _u = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_uint
 

@@ -448,7 +448,9 @@ extern "C" int a3d_dense_wgrad_adam(a3d_ctx* ctx, const uint16_t* x, int ldx, co
   // a TF-Adam epilogue, 535 us, against 277 us.)
   int rc = a3d_mma_dense_wgrad_adam(ctx, x, ldx, dy, lddy, w, m, v, w_bf16, M, N, K, lr_t, beta1, beta2, eps, grad_scale,
                                     lr_t_dev, st);
-  if (rc == A3D_ENOTSUP) a3d_set_error("dense wgrad+adam: needs batch <= 32, K %% 256 == 0 and 16-byte aligned w/m/v");
+  if (rc == A3D_ENOTSUP)
+    a3d_set_error("dense wgrad+adam: needs batch <= %d, K %% 256 == 0 and 16-byte aligned w/m/v (batch %d, K %d)",
+                  A3D_DENSE_WGRAD_ADAM_MAX_M, M, K);
   return rc;
 }
 

@@ -1095,7 +1095,7 @@ dense_wgrad_adam_mma_kernel(const uint16_t* __restrict__ x, int ldx, const uint1
 int a3d_mma_dense_wgrad_adam(a3d_ctx* ctx, const uint16_t* x, int ldx, const uint16_t* dy, int lddy, float* w, float* m,
                              float* v, uint16_t* wb, int M, int N, int K, float lr_t, float beta1, float beta2, float eps,
                              float grad_scale, const float* lr_t_dev, cudaStream_t st) {
-  if (M > 32 || K % 256 || !aligned16(w) || !aligned16(m) || !aligned16(v) || (wb && (reinterpret_cast<uintptr_t>(wb) & 7)))
+  if (M > A3D_DENSE_WGRAD_ADAM_MAX_M || K % 256 || !aligned16(w) || !aligned16(m) || !aligned16(v) || (wb && (reinterpret_cast<uintptr_t>(wb) & 7)))
     return A3D_ENOTSUP;
   const int kblocks = K / (128 * kAdamQN);
   int gy = kAdamBPS * ctx->sm_count / kblocks;       // one resident wave

@@ -8,7 +8,8 @@
 // hosts), activations, routing records and scratch out of it.  Every launch goes to the caller's stream; a step has no
 // host synchronisation and no allocation, i.e. it is CUDA-graph capturable once the first (autotuning) call is done.
 // Schedule: the sequential single-stream form of ann3depth_b200/msdn.py (forward of both stacks + both losses; backward
-// of the active tf.case branch with the dense weight gradients fused into TF-Adam; TF-Adam of the branch's groups;
+// of the active tf.case branch with the dense weight gradients fused into TF-Adam up to batch A3D_DENSE_WGRAD_ADAM_MAX_M
+// (separate wgrad + TF-Adam above it); TF-Adam of the branch's groups;
 // global_step += 1).  BF16 storage, tcgen05 kernels.  The Python host adds the multi-stream overlap (stream placement as
 // annotations on the same launch sequence: msdn.py's _Lanes), data parallelism and the TF32 mode on top of the same kernels.
 #include "common.cuh"
@@ -276,13 +277,26 @@ int backward_coarse(a3d_msdn* n, void* st) {
   const int B = n->B;
   auto W = [&](const char* nm) { return n->wb + seg_off(n, nm); };
   auto G = [&](const char* nm) { return n->g + seg_off(n, nm); };
-  // dense_1: dgrad (+ DropoutGrad + ReluGrad of dense_0), then its fused wgrad + TF-Adam (after the last reader of w)
+  // dense_1: dgrad (+ DropoutGrad + ReluGrad of dense_0), then its fused wgrad + TF-Adam (after the last reader of w).
+  // The fused kernel takes batches up to A3D_DENSE_WGRAD_ADAM_MAX_M; a larger batch writes both weight gradients and
+  // updates the CoarseDense group once both dgrads have read the weights.
+  const bool fused = B <= A3D_DENSE_WGRAD_ADAM_MAX_M;
+  if (!fused)
+    CK(a3d_dense_wgrad(c, n->d0, 4096, n->g_coarse, 4096, G("coarse/dense/dense_1/kernel"), G("coarse/dense/dense_1/bias"), B,
+                       N_PIX, 4096, A3D_IMPL_AUTO, st));
   CK(a3d_dense_dgrad_act(c, n->g_coarse, 4096, W("coarse/dense/dense_1/kernel"), n->g_d0, n->dense_acc, B, N_PIX, 4096,
                          A3D_IMPL_AUTO, n->d0, n->keep, 0.5f, A3D_EPI_RELU, st));
-  CK(dense_wgrad_adam(n, "coarse/dense/dense_1/kernel", "coarse/dense/dense_1/bias", n->d0, 4096, n->g_coarse, N_PIX, st));
+  if (fused)
+    CK(dense_wgrad_adam(n, "coarse/dense/dense_1/kernel", "coarse/dense/dense_1/bias", n->d0, 4096, n->g_coarse, N_PIX, st));
+  else
+    CK(a3d_dense_wgrad(c, n->c4, 12288, n->g_d0, 4096, G("coarse/dense/dense_0/kernel"), G("coarse/dense/dense_0/bias"), B, 4096,
+                       12288, A3D_IMPL_AUTO, st));
   CK(a3d_dense_dgrad_act(c, n->g_d0, 4096, W("coarse/dense/dense_0/kernel"), n->g_c4, n->dense_acc, B, 4096, 12288, A3D_IMPL_AUTO,
                          n->c4, nullptr, 0.f, A3D_EPI_RELU, st));
-  CK(dense_wgrad_adam(n, "coarse/dense/dense_0/kernel", "coarse/dense/dense_0/bias", n->c4, 12288, n->g_d0, 4096, st));
+  if (fused)
+    CK(dense_wgrad_adam(n, "coarse/dense/dense_0/kernel", "coarse/dense/dense_0/bias", n->c4, 12288, n->g_d0, 4096, st));
+  else
+    CK(adam_range(n, G_DENSE, n->group_lo[G_DENSE], n->group_hi[G_DENSE], st));
   // conv stack, top down
   CK(a3d_conv2d_wgrad(c, &n->d_c4, n->c3, n->g_c4, G("coarse/conv/conv2d_4/kernel"), G("coarse/conv/conv2d_4/bias"), n->scratch,
                       n->scratch_bytes, st));

@@ -113,7 +113,11 @@ _SEQUENTIAL = _Lanes()
 
 class MSDNNet:
     """Buffers + launch sequence for one replica with a static batch size (the reference requires a
-    static batch dimension too: `int(images.shape[0])`, src/models.py:225,256,299)."""
+    static batch dimension too: `int(images.shape[0])`, src/models.py:225,256,299).
+
+    `fuse_dense_adam=True` fuses the dense weight gradients into TF-Adam where the kernel supports it: on one GPU, at a
+    batch of at most `L.DENSE_WGRAD_ADAM_MAX_M`.  A larger batch, like `fuse_dense_adam=False`, runs the separate dense
+    wgrad and TF-Adam kernels over the CoarseDense group."""
 
     def __init__(self, ctx: ops.Context, batch: int, in_hw=(480, 640), depth_hw=(55, 73), train=True,
                  beta2=ADAM_BETA2_REFERENCE, impl=L.IMPL_AUTO, dropout_seed=2, comm=None, grad_dtype=torch.float32,
@@ -153,7 +157,7 @@ class MSDNNet:
         # inside the HBM-bound TF-Adam pass (a3d_dense_wgrad_adam), so the 67 M-element f32 gradient is never written
         # or re-read: 26 instead of 38 bytes per dense parameter and step.  Data parallel runs need the gradient in
         # memory for the reduce-scatter and keep the separate kernels (dp.py shards the optimizer instead).
-        self.fuse_dense_adam = fuse_dense_adam
+        self.fuse_dense_adam = fuse_dense_adam and batch <= L.DENSE_WGRAD_ADAM_MAX_M
         self._streams = None          # the phase-1 step's streams (_Lanes), created on first use
         self._wflip = None            # flipped filters of the stride-1 dgrads (refreshed at the start of every step)
         self.dev = torch.device(f"cuda:{ctx.device}")

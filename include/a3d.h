@@ -181,7 +181,10 @@ int a3d_dense_wgrad(a3d_ctx*, const uint16_t* x, int ldx, const uint16_t* dy, in
 /* dense wgrad fused with the TF-Adam update of that kernel (single GPU): the gradient tiles are consumed
  * from tensor memory by the optimizer and never written to HBM.  w/m/v f32 [N,K] updated in place, w_bf16
  * (nullable) refreshed; db (nullable) f32 [N] receives the bias gradient.  Same formula and arguments as
- * a3d_adam_tf.  Requires K % 64 == 0 and 16-byte aligned row pitches. */
+ * a3d_adam_tf.  Requires K % 64 == 0 and 16-byte aligned row pitches.  The batch M is at most
+ * A3D_DENSE_WGRAD_ADAM_MAX_M (the gradient is formed in two 16-deep mma.sync steps); a larger M, K % 256 != 0 or
+ * w/m/v not 16-byte aligned return A3D_ENOTSUP: such callers run a3d_dense_wgrad + a3d_adam_tf instead. */
+#define A3D_DENSE_WGRAD_ADAM_MAX_M 32
 int a3d_dense_wgrad_adam(a3d_ctx*, const uint16_t* x, int ldx, const uint16_t* dy, int lddy, float* db,
                          float* w, float* m, float* v, uint16_t* w_bf16, int M, int N, int K,
                          float lr_t, float beta1, float beta2, float eps, float grad_scale,

@@ -55,8 +55,8 @@ def test_product_never_imports_oracle(repo_root):
 
 
 def test_conv_desc_layout_matches_header(repo_root, tmp_path):
-    """The ctypes mirror of a3d_conv_desc must have the C struct's size and field offsets (the struct grew in ABI 200):
-    a C program compiled against include/a3d.h prints them."""
+    """The ctypes mirror of a3d_conv_desc must have the C struct's size and field offsets (the struct grew in ABI 200), and
+    the mirrored constants the header's values: a C program compiled against include/a3d.h prints them."""
     import subprocess
     from ann3depth_b200 import _lib
     fields = [n for n, _ in _lib.ConvDesc._fields_]
@@ -64,10 +64,12 @@ def test_conv_desc_layout_matches_header(repo_root, tmp_path):
     src.write_text("#include <stdio.h>\n#include <stddef.h>\n#include \"a3d.h\"\nint main(void) {\n"
                    "  printf(\"%zu\\n\", sizeof(a3d_conv_desc));\n" +
                    "".join(f"  printf(\"%zu\\n\", offsetof(a3d_conv_desc, {f}));\n" for f in fields) +
+                   "  printf(\"%d\\n\", A3D_DENSE_WGRAD_ADAM_MAX_M);\n"
                    "  printf(\"%d\\n\", A3D_VERSION);\n  return 0;\n}\n")
     exe = tmp_path / "layout"
     subprocess.run(["gcc", "-I", os.path.join(repo_root, "include"), "-o", str(exe), str(src)], check=True)
     out = [int(x) for x in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.split()]
     assert out[0] == ctypes.sizeof(_lib.ConvDesc)
-    assert out[1:-1] == [getattr(_lib.ConvDesc, f).offset for f in fields]
+    assert out[1:-2] == [getattr(_lib.ConvDesc, f).offset for f in fields]
+    assert out[-2] == _lib.DENSE_WGRAD_ADAM_MAX_M
     assert out[-1] == _lib.ABI_VERSION

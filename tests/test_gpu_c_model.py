@@ -3,6 +3,7 @@ ctypes ALONE -- no ann3depth_b200 host logic on the path, torch only owns the de
 of the Python host (`models.msdn`, same kernels, same sequential schedule) and the float64 oracle.  This is the boundary a
 non-Python host binds (INTEGRATION.md): `session.run(model_op)` of src/ann3depth.py:126-127 for src/models.py:203-367."""
 import ctypes as C
+import math
 
 import pytest
 import torch
@@ -110,8 +111,9 @@ def test_segment_table_matches_the_python_arena():
     net.close()
 
 
-def test_c_step_equals_python_step_and_oracle():
-    B = 2
+def c_step_and_python_step(B):
+    """One phase-1 step of a fresh C net and of the Python host (same kernels, sequential schedule, no graph) from the same
+    weights, inputs and dropout mask, checked against each other.  Returns what the oracle comparison needs."""
     images, depths, mask, p = make(B)
     a = packed_arena(p)
     im, dp, mk = images.to(DEV), depths.to(DEV), mask.to(DEV)
@@ -120,13 +122,13 @@ def test_c_step_equals_python_step_and_oracle():
     phase, losses = net.step(im, dp, mk)
     torch.cuda.synchronize()
     assert phase == 1 and net.lib.a3d_msdn_global_step(net.net) == 1
-    # the Python host on the same kernels (sequential schedule, no graph)
     op = models.msdn(im.clone(), dp.clone(), train=True, beta2=0.999, overlap=False)
     op.net.load_params(p)
     op.net.set_dropout_mask(mk)
     op.run(use_graph=False)
     torch.cuda.synchronize()
     lc, lf = float(losses[0]), float(losses[1])
+    assert math.isfinite(lc) and math.isfinite(lf)
     assert abs(lc - float(op.net.loss_coarse)) <= 1e-4 * abs(lc) and abs(lf - float(op.net.loss_fine)) <= 1e-4 * abs(lf)
     cm, cw = net.view(net.m_ptr), net.view(net.w_ptr)
     lo, hi = a.group_range("CoarseDense")[0], a.group_range("CoarseConv")[1]
@@ -134,6 +136,20 @@ def test_c_step_equals_python_step_and_oracle():
     assert cos(cw[lo:hi] - a.w[lo:hi].to(DEV), op.net.arena.w[lo:hi] - a.w[lo:hi].to(DEV)) > 0.99
     lo, hi = a.group_range("FineA")[0], a.group_range("FineB")[1]
     assert float(cm[lo:hi].abs().max()) == 0.0 and torch.equal(cw[lo:hi], a.w[lo:hi].to(DEV))    # phase 1: fine untouched
+    return net, a, images, depths, mask, p, lc, lf, cm
+
+
+def test_c_step_equals_python_step_and_oracle():
+    c_step_equals_python_step_and_oracle(2)
+
+
+def test_c_step_equals_python_step_and_oracle_above_fused_batch_limit():
+    """batch 33, past the fused dense wgrad + TF-Adam kernel's batch limit: the C model runs the separate kernels."""
+    c_step_equals_python_step_and_oracle(33)
+
+
+def c_step_equals_python_step_and_oracle(B):
+    net, a, images, depths, mask, p, lc, lf, cm = c_step_and_python_step(B)
     # ... and the float64 oracle at the BF16 storage points
     st = OM.TrainState({k: v.double() for k, v in p.items()}, beta2=0.999)
     out, _ = OM.train_step(st, images.double(), depths.double(), mask.double(), q=OM.bf16_round)
@@ -143,6 +159,11 @@ def test_c_step_equals_python_step_and_oracle():
                  "coarse/dense/dense_1/bias"):
         assert cos(got_m[name], st.m[name]) > 0.999, name
     net.close()
+
+
+def test_c_step_at_the_largest_batch():
+    """batch 256, the upper bound a3d_msdn_create accepts: phase 1 runs with finite losses and equals the Python step."""
+    c_step_and_python_step(256)[0].close()
 
 
 def test_c_phase2_and_inference():

@@ -141,23 +141,33 @@ def infer(label, B, dtype="bf16"):
     torch.cuda.synchronize()
 
 
+def dcnf(label, B, train, **kw):
+    config[0] = label
+    g = torch.Generator().manual_seed(B)
+    images = torch.rand(B, 480, 640, 3, generator=g).cuda()
+    depths = (torch.rand(B, 480, 640, 1, generator=g) * 0.95 + 0.05).cuda()
+    models.dcnf(images, depths, train=train, **kw).run()
+    torch.cuda.synchronize()
+
+
+# Besides the benchmark's batches, one batch per batch-dependent code path (DESIGN section 2): the dense layers' batch is
+# their GEMM's M, and the tile width, the chunking above 256 rows and the kernel choice above 32 / 128 rows follow it.
 train("msdn bf16 B=32", 32)
 train("msdn bf16 B=32 sequential", 32, phases=(1,), overlap=False, fuse_dense_adam=False)
-for B in (1, 32, 512):
+for B in (1, 5, 33, 100, 130):
+    train(f"msdn bf16 B={B}", B)
+for B in (1, 7, 32, 100, 300, 512):
     infer(f"msdn bf16 inference B={B}", B)
 for dtype in ("tf32", "tf32x3"):
-    for B in (2, 32):
+    for B in (2, 32, 33):
         train(f"msdn {dtype} B={B}", B, dtype)
         infer(f"msdn {dtype} inference B={B}", B, dtype)
-g = torch.Generator().manual_seed(16)
-images = torch.rand(16, 480, 640, 3, generator=g).cuda()
-depths = (torch.rand(16, 480, 640, 1, generator=g) * 0.95 + 0.05).cuda()
-for label, train_, kw in (("dcnf B=16", True, {}),
-                          ("dcnf B=16 grid4", True, dict(graph="grid4", r_nonneg=True, train_pairwise=True, predict="map")),
-                          ("dcnf inference B=16", False, {})):
-    config[0] = label
-    models.dcnf(images, depths, train=train_, **kw).run()
-    torch.cuda.synchronize()
+dcnf("dcnf B=16", 16, True)
+dcnf("dcnf B=16 grid4", 16, True, graph="grid4", r_nonneg=True, train_pairwise=True, predict="map")
+dcnf("dcnf inference B=16", 16, False)
+for B in (1, 3, 6):
+    dcnf(f"dcnf B={B}", B, True)
+dcnf("dcnf inference B=6", 6, False)
 out.close()
 """
 
@@ -936,9 +946,11 @@ def r_pairwise_dense_bwd(c):
 def r_mean_f32(c):
     v = c.v
     n = v["v"].numel()
-    assert n & (n - 1) == 0, "a power-of-two count makes the mean exact"
     x = c.ints((n,), 64)
     c.put(v["v"], x)
+    # the integer sum is exact and the kernel's division rounds to nearest; so does float64 -> float32 of the quotient,
+    # which for a count this small never lies within a float64 ulp of a float32 tie (a batch of 3 or 6 is not a power of 2)
+    assert n < 2 ** 16
     c.expect("mean", c.flat(v["out"], 1), (x.sum() / n).view(1).float())
 
 
@@ -1019,6 +1031,17 @@ def required_signatures():
         "bias_grad_f32 past 4096 rows": lambda r: r["m"] == "bias_grad_bf16" and f32(r, 0, "dy") and
         rows(r, 0, "dy") > 4096,
         "scale_cast_bf16": lambda r: r["m"] == "scale_cast_bf16",
+        # the batch-dependent dense paths (tc_gemm.cu, conv.cu): forward tiles bn = 64 / 128 / 256 and a partial 44-row
+        # chunk past 256 rows; the SIMT dgrad + separate epilogue above 128 rows; the rows dgrad at row counts that are
+        # not multiples of 128; the TF32 tiles of bn = 64
+        **{f"bf16 dense_fwd at M = {m}": (lambda m: lambda r: r["m"] == "dense_fwd" and bf16(r, 0, "x") and
+                                          rows(r, 0, "x") == m)(m) for m in (33, 100, 130, 300)},
+        "dense_dgrad_act at M = 130": lambda r: r["m"] == "dense_dgrad_act" and rows(r, 0, "dy") == 130,
+        **{f"DCNF dense_dgrad at M = {m}": (lambda m: lambda r: r["m"] == "dense_dgrad" and bf16(r, 0, "dy") and
+                                            rows(r, 0, "dy") == m)(m) for m in (144, 288)},
+        "tf32 dense wgrad at M = 33": lambda r: r["m"] == "dense_wgrad" and f32(r, 0, "x") and rows(r, 1, "dy") == 33,
+        "tf32 dense dgrad at M = 33": lambda r: r["m"] == "dense_dgrad_act" and f32(r, 0, "dy") and
+        rows(r, 0, "dy") == 33,
     }
 
 
@@ -1041,6 +1064,18 @@ def test_inventory_is_classified(inventory, capsys):
     assert not set(REPLAY) & set(EXCLUDED)
     missing = [name for name, ok in required_signatures().items() if not any(ok(rec) for _, rec in calls)]
     assert not missing, f"signatures the models no longer record: {missing}"
+
+
+def test_fused_dense_update_stays_within_its_batch_limit(inventory):
+    """a3d_dense_wgrad_adam takes at most L.DENSE_WGRAD_ADAM_MAX_M rows: above it the MSDN step must record the separate
+    weight gradients of both coarse dense kernels instead (which TF-Adam then updates as a group)."""
+    calls = inventory[0]
+    over = [describe(cfg, rec) for cfg, rec in calls
+            if rec["m"] == "dense_wgrad_adam" and _tensor_arg(rec, 1, "dy")["T"][0] > L.DENSE_WGRAD_ADAM_MAX_M]
+    assert not over, over
+    widths = {_tensor_arg(rec, 0, "x")["T"][1] for cfg, rec in calls
+              if "msdn bf16 B=33 phase 1" in cfg and rec["m"] == "dense_wgrad" and _tensor_arg(rec, 1, "dy")["T"][0] == 33}
+    assert widths == {4096, 12288}, widths          # dense_1 reads d0 [B, 4096], dense_0 reads c4 [B, 12288]
 
 
 @pytest.mark.parametrize("method", sorted(REPLAY))

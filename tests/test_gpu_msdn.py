@@ -189,7 +189,16 @@ def test_train_step_general_adam_matches_oracle():
 
 def test_overlapped_step_equals_sequential_step():
     """The three-stream phase-1 schedule must produce exactly the sequential schedule's results."""
-    B = 2
+    overlapped_vs_sequential(2)
+
+
+def test_overlapped_step_equals_sequential_step_above_fused_batch_limit():
+    """As above at batch 33, past the fused dense wgrad + TF-Adam kernel's batch limit: both schedules run the separate
+    dense weight gradients and TF-Adam."""
+    overlapped_vs_sequential(33)
+
+
+def overlapped_vs_sequential(B):
     images, depths, mask = make_inputs(B)
     p = conditioned_params()
     res = []

@@ -151,21 +151,27 @@ def msdn(B, train, dtype="bf16"):
     op.net.load_params(glorot_params(1))
     return op
 
-op = msdn(32, True)
-op.run(use_graph=True)                    # phase 1: eager warm-up (tunes), capture, replay
-op.net.global_step = 2000000 // 32        # first step of phase 2 (msdn.phase_of)
-op.run(use_graph=True)
-del op
-for B in (1, 32, 512):                    # inference as tools/fp8_infer_bench.py
+def train(B, use_graph):
+    op = msdn(B, True)
+    op.run(use_graph=use_graph)           # phase 1 (with the graph: eager warm-up (tunes), capture, replay)
+    op.net.global_step = 2000000 // B     # first step of phase 2 (msdn.phase_of)
+    op.run(use_graph=use_graph)
+
+train(32, True)
+# one batch per batch-dependent GEMM configuration (test_gpu_model_launches.py RECORD_SCRIPT, DESIGN section 2)
+for B in (1, 5, 33, 100, 130):
+    train(B, False)
+for B in (1, 7, 32, 100, 300, 512):       # inference as tools/fp8_infer_bench.py, and the dense tiles past it
     for dtype in ("bf16", "fp8"):
         op = msdn(B, False, dtype)
         op.run()
         del op
-g = torch.Generator().manual_seed(16)
-images = torch.rand(16, 480, 640, 3, generator=g).cuda()
-depths = (torch.rand(16, 480, 640, 1, generator=g) * 0.95 + 0.05).cuda()
-models.dcnf(images, depths, train=True).run()
-models.dcnf(images, depths, train=False).run()
+for B in (16, 6):
+    g = torch.Generator().manual_seed(B)
+    images = torch.rand(B, 480, 640, 3, generator=g).cuda()
+    depths = (torch.rand(B, 480, 640, 1, generator=g) * 0.95 + 0.05).cuda()
+    models.dcnf(images, depths, train=True).run()
+    models.dcnf(images, depths, train=False).run()
 torch.cuda.synchronize()
 """
 
