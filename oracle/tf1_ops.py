@@ -15,6 +15,17 @@ import torch.nn.functional as F
 
 
 # ----------------------------------------------------------------------------- resize
+def resize_axis(n_in: int, n_out: int):
+    """(lo, hi, lerp) of one axis of the TF1 legacy bilinear resize: source rows / columns and float32 weights.
+    TF computes the scale and the source coordinate in float32 (CalculateResizeScale, `in = dst * scale`), whatever
+    the image dtype: mirror that so floor()/lerp agree bit-wise."""
+    scale = torch.tensor(float(n_in), dtype=torch.float32) / torch.tensor(float(n_out), dtype=torch.float32)
+    src = torch.arange(n_out, dtype=torch.float32) * scale
+    lo = torch.floor(src).to(torch.long)
+    hi = torch.clamp(lo + 1, max=n_in - 1)
+    return lo, hi, src - lo.to(torch.float32)
+
+
 def resize_bilinear_tf1(x: torch.Tensor, out_h: int, out_w: int) -> torch.Tensor:
     """``tf.image.resize_images(x, [out_h, out_w])`` (BILINEAR, align_corners=False).
 
@@ -28,19 +39,9 @@ def resize_bilinear_tf1(x: torch.Tensor, out_h: int, out_w: int) -> torch.Tensor
     if h == out_h and w == out_w:
         return x
     dt = x.dtype
-
-    def axis(n_in, n_out):
-        # TF computes the scale and the source coordinate in float32 (CalculateResizeScale,
-        # `in = dst * scale`), whatever the image dtype: mirror that so floor()/lerp agree bit-wise.
-        scale = torch.tensor(float(n_in), dtype=torch.float32) / torch.tensor(float(n_out), dtype=torch.float32)
-        src = torch.arange(n_out, dtype=torch.float32) * scale
-        lo = torch.floor(src).to(torch.long)
-        hi = torch.clamp(lo + 1, max=n_in - 1)
-        lerp = (src - lo.to(torch.float32)).to(dt)
-        return lo, hi, lerp
-
-    ylo, yhi, yl = axis(h, out_h)
-    xlo, xhi, xl = axis(w, out_w)
+    ylo, yhi, yl = resize_axis(h, out_h)
+    xlo, xhi, xl = resize_axis(w, out_w)
+    yl, xl = yl.to(dt), xl.to(dt)
     top = x[:, ylo]                      # [B, out_h, W, C]
     bot = x[:, yhi]
     xl_ = xl.view(1, 1, out_w, 1)

@@ -20,6 +20,8 @@ from oracle import dcnf as OD
 from oracle import msdn as OM
 from oracle import tf1_ops as T
 
+import test_gpu_model_launches as ML
+
 DEV = "cuda:0"
 
 
@@ -450,11 +452,13 @@ def test_dense_bwd_unaligned_falls_back(ctx):
 def test_resize_vs_oracle(ctx, shape, out):
     g = torch.Generator().manual_seed(40)
     x = torch.rand(*shape, generator=g)
-    ref = T.resize_bilinear_tf1(x.double(), *out).float()
+    ref, mag = ML.resize_ref(x.double().to(DEV), *out)
+    assert torch.equal(ref.cpu(), T.resize_bilinear_tf1(x.double(), *out))
+    bound = ML.LERP_U * ML.U * mag                               # the float32 lerp (test_gpu_model_launches)
     y = ctx.resize_bilinear_tf1(x.to(DEV), out[0], out[1])
-    assert float((y.cpu() - ref).abs().max()) < 1e-5
+    assert ML.within(y, ref, bound, "float32")[0] is None
     yb = ctx.resize_bilinear_tf1(x.to(DEV), out[0], out[1], dstC=shape[3] + 1, dtype=torch.bfloat16)
-    assert float((yb[..., :shape[3]].float().cpu() - ref).abs().max()) < 5e-3
+    assert ML.rounded(yb[..., :shape[3]], ref, bound, "bf16")[0] is None            # round to nearest even
     assert float(yb[..., shape[3]:].abs().max()) == 0.0
 
 
@@ -521,12 +525,18 @@ def test_silog_loss_vs_oracle(ctx, quantised):
     o64 = out.double().requires_grad_(True)
     ref = OM.silog_loss(o64, tar.double())
     (gref,) = torch.autograd.grad(ref, o64)
+    # the per-element bounds of the float32 arithmetic on the float32 arguments fl(o + eps) (silog_reference); the
+    # oracle (float64 arguments) agrees with that reference far inside them
+    lon = float(torch.tensor(0.5 / 4070, dtype=torch.float32))
+    r = ML.silog_reference(out.to(DEV), tar.to(DEV), lon)
+    assert abs(float(r["loss"][0]) - float(ref.detach())) < 1e-7 * abs(float(ref.detach()))
+    assert float((r["grad"][0].cpu() - gref).abs().max()) < 1e-7 * float(gref.abs().max())
     loss, lps, dout, _ = ctx.silog_loss(out.to(DEV), tar.to(DEV))
-    assert abs(float(loss) - float(ref)) / abs(float(ref)) < 1e-4
-    denom = float(gref.abs().max())
-    assert float((dout.cpu().double() - gref).abs().max()) / denom < 1e-4
+    for got, key in ((loss, "loss"), (lps, "loss_ps"), (dout, "grad")):
+        assert ML.within(got, *r[key], key)[0] is None
+    assert bool((dout[out.to(DEV) < 0] == 0).all())                # the NaN branch: exactly 0
     _, _, _, db = ctx.silog_loss(out.to(DEV), tar.to(DEV), grad_bf16=True)
-    assert float((db.float().cpu().double() - gref).abs().max()) / denom < 1e-2
+    assert ML.rounded(db, *r["grad"], "bf16 grad")[0] is None
 
 
 @pytest.mark.parametrize("beta2", [1.0, 0.999])
@@ -580,10 +590,15 @@ def test_crf_vs_oracle(ctx):
                   want_dr=True)
     assert int(res["status"].abs().max()) == 0
     assert float((res["ystar"].cpu().double() - ystar.reshape(B, n)).abs().max()) < 1e-5      # north-star: 1e-5
-    assert float((res["nll"].cpu().double() - nll.detach()).abs().max()) < 1e-3
-    assert float((res["logdet"].cpu().double() - torch.linalg.slogdet(A.detach())[1]).abs().max()) < 1e-4
-    assert float((res["dz"].cpu().double() - gz.reshape(B, n)).abs().max()) < 1e-4
-    assert float((res["dr"].cpu().double() - gr.reshape(B, 48)).abs().max()) < 1e-4
+    # per-element bounds of the float32 arithmetic (crf_reference) on the float32 inputs
+    ref = ML.crf_reference(z.float().reshape(B, n), y.float().reshape(B, n), r.float().reshape(B, 48), pl, pr, 1.0, False)
+    for key in ("ystar", "nll", "logdet", "dz", "dr"):
+        assert ML.within(res[key].cpu(), *ref[key], key)[0] is None
+    assert ML.crf_solution_checks({}, res["ystar"], ref) is None
+    # the float32 inputs are within 1e-7 of the float64 ones: the oracle on those agrees far inside 1e-4
+    assert float((ref["nll"][0] - nll.detach()).abs().max()) < 1e-4
+    assert float((ref["dz"][0] - gz.reshape(B, n)).abs().max()) < 1e-4
+    assert float((ref["dr"][0] - gr.reshape(B, 48)).abs().max()) < 1e-4
     # not SPD -> status, zeros instead of NaNs
     rbad = -torch.ones(2, 48)
     res = ctx.crf(z.float().reshape(B, n)[:2].to(DEV), y.float().reshape(B, n)[:2].to(DEV), rbad.to(DEV),
@@ -592,16 +607,24 @@ def test_crf_vs_oracle(ctx):
 
 
 def test_pairwise_features_tile_means_patches(ctx):
+    """similarities on tile-wise constant colours with a few pixels moved between histogram bins (exact features,
+    test_gpu_model_launches.pairwise_image), spanning (0.05, 0.95) in both features; tile means of dyadic depths, exact"""
     g = torch.Generator().manual_seed(48)
-    im = torch.rand(2, 240, 320, 3, generator=g)
-    dp = torch.rand(2, 240, 320, 1, generator=g)
+    im = ML.pairwise_image(2, 240, 320, g)
     pl, pr = OD.pair_indices()
     ref = OD.pairwise_features(im.double())
+    ML.assert_similarities_span(ref)
     sims = ctx.pairwise_features(im.to(DEV), torch.tensor(pl, dtype=torch.int32, device=DEV),
                                  torch.tensor(pr, dtype=torch.int32, device=DEV))
-    assert float((sims.cpu().double() - ref).abs().max()) < 1e-5
-    ym = ctx.tile_means(dp.to(DEV))
-    assert float((ym.cpu().double() - OD.tile_means(dp.double()).reshape(2, 48)).abs().max()) < 1e-6
+    ref64, bound = ML.pairwise_reference(im, pl, pr)
+    assert torch.equal(ref64, ref)
+    assert ML.within(sims.cpu(), ref, bound, "similarities")[0] is None
+    dp = torch.randint(0, 4096, (2, 240, 320, 1), generator=g).double() / 4096       # the 1600-term sums are exact
+    q = OD.tile_means(dp).reshape(2, 48)
+    ML.assert_no_f32_tie(q)
+    ym = ctx.tile_means(dp.float().to(DEV))
+    assert torch.equal(ym.cpu(), q.float())
+    im = torch.rand(2, 240, 320, 3, generator=g)
     pt = ctx.extract_patches(im.to(DEV), dstC=16)
     refp = OD.patches(im).reshape(96, 100, 100, 3).to(torch.bfloat16)
     assert torch.equal(pt[..., :3].cpu(), refp) and float(pt[..., 3:].abs().max()) == 0
