@@ -138,6 +138,7 @@ SIGNATURES = {
     "a3d_maxpool2x2_idx_bwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "a3d_relu_bwd": (_i, [_vp, _vp, _vp, _i, _vp, _sz, _i, _vp]),
     "a3d_silog_loss": (_i, [_vp, _vp, _vp, _i, _i, _f, _vp, _vp, _vp, _vp, _i, _vp]),
+    "a3d_ssi_loss": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _i, _vp, _vp, _vp, _vp, _i, _vp]),
     "a3d_adam_tf": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _sz, _f, _f, _f, _f, _f, _vp, _vp]),
     "a3d_adam_tf_bf16g": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _sz, _f, _f, _f, _f, _f, _vp, _vp]),
     "a3d_sgd": (_i, [_vp, _vp, _vp, _vp, _sz, _f, _f, _vp]),

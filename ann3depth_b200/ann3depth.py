@@ -124,7 +124,8 @@ def setup_model(args, comm=None):
     model = getattr(models, args.model)
     inp = data.inputs(args.datadir, args.dataset, args.batchsize, seed=100 + int(os.environ.get("RANK", 0)))
     aug = augment_from_flag(getattr(args, "augment", "none"))          # the training op only; evaluation sees raw inputs
-    op = model(inp.images, inp.depths, comm=comm, augment=aug)
+    kw = {"loss": args.loss} if getattr(args, "loss", "silog") != "silog" else {}   # parse_args admits it for msdn only
+    op = model(inp.images, inp.depths, comm=comm, augment=aug, **kw)
     op.net.load_params(glorot_params(seed=1, model=args.model))
     return op, inp
 
@@ -294,10 +295,17 @@ def parse_args(argv=None):
     parser.add_argument("--augment", default="none", choices=["none", "eigen"],
                         help="Training-time augmentation: 'eigen' = random scale, rotation, crop, flip and colour of "
                              "Eigen et al. 2014, section 3.3, on the GPU (beyond the reference).")
+    parser.add_argument("--loss", default="silog", choices=["silog", "ssi"],
+                        help="Training objective of MSDN: the reference's scale-invariant log loss (silog), or the "
+                             "scale-and-shift-invariant loss of Ranftl et al. 2020 (ssi) for ground truth known only up "
+                             "to a scale and a shift per image (beyond the reference).")
     parser.add_argument("--cluster-spec", default="", type=str, help="(ignored: no parameter servers)")
     parser.add_argument("--job-name", default="local", type=str, help="(ignored)")
     parser.add_argument("--task-index", default=0, type=int, help="(ignored)")
-    return parser.parse_args(argv)
+    args = parser.parse_args(argv)
+    if args.loss != "silog" and args.model != "msdn":
+        parser.error(f"--loss {args.loss} applies to --model msdn only ({args.model} trains on its own objective)")
+    return args
 
 
 if __name__ == "__main__":

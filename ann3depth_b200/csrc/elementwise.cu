@@ -285,6 +285,170 @@ extern "C" int a3d_silog_loss(a3d_ctx* ctx, const float* out, const float* tar, 
   return 0;
 }
 
+// ------------------------------------------------------------------------------------ scale-and-shift-invariant loss
+// The formula is stated in include/a3d.h (a3d_ssi_loss).  One CTA per image, p and g staged in shared memory.
+// Pass 1: double moments + min/max of p, then the fit (s, t).  Pass 2: sum r^2, the weighted sum of |D| over the
+// scales' pairs, and Q.  Pass 3: the gradient; each pixel gathers the signs of its own <= 4 pairs per scale.
+// Residuals are recomputed from p and g wherever a pass needs one (three float32 roundings, so every thread
+// that touches pixel j gets the same r_j).  Every reduction runs in a fixed order and there are no atomics.
+constexpr int SSI_THREADS = 512;
+constexpr int SSI_MAX_SCALES = 4;
+
+// v[] summed over the block; every thread receives the totals.  The shuffle tree and the pass over the warp partials
+// have a fixed order, so the result does not depend on scheduling.
+template <int NV>
+__device__ __forceinline__ void ssi_block_sum(double (&v)[NV], double (*red)[SSI_THREADS / 32]) {
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int j = 0; j < NV; ++j) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[j] += __shfl_xor_sync(0xffffffffu, v[j], o);
+    if (lane == 0) red[j][wid] = v[j];
+  }
+  __syncthreads();
+#pragma unroll
+  for (int j = 0; j < NV; ++j) {
+    double s = 0.0;
+    for (int w = 0; w < SSI_THREADS / 32; ++w) s += red[j][w];
+    v[j] = s;
+  }
+  __syncthreads();
+}
+
+__device__ __forceinline__ float ssi_residual(float s, float t, float p, float g) {
+  return __fsub_rn(__fadd_rn(__fmul_rn(s, p), t), g);          // no contraction into an FMA
+}
+
+__device__ __forceinline__ double ssi_sign(float d) { return d > 0.f ? 1.0 : (d < 0.f ? -1.0 : 0.0); }
+
+__global__ void __launch_bounds__(SSI_THREADS, 1)
+ssi_loss_kernel(const float* __restrict__ out, const float* __restrict__ tar, int H, int W, int B, float alpha,
+                int scales, float* __restrict__ loss_ps, float* __restrict__ dout_f32, uint16_t* __restrict__ dout_bf16,
+                int ld) {
+  extern __shared__ float ssi_sm[];                       // p [n] | g [n]
+  __shared__ double red[4][SSI_THREADS / 32];
+  __shared__ float redf[2][SSI_THREADS / 32];
+  const int n = H * W, b = blockIdx.x;
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  float* sp = ssi_sm;
+  float* sg = ssi_sm + n;
+  const float* o = out + (size_t)b * n;
+  const float* t = tar + (size_t)b * n;
+  // pass 1: Sp, Sg, Spp, Spg and the range of p
+  double m[4] = {0.0, 0.0, 0.0, 0.0};
+  float mn = INFINITY, mx = -INFINITY;
+  for (int i = threadIdx.x; i < n; i += SSI_THREADS) {
+    const float p = o[i], g = t[i];
+    sp[i] = p;
+    sg[i] = g;
+    const double pd = p, gd = g;
+    m[0] += pd;
+    m[1] += gd;
+    m[2] += pd * pd;
+    m[3] += pd * gd;
+    mn = fminf(mn, p);
+    mx = fmaxf(mx, p);
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, off));
+    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
+  }
+  if (lane == 0) { redf[0][wid] = mn; redf[1][wid] = mx; }
+  ssi_block_sum(m, red);                                  // its barrier also publishes sp, sg and redf
+  for (int w = 0; w < SSI_THREADS / 32; ++w) { mn = fminf(mn, redf[0][w]); mx = fmaxf(mx, redf[1][w]); }
+  const double nd = (double)n, Sp = m[0], Sg = m[1];
+  const double D = m[2] - Sp * Sp / nd, N = m[3] - Sp * Sg / nd;
+  const bool flat = !(mn < mx) || !(D > 0.0);             // constant prediction: s = 0, t = mean g, gradient 0
+  const double sd = flat ? 0.0 : N / D;
+  const float s = (float)sd;
+  const float tt = (float)(__dsub_rn(Sg, __dmul_rn(sd, Sp)) / nd);
+  double inv_nk[SSI_MAX_SCALES];
+#pragma unroll
+  for (int k = 0; k < SSI_MAX_SCALES; ++k) {
+    const int h = 1 << k;
+    inv_nk[k] = 1.0 / ((double)((H + h - 1) >> k) * (double)((W + h - 1) >> k));
+  }
+  // pass 2: sum r^2, sum_k (1/n_k) sum |D|, Q
+  double a[3] = {0.0, 0.0, 0.0};
+  for (int i = threadIdx.x; i < n; i += SSI_THREADS) {
+    const int y = i / W, x = i - y * W;
+    const float ri = ssi_residual(s, tt, sp[i], sg[i]);
+    a[0] += (double)ri * (double)ri;
+#pragma unroll
+    for (int k = 0; k < SSI_MAX_SCALES; ++k) {
+      const int h = 1 << k;
+      if (k >= scales || ((y | x) & (h - 1))) break;      // off grid k means off every coarser grid too
+      if (x + h < W) {
+        const float d = __fsub_rn(ri, ssi_residual(s, tt, sp[i + h], sg[i + h]));
+        a[1] += inv_nk[k] * fabs((double)d);
+        a[2] += inv_nk[k] * ssi_sign(d) * ((double)sp[i] - (double)sp[i + h]);
+      }
+      if (y + h < H) {
+        const float d = __fsub_rn(ri, ssi_residual(s, tt, sp[i + h * W], sg[i + h * W]));
+        a[1] += inv_nk[k] * fabs((double)d);
+        a[2] += inv_nk[k] * ssi_sign(d) * ((double)sp[i] - (double)sp[i + h * W]);
+      }
+    }
+  }
+  ssi_block_sum(a, red);
+  const double al = (double)alpha;
+  if (threadIdx.x == 0) loss_ps[b] = (float)(a[0] / (2.0 * nd) + al * a[1]);
+  if (!dout_f32 && !dout_bf16) return;
+  // pass 3: dL/dp_i / B
+  const double Q = a[2], mp = Sp / nd, mg = Sg / nd, sf = (double)s;
+  for (int i = threadIdx.x; i < n; i += SSI_THREADS) {
+    double gr = 0.0;
+    if (!flat) {
+      const int y = i / W, x = i - y * W;
+      const float ri = ssi_residual(s, tt, sp[i], sg[i]);
+      double c = 0.0;
+#pragma unroll
+      for (int k = 0; k < SSI_MAX_SCALES; ++k) {
+        const int h = 1 << k;
+        if (k >= scales || ((y | x) & (h - 1))) break;
+        double ck = 0.0;                                  // i is the first point (a) of its right / lower pair ...
+        if (x + h < W) ck += ssi_sign(__fsub_rn(ri, ssi_residual(s, tt, sp[i + h], sg[i + h])));
+        if (y + h < H) ck += ssi_sign(__fsub_rn(ri, ssi_residual(s, tt, sp[i + h * W], sg[i + h * W])));
+        if (x >= h) ck -= ssi_sign(__fsub_rn(ssi_residual(s, tt, sp[i - h], sg[i - h]), ri));   // ... the second (b)
+        if (y >= h) ck -= ssi_sign(__fsub_rn(ssi_residual(s, tt, sp[i - h * W], sg[i - h * W]), ri));
+        c += inv_nk[k] * ck;
+      }
+      const double ds = (((double)sg[i] - mg) - 2.0 * sd * ((double)sp[i] - mp)) / D;
+      gr = (sf * (double)ri / nd + al * (sf * c + Q * ds)) / (double)B;
+    }
+    const float gv = (float)gr;
+    if (dout_f32) dout_f32[(size_t)b * ld + i] = gv;
+    if (dout_bf16) dout_bf16[(size_t)b * ld + i] = f32_to_bf16_bits(gv);
+  }
+}
+
+extern "C" int a3d_ssi_loss(a3d_ctx* ctx, const float* out, const float* tar, int B, int H, int W, float alpha,
+                            int scales, float* loss_per_sample, float* loss, float* dout_f32, uint16_t* dout_bf16,
+                            int dout_ld, void* stream) {
+  A3D_REQUIRE(ctx, "ssi_loss: null context");
+  A3D_REQUIRE(out, "ssi_loss: out is null");
+  A3D_REQUIRE(tar, "ssi_loss: tar is null");
+  A3D_REQUIRE(loss_per_sample, "ssi_loss: loss_per_sample is null");
+  A3D_REQUIRE(loss, "ssi_loss: loss is null");
+  A3D_REQUIRE(B > 0 && H > 0 && W > 0, "ssi_loss: bad shape B=%d H=%d W=%d", B, H, W);
+  const size_t n = (size_t)H * (size_t)W, smem = 2 * n * sizeof(float);
+  A3D_REQUIRE(smem <= 200 * 1024, "ssi_loss: H*W = %zu exceeds the shared-memory bound of %d pixels", n,
+              200 * 1024 / (int)(2 * sizeof(float)));
+  if (dout_ld <= 0) dout_ld = (int)n;
+  A3D_REQUIRE((size_t)dout_ld >= n, "ssi_loss: dout_ld = %d < H*W = %zu", dout_ld, n);
+  A3D_REQUIRE(alpha >= 0.f, "ssi_loss: alpha = %g must be >= 0", (double)alpha);
+  A3D_REQUIRE(scales >= 1 && scales <= SSI_MAX_SCALES, "ssi_loss: scales = %d outside 1..%d", scales, SSI_MAX_SCALES);
+  if (smem > 48 * 1024)
+    A3D_CHECK_CUDA(cudaFuncSetAttribute(ssi_loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  ssi_loss_kernel<<<B, SSI_THREADS, smem, as_stream(stream)>>>(out, tar, H, W, B, alpha, scales, loss_per_sample,
+                                                              dout_f32, dout_bf16, dout_ld);
+  A3D_LAUNCH_OK(ctx);
+  mean_kernel<<<1, 32, 0, as_stream(stream)>>>(loss_per_sample, B, loss);
+  A3D_LAUNCH_OK(ctx);
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------ optimizers
 // TF1 ApplyAdam; one pass, 128-bit loads/stores: 16 B read + 12 B written per parameter (+2 B bf16 mirror).
 __global__ void adam_tf_kernel(float4* __restrict__ w, const float4* __restrict__ g, float4* __restrict__ m,

@@ -20,6 +20,9 @@ IN_H, IN_W = 228, 304          # src/models.py:282
 OUT_H, OUT_W = 55, 74          # src/models.py:283
 N_PIX = OUT_H * OUT_W          # 4070 == the 74*55 of src/models.py:269
 LAMBDA_OVER_N = 0.5 / (74 * 55)
+# loss="ssi": the scale-and-shift-invariant objective of MiDaS (Ranftl et al. 2020), gradient-matching weight and scales
+SSI_ALPHA, SSI_SCALES = 0.5, 4
+LOSSES = ("silog", "ssi")
 
 # src/models.py:318-345 -- (learning rate) per Adam instance; beta1 = 0.9 ('momentum'), eps = 1e-8
 ADAM_LR = {"CoarseConv": 0.001, "CoarseDense": 0.1, "FineA": 0.001, "FineB": 0.01}
@@ -117,11 +120,18 @@ class MSDNNet:
 
     `fuse_dense_adam=True` fuses the dense weight gradients into TF-Adam where the kernel supports it: on one GPU, at a
     batch of at most `L.DENSE_WGRAD_ADAM_MAX_M`.  A larger batch, like `fuse_dense_adam=False`, runs the separate dense
-    wgrad and TF-Adam kernels over the CoarseDense group."""
+    wgrad and TF-Adam kernels over the CoarseDense group.
+
+    `loss` picks the objective of both maps: "silog" (default) is the reference's scale-invariant log loss; "ssi" is the
+    scale-and-shift-invariant loss (include/a3d.h a3d_ssi_loss, alpha 0.5, 4 scales), for ground truth that is known
+    only up to a scale and a shift per image, as the min-max scaled targets of the preprocessing are."""
 
     def __init__(self, ctx: ops.Context, batch: int, in_hw=(480, 640), depth_hw=(55, 73), train=True,
                  beta2=ADAM_BETA2_REFERENCE, impl=L.IMPL_AUTO, dropout_seed=2, comm=None, grad_dtype=torch.float32,
-                 overlap=True, fuse_dense_adam=True, dtype="bf16", augment=None, augment_seed=3):
+                 overlap=True, fuse_dense_adam=True, dtype="bf16", augment=None, augment_seed=3, loss="silog"):
+        if loss not in LOSSES:
+            raise ValueError(f"loss must be one of {LOSSES}, not {loss!r}")
+        self.loss = loss
         self.ctx, self.B, self.train, self.beta2, self.impl = ctx, batch, train, beta2, impl
         # dtype = "fp8": inference only.  Every convolution and dense product runs on E4M3 codes (tcgen05 kind::f8f6f4)
         # with one scale per weight row and one per image (include/a3d.h "FP8 inference"); the bf16 buffers below stay as
@@ -422,12 +432,19 @@ class MSDNNet:
                          out=self.fine.view(B, 55, 74, 1))
         # losses (src/models.py:288-290); the gradient of the active branch is produced in the same pass
         gk = "dout" if self.tf32 else "dout_bf16"          # the gradient w.r.t. the prediction, in the storage type
-        c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse,
-                     loss=self.loss_coarse, dout_ld=4096, **{gk: self.g_coarse if self.train else None})
+        self._loss(self.coarse, loss_ps=self.lps_coarse, loss=self.loss_coarse, dout_ld=4096,
+                   **{gk: self.g_coarse if self.train else None})
         with s.lane("fine"):
-            c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine,
-                         dout_ld=N_PIX, **{gk: self.g_fine if self.train else None})
+            self._loss(self.fine, loss_ps=self.lps_fine, loss=self.loss_fine, dout_ld=N_PIX,
+                       **{gk: self.g_fine if self.train else None})
             c.stamp("fine fwd + loss done")
+
+    def _loss(self, pred, **kw):
+        """The loss of one map [B, 4070] against the resized target (and its gradient where `kw` names a buffer)."""
+        if self.loss == "ssi":
+            self.ctx.ssi_loss(pred, self.tar, OUT_H, OUT_W, SSI_ALPHA, SSI_SCALES, want_grad=False, **kw)
+        else:
+            self.ctx.silog_loss(pred, self.tar, LAMBDA_OVER_N, want_grad=False, **kw)
 
     def _forward_fp8(self):
         """The inference forward on E4M3 operands.  Storage points (oracle/fp8.py restates them): the resized image with
@@ -459,8 +476,8 @@ class MSDNNet:
                          relu=True, out=self.f2)
         c.conv2d_fwd(self.d_f3, self.f2, self.w("fine/third/kernel"), self.bias("fine/third"), relu=False,
                      out=self.fine.view(B, 55, 74, 1))
-        c.silog_loss(self.coarse, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_coarse, loss=self.loss_coarse)
-        c.silog_loss(self.fine, self.tar, LAMBDA_OVER_N, want_grad=False, loss_ps=self.lps_fine, loss=self.loss_fine)
+        self._loss(self.coarse, loss_ps=self.lps_coarse, loss=self.loss_coarse)
+        self._loss(self.fine, loss_ps=self.lps_fine, loss=self.loss_fine)
 
     # ------------------------------------------------------------------ backward
     def _dense_wgrad_adam(self, layer, x, dy):

@@ -286,6 +286,25 @@ class Context:
                                         _ptr(dout), _ptr(dout_bf16), dout_ld, _stream()), "silog_loss")
         return loss, loss_ps, dout, dout_bf16
 
+    def ssi_loss(self, out, tar, H, W, alpha=0.5, scales=4, want_grad=True, grad_bf16=False,
+                 loss_ps=None, loss=None, dout=None, dout_bf16=None, dout_ld=0):
+        """Scale-and-shift-invariant loss (include/a3d.h a3d_ssi_loss) of out vs tar, each [B, H*W] (any shape with B
+        leading rows of H*W floats), with the same outputs and keywords as silog_loss."""
+        B = out.shape[0]
+        n = H * W
+        if out.numel() != B * n or tar.numel() != B * n:
+            raise ValueError(f"ssi_loss: out and tar must hold {B} x {H} x {W} floats")
+        dev = out.device
+        loss_ps = loss_ps if loss_ps is not None else torch.empty(B, dtype=torch.float32, device=dev)
+        loss = loss if loss is not None else torch.empty(1, dtype=torch.float32, device=dev)
+        if want_grad and dout is None and not grad_bf16:
+            dout = torch.empty(B, n, dtype=torch.float32, device=dev)
+        if want_grad and grad_bf16 and dout_bf16 is None:
+            dout_bf16 = torch.empty(B, n, dtype=torch.bfloat16, device=dev)
+        L.check(self.lib.a3d_ssi_loss(self.h, _ptr(out), _ptr(tar), B, H, W, alpha, scales, _ptr(loss_ps), _ptr(loss),
+                                      _ptr(dout), _ptr(dout_bf16), dout_ld, _stream()), "ssi_loss")
+        return loss, loss_ps, dout, dout_bf16
+
     def adam_tf(self, w, g, m, v, w_bf16, lr, beta1, beta2, eps, t, grad_scale=1.0, n=None, lr_t_dev=None):
         """TF1 ApplyAdam.  `lr_t_dev` (1-element f32 device tensor) overrides the host-computed lr_t."""
         lr_t = adam_lr_t(lr, beta1, beta2, t)

@@ -231,6 +231,25 @@ int a3d_silog_loss(a3d_ctx*, const float* out, const float* tar, int B, int n, f
                    float* loss_per_sample, float* loss, float* dout_f32, uint16_t* dout_bf16,
                    int dout_ld, void* stream);
 
+/* ---- scale-and-shift-invariant loss (MiDaS, Ranftl et al. 2020) + its gradient -------------------
+ * A training objective for relative depth (targets known up to a scale and a shift per image).  out, tar f32 [B, H*W],
+ * each row an H x W row-major map; every pixel counts.  Per image, with n = H*W and sums in double over the floats:
+ *   fit       D = Spp - Sp^2/n, N = Spg - Sp*Sg/n, sd = N/D, s = float(sd), t = float((Sg - sd*Sp)/n)
+ *             (constant prediction, min p == max p or D <= 0: s = 0, t = float(Sg/n), gradient 0)
+ *   residual  r_i = (float(s*p_i) + t) - g_i                (float32, no fused multiply-add)
+ *   scales    k = 0..scales-1, h = 2^k: grid G_k = {y % h == 0, x % h == 0}, n_k = |G_k|; pairs = horizontally or
+ *             vertically adjacent points of G_k (h pixels apart), a before b; D_ab = float(r_a - r_b)
+ *   loss      L_b = sum r_i^2 / (2n) + alpha * sum_k (1/n_k) sum_pairs |D_ab|   (double, stored as float)
+ *   gradient  dL_b/dp_i = s*r_i/n + alpha*(s*c_i + Q*(g_i - Sg/n - 2*sd*(p_i - Sp/n)) / D), with
+ *             c_i = sum_k (1/n_k) sum_{pairs with i} (+sign(D_ab) if i == a, -sign(D_ab) if i == b), sign(0) = 0,
+ *             Q = sum_k (1/n_k) sum_pairs sign(D_ab) * (p_a - p_b)
+ * loss_per_sample f32 [B]; loss f32 [1] (batch mean); dout as in a3d_silog_loss: d loss / d out (the 1/B included),
+ * f32 and/or bf16 (either may be null), row stride dout_ld (0 = H*W).  alpha >= 0, 1 <= scales <= 4,
+ * 2*H*W floats must fit in 200 KB of shared memory.  No atomics: the same inputs give the same bits. */
+int a3d_ssi_loss(a3d_ctx*, const float* out, const float* tar, int B, int H, int W, float alpha, int scales,
+                 float* loss_per_sample, float* loss, float* dout_f32, uint16_t* dout_bf16, int dout_ld,
+                 void* stream);
+
 /* ---- optimizers (src/models.py:307-345 Adam x4, :198-200 SGD) ------------------------------- */
 /* TF1 ApplyAdam on a flat segment: m = b1*m+(1-b1)*g ; v = b2*v+(1-b2)*g^2 ;
  * w -= lr_t*m/(sqrt(v)+eps), lr_t = lr*sqrt(1-b2^t)/(1-b1^t) computed by the caller in double.
